@@ -6,6 +6,7 @@ Mpix/s and 4K frames/s at 1/2/4/8 GPUs, % of HBM roofline).
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # the reference's CPU path (oracle port) on host cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's outputs to DIR/<name>.npy
 
 Workload (BASELINE.json configs[4], the one the metric is quoted on): a synthetic 4K (3840x2160)
 60-frame uint8 video batch PER GPU (weak scaling: frames are independent, no collective), species
@@ -170,6 +171,33 @@ def make_host_frames(rank: int, world: int, n_frames: int, H: int, W: int, pinne
             view[j] = np.random.default_rng(s).integers(0, 256, (H, W, 3), dtype=np.uint8)
         out[sp] = t
     return out
+
+
+DUMP_BYTES = 64 * 10 ** 6
+DUMP_SEED = 0
+
+
+def dump_outputs(directory: str, dev_out):
+    """Write the outputs of the last timed step as float32 .npy files, DUMP_BYTES in all, so that two builds can
+    be compared output for output.  An output larger than its share of the budget is sampled: the same
+    default_rng(DUMP_SEED) draw of pixels (all three channels, in raster order) for every output of that shape."""
+    import torch
+    arrays = {"dog": dev_out["Dog"], "cat_human": dev_out["Cat"][0], "cat_view": dev_out["Cat"][1],
+              "honeybee": dev_out["HoneyBee"]}
+    budget_px = (DUMP_BYTES // len(arrays) - 1024) // (3 * 4)        # 1 KB per file for the .npy header
+    os.makedirs(directory, exist_ok=True)
+    picks = {}
+    for name, t in arrays.items():
+        n_px = t.numel() // 3
+        if n_px <= budget_px:
+            a = t.float().cpu().numpy()
+        else:
+            if t.shape not in picks:
+                idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n_px, budget_px, replace=False))
+                picks[t.shape] = torch.from_numpy(idx).to(t.device)
+            a = t.reshape(n_px, 3).index_select(0, picks[t.shape]).float().cpu().numpy()
+        np.save(os.path.join(directory, name + ".npy"), a)
+    log(f"[rank 0] outputs of the last timed step written to {directory} ({', '.join(arrays)})")
 
 
 def peak_numbers():
@@ -581,6 +609,8 @@ def run_b200(args):
     t_wall1 = time.time()
     ms_step = max_over_ranks(e0.elapsed_time(e1) / args.steps)
     launches = eng.launches - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dev_out)
 
     # ---- per-kernel timing over the same steps (roofline leg): CUDA events around every launch
     prof_steps = max(1, min(args.steps, 3))
@@ -739,7 +769,14 @@ def main():
     ap.add_argument("--no-configs", action="store_true", help="skip the per-config 1080p single-frame legs")
     ap.add_argument("--streams", type=int, default=1, help="streams per species batch in the device-resident step (the batch is cut into that many parts); 0: a single stream")
     ap.add_argument("--mstpp-batch", type=int, default=4, help="482x512 patches per GPU in the MST++ leg (0: skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step (rank 0's frames) as DIR/<name>.npy, float32, "
+                         "at most 64 MB in all: a fixed seeded pixel sample of a larger output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl b200)")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
