@@ -16,7 +16,8 @@ from . import _build
 _lock = threading.Lock()
 _lib = None
 
-AVB_VERSION = 120            # include/avb200.h AVB_VERSION
+AVB_VERSION = 130            # include/avb200.h AVB_VERSION
+AVB_JPEG_HEADER_MAX = 1024
 AVB_NORM_DIV255 = 0
 AVB_NORM_AUTO = 1
 AVB_ENC_TABLE_MAX = 2048
@@ -63,6 +64,9 @@ SIGNATURES = {
     "avb_vm_run": (_i, [_p, _i, _i, _i, _i, _i, _p, _i, _p, _i, _p]),
     "avb_img_remap": (_i, [_p, _p, _i, _i, _i, _i, _p, _p, _p]),
     "avb_uv_map_u8": (_i, [_p, _p, _i, _i, _i, _i64, _i64, _i64, _i64, _p, _p, _p, _p, _i, _f, _i, _p, _i, _i, _p, _f, _p, _p, _p]),
+    "avb_jpeg_bound_bytes": (_i64, [_i, _i]),
+    "avb_jpeg_workspace_bytes": (_i64, [_i, _i, _i]),
+    "avb_jpeg_encode_u8": (_i, [_p, _i, _i, _i, _i64, _i64, _p, _i, _p, _p, _i64, _p, _p, _p]),
 }
 
 

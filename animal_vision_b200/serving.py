@@ -4,9 +4,13 @@
 The reference handles one socket's frame at a time: JPEG bytes -> temp.jpg -> cv2.imread -> `filter.visualize(img)[1]` ->
 tempexport.jpg -> base64 data URI, and the asyncio loop blocks on it.  Here every frame that is waiting -- from any
 number of sockets -- is grouped by (species key, frame shape) and each group runs as ONE device batch through
-`visualize_batch`; JPEG decode / encode stay on the host and in memory (no temp files).  `FrameBatcher.submit` is thread
+`visualize_batch`; JPEG decode stays on the host and in memory (no temp files).  `FrameBatcher.submit` is thread
 safe and returns a `concurrent.futures.Future`; `process_image` is the drop-in for `processimage` (same arguments, same
-data-URI result, same string keys: "human", "cat", "cow", ... as utils.py:145-191, plus keys for the UV species)."""
+data-URI result, same string keys: "human", "cat", "cow", ... as utils.py:145-191, plus keys for the UV species).
+
+`FrameBatcher.submit_jpeg` asks for the JPEG file of the species view instead of its pixels.  Where the batch result
+lives decides the encoder: a view left on the device by the default runner is encoded there (K8, `jpeg.encode_jpeg`,
+the bytes of cv2.imencode) and only the compressed bytes come back; a NumPy result is encoded with cv2.imencode."""
 from __future__ import annotations
 
 import base64
@@ -32,8 +36,9 @@ SERVER_KEYS: Dict[str, str] = {
 }
 
 
-def _device_runner(device=None) -> Callable[[str, np.ndarray], np.ndarray]:
-    """run(key, frames[k,H,W,3] uint8) -> the species view of every frame, [k,H,W,3] uint8 (index [1] of `visualize`)."""
+def _device_runner(device=None) -> Callable[[str, np.ndarray], object]:
+    """run(key, frames[k,H,W,3] uint8) -> the species view of every frame, a [k,H,W,3] uint8 CUDA tensor (index [1] of
+    `visualize`), enqueued on the current stream."""
     from .engine import get_engine
     species: Dict[str, object] = {}
 
@@ -46,12 +51,40 @@ def _device_runner(device=None) -> Callable[[str, np.ndarray], np.ndarray]:
         with t.cuda.device(eng.device):
             pin = t.from_numpy(frames).pin_memory()
             dev = pin.to(eng.device, non_blocking=True)
-            res = sp.visualize_batch(dev)
-            out = t.empty(tuple(frames.shape), dtype=t.uint8).pin_memory()
-            out.copy_(res[1], non_blocking=True)
-            t.cuda.current_stream(eng.device).synchronize()
-            return out.numpy()
+            return sp.visualize_batch(dev)[1]
     return run
+
+
+def _pixels(view, idx: List[int]) -> List[np.ndarray]:
+    """The frames `idx` of a batch result as host arrays (one D2H copy for a device result)."""
+    if isinstance(view, np.ndarray):
+        return [np.array(view[i], copy=True) for i in idx]
+    import torch
+    with torch.cuda.device(view.device):
+        sel = view if len(idx) == view.shape[0] else view[torch.tensor(idx, device=view.device)]
+        pin = torch.empty(tuple(sel.shape), dtype=torch.uint8).pin_memory()
+        pin.copy_(sel, non_blocking=True)
+        torch.cuda.current_stream(view.device).synchronize()
+        return [pin[k].numpy() for k in range(len(idx))]
+
+
+def _encode_host(frame: np.ndarray) -> bytes:
+    import cv2
+    ok, enc = cv2.imencode(".jpg", frame)
+    if not ok:
+        raise ValueError("could not encode the result")
+    return enc.tobytes()
+
+
+def _jpegs(view, idx: List[int]) -> List[bytes]:
+    """JPEG files (cv2.imencode's bytes, quality 95) of the frames `idx` of a batch result."""
+    if isinstance(view, np.ndarray):
+        return [_encode_host(view[i]) for i in idx]
+    import torch
+    from .jpeg import encode_jpeg
+    with torch.cuda.device(view.device):
+        sel = view if len(idx) == view.shape[0] else view[torch.tensor(idx, device=view.device)]
+        return encode_jpeg(sel, 95)
 
 
 class FrameBatcher:
@@ -73,6 +106,14 @@ class FrameBatcher:
         self._worker.start()
 
     def submit(self, frame: np.ndarray, animal: str) -> Future:
+        """Future of the species view of `frame`, an HxWx3 uint8 array."""
+        return self._submit(frame, animal, False)
+
+    def submit_jpeg(self, frame: np.ndarray, animal: str) -> Future:
+        """Future of the JPEG file (bytes) of the species view, the bytes cv2.imencode(".jpg", view) gives."""
+        return self._submit(frame, animal, True)
+
+    def _submit(self, frame: np.ndarray, animal: str, jpeg: bool) -> Future:
         fut: Future = Future()
         if animal != "human" and animal not in SERVER_KEYS:
             fut.set_exception(KeyError(f"no case implemented for {animal!r}"))             # utils.py:192-193 prints and fails later
@@ -81,12 +122,18 @@ class FrameBatcher:
             fut.set_exception(AssertionError("frame must be a HxWx3 uint8 array"))
             return fut
         if animal == "human":                                                               # utils.py:146-147
-            fut.set_result(frame)
+            if not jpeg:
+                fut.set_result(frame)
+                return fut
+            try:
+                fut.set_result(_encode_host(frame))
+            except Exception as e:          # noqa: BLE001
+                fut.set_exception(e)
             return fut
         with self._cv:
             if self._stop:
                 raise RuntimeError("FrameBatcher is closed")
-            self._q.append((animal, frame, fut))
+            self._q.append((animal, frame, fut, jpeg))
             self._cv.notify()
         return fut
 
@@ -106,18 +153,23 @@ class FrameBatcher:
                 pending = list(self._q)
                 self._q.clear()
             groups: "OrderedDict[Tuple[str, Tuple[int, ...]], list]" = OrderedDict()
-            for animal, frame, fut in pending:
-                groups.setdefault((animal, frame.shape), []).append((frame, fut))
+            for animal, frame, fut, jpeg in pending:
+                groups.setdefault((animal, frame.shape), []).append((frame, fut, jpeg))
             for (animal, _shape), items in groups.items():
                 for a in range(0, len(items), self.max_batch):
                     part = items[a:a + self.max_batch]
                     try:
-                        out = self._run(animal, np.stack([f for f, _ in part]))
+                        out = self._run(animal, np.stack([f for f, _, _ in part]))
                         self.batches.append((animal, len(part)))
-                        for i, (_, fut) in enumerate(part):
-                            fut.set_result(np.array(out[i], copy=True))
+                        pix = [i for i, (_, _, jpeg) in enumerate(part) if not jpeg]
+                        jpg = [i for i, (_, _, jpeg) in enumerate(part) if jpeg]
+                        res = dict(zip(pix, _pixels(out, pix))) if pix else {}
+                        if jpg:
+                            res.update(zip(jpg, _jpegs(out, jpg)))
+                        for i, (_, fut, _) in enumerate(part):
+                            fut.set_result(res[i])
                     except Exception as e:          # noqa: BLE001  (a failed batch fails its own requests, the loop lives on)
-                        for _, fut in part:
+                        for _, fut, _ in part:
                             if not fut.done():
                                 fut.set_exception(e)
 
@@ -153,8 +205,5 @@ def process_image(imagedata: bytes, animal: str, batcher: Optional[FrameBatcher]
     img = cv2.imdecode(np.frombuffer(imagedata, np.uint8), cv2.IMREAD_COLOR)
     if img is None:
         raise ValueError("could not decode the image")
-    out = (batcher or default_batcher()).submit(img, animal).result()
-    ok, enc = cv2.imencode(".jpg", out)
-    if not ok:
-        raise ValueError("could not encode the result")
-    return "data:image/jpeg;base64," + base64.b64encode(enc.tobytes()).decode("utf-8")
+    enc = (batcher or default_batcher()).submit_jpeg(img, animal).result()
+    return "data:image/jpeg;base64," + base64.b64encode(enc).decode("utf-8")

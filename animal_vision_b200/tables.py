@@ -477,3 +477,58 @@ def panorama_geometry(W: int, scale_x: float):
 def scaled_hw(H: int, W: int, scale: float):
     """uv_helpers.py:169-171 classic_rgb_to_hsi_scaled: size of the down-sampled frame."""
     return max(1, int(round(H * scale))), max(1, int(round(W * scale)))
+
+
+# ---------------------------------------------------------------------------------------------------- JPEG (K8)
+# What libjpeg(-turbo) writes for cv2.imencode(".jpg", frame, [IMWRITE_JPEG_QUALITY, q]) with OpenCV's defaults.
+JPEG_ZIGZAG = np.array([0, 1, 8, 16, 9, 2, 3, 10, 17, 24, 32, 25, 18, 11, 4, 5, 12, 19, 26, 33, 40, 48, 41, 34, 27, 20, 13, 6,
+                        7, 14, 21, 28, 35, 42, 49, 56, 57, 50, 43, 36, 29, 22, 15, 23, 30, 37, 44, 51, 58, 59, 52, 45, 38, 31,
+                        39, 46, 53, 60, 61, 54, 47, 55, 62, 63])
+_JPEG_STD_Q = (  # ITU-T T.81 Annex K.1, natural order: luminance, chrominance
+    [16, 11, 10, 16, 24, 40, 51, 61, 12, 12, 14, 19, 26, 58, 60, 55, 14, 13, 16, 24, 40, 57, 69, 56, 14, 17, 22, 29, 51, 87, 80,
+     62, 18, 22, 37, 56, 68, 109, 103, 77, 24, 35, 55, 64, 81, 104, 113, 92, 49, 64, 78, 87, 103, 121, 120, 101, 72, 92, 95, 98,
+     112, 100, 103, 99],
+    [17, 18, 24, 47] + [99] * 4 + [18, 21, 26, 66] + [99] * 4 + [24, 26, 56] + [99] * 5 + [47, 66] + [99] * 38)
+_JPEG_STD_HUFF = (  # ITU-T T.81 Annex K.3 as (table class/id, bits[1..16], values): DC0, AC0, DC1, AC1
+    (0x00, "00010501010101010100000000000000", "000102030405060708090a0b"),
+    (0x10, "0002010303020403050504040000017d",
+     "01020300041105122131410613516107227114328191a1082342b1c11552d1f02433627282090a161718191a25262728292a3435363738"
+     "393a434445464748494a535455565758595a636465666768696a737475767778797a838485868788898a92939495969798999aa2a3a4a5"
+     "a6a7a8a9aab2b3b4b5b6b7b8b9bac2c3c4c5c6c7c8c9cad2d3d4d5d6d7d8d9dae1e2e3e4e5e6e7e8e9eaf1f2f3f4f5f6f7f8f9fa"),
+    (0x01, "00030101010101010101010000000000", "000102030405060708090a0b"),
+    (0x11, "00020102040403040705040400010277",
+     "000102031104052131061241510761711322328108144291a1b1c109233352f0156272d10a162434e125f11718191a262728292a35363738"
+     "393a434445464748494a535455565758595a636465666768696a737475767778797a82838485868788898a92939495969798999aa2a3a4a5"
+     "a6a7a8a9aab2b3b4b5b6b7b8b9bac2c3c4c5c6c7c8c9cad2d3d4d5d6d7d8d9dae2e3e4e5e6e7e8e9eaf2f3f4f5f6f7f8f9fa"),
+)
+
+
+def jpeg_quant_tables(quality: int) -> np.ndarray:
+    """[2, 64] uint8 quantisers in zigzag order (luma, chroma), i.e. the payloads of the two DQT segments:
+    jcparam.c jpeg_quality_scaling (5000/q below 50, 200-2q otherwise), (std*scale + 50)/100 clamped to [1, 255]."""
+    q = int(quality)
+    if not 1 <= q <= 100:
+        raise ValueError(f"JPEG quality must lie in [1, 100], got {quality!r}")
+    scale = 5000 // q if q < 50 else 200 - 2 * q
+    t = np.clip((np.array(_JPEG_STD_Q, np.int64) * scale + 50) // 100, 1, 255)
+    return t[:, JPEG_ZIGZAG].astype(np.uint8)
+
+
+def _jpeg_segment(marker: int, payload: bytes) -> bytes:
+    return bytes([0xFF, marker]) + (len(payload) + 2).to_bytes(2, "big") + payload
+
+
+def jpeg_header(H: int, W: int, quality: int) -> bytes:
+    """Every byte cv2.imencode writes before the entropy-coded data: SOI, APP0 JFIF 1.01 (density 1:1, no units),
+    DQT luma / chroma, SOF0 (3 components, 4:2:0), DHT DC0 / AC0 / DC1 / AC1, SOS."""
+    if not (1 <= int(H) <= 65535 and 1 <= int(W) <= 65535):
+        raise ValueError(f"JPEG frame size must lie in [1, 65535]^2, got {H}x{W}")
+    qt = jpeg_quant_tables(quality)
+    out = b"\xff\xd8" + _jpeg_segment(0xE0, b"JFIF\x00\x01\x01\x00\x00\x01\x00\x01\x00\x00")
+    for i in range(2):
+        out += _jpeg_segment(0xDB, bytes([i]) + qt[i].tobytes())
+    out += _jpeg_segment(0xC0, bytes([8]) + int(H).to_bytes(2, "big") + int(W).to_bytes(2, "big")
+                         + bytes([3, 1, 0x22, 0, 2, 0x11, 1, 3, 0x11, 1]))
+    for tc, bits, vals in _JPEG_STD_HUFF:
+        out += _jpeg_segment(0xC4, bytes([tc]) + bytes.fromhex(bits) + bytes.fromhex(vals))
+    return out + _jpeg_segment(0xDA, bytes([3, 1, 0x00, 2, 0x11, 3, 0x11, 0, 63, 0]))

@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define AVB_VERSION 120            /* 0.1.2 */
+#define AVB_VERSION 130            /* 0.1.3 */
 
 #define AVB_OK 0
 #define AVB_E_ARG (-1)             /* bad argument (null pointer, non-positive size, unsupported radius ...) */
@@ -347,6 +347,24 @@ AVB_API int avb_vm_run(const avb_vm_ins *prog_dev, int n_ins, int n_regs, int n,
  * (animals/anableps.py:224-237): map coordinates quantised to 1/32 px exactly as OpenCV does. */
 AVB_API int avb_img_remap(const float *in_dev, float *out_dev, int n, int H, int W, int C, const float *mapx_dev,
                           const float *mapy_dev, avb_stream_t stream);
+
+/* ---- K8: baseline JPEG encode (csrc/k8_jpeg.cu) ---------------------------------------------------------
+ * The bytes of cv2.imencode(".jpg", frame, [IMWRITE_JPEG_QUALITY, q]) with OpenCV's defaults (libjpeg-turbo:
+ * baseline, 4:2:0, standard Huffman tables, no restart interval) for n packed 8-bit 3-channel frames in the channel
+ * order cv2 expects (BGR); replaces the host encode of the reference's processimage (utils.py:133-199).
+ *   header_host     the bytes before the entropy-coded data (SOI .. SOS; animal_vision_b200/tables.py jpeg_header),
+ *                   header_len <= AVB_JPEG_HEADER_MAX; copied in front of every frame's data
+ *   qtables_host    2 x 64 quantiser values in zigzag order (luma, chroma; the DQT payloads of the header), 1..255
+ *   out             n slots of out_slot_stride >= avb_jpeg_bound_bytes(H, W) bytes: frame f's file is written from
+ *                   out + f * out_slot_stride, its length (header + data + EOI) to out_lengths_dev[f] (device int64)
+ *   workspace_dev   avb_jpeg_workspace_bytes(n, H, W) bytes, 16-byte aligned
+ * H and W lie in [1, 65535] (the SOF0 fields). */
+#define AVB_JPEG_HEADER_MAX 1024
+AVB_API int64_t avb_jpeg_bound_bytes(int H, int W);
+AVB_API int64_t avb_jpeg_workspace_bytes(int n, int H, int W);
+AVB_API int avb_jpeg_encode_u8(const uint8_t *in, int n, int H, int W, int64_t in_frame_stride, int64_t in_row_stride,
+                               const uint8_t *header_host, int header_len, const uint8_t *qtables_host, uint8_t *out,
+                               int64_t out_slot_stride, int64_t *out_lengths_dev, void *workspace_dev, avb_stream_t stream);
 
 #ifdef __cplusplus
 }
