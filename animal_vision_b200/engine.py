@@ -210,6 +210,31 @@ class Engine:
         check(rc, "avb_uv_map_u8")
         self.launches += 3 + (4 if map_mode != 2 else 0)      # stats, prep, [hist, scan, collect, select], map
 
+    def split_stencil(self, h: int, w: int, left: str, right: str):
+        """(band_rows, class map, tables) of the corner labels of an h x w split frame on this device
+        (tables.split_label_stencil), built and uploaded once per (h, w, labels)."""
+        def build():
+            st = tables.split_label_stencil(int(h), int(w), str(left), str(right))
+            with self.torch.cuda.device(self.device):
+                return st.band_rows, self._dev(st.classes.view(np.int16)), self._dev(st.luts)
+        return self.cached(("split_labels", int(h), int(w), str(left), str(right)), build)
+
+    @_on_device
+    def split_compose(self, left, right, out, seam: bool, stencil=None):
+        """K9 (avb_split_compose_u8) on the current stream: `out` = left half of `left`, right half of `right`, the seam,
+        and the labels of `stencil` (from split_stencil; None for none)."""
+        n, h, w, lfs, lrs = self.check_frames(left, "original")
+        _, _, _, rfs, rrs = self.check_frames(right, "modified")
+        _, _, _, ofs, ors = self.check_frames(out, "out")
+        if n == 0 or h == 0 or w == 0:
+            return
+        band, cls, lut = stencil if stencil is not None else (0, None, None)
+        rc = self.lib.avb_split_compose_u8(
+            left.data_ptr(), right.data_ptr(), out.data_ptr(), n, h, w, lfs, lrs, rfs, rrs, ofs, ors, int(seam), band,
+            None if cls is None else cls.data_ptr(), None if lut is None else lut.data_ptr(), self.stream_ptr())
+        check(rc, "avb_split_compose_u8")
+        self.launches += 1
+
     # ------------------------------------------------------------------ NumPy shim staging
     @_on_device
     def staging(self, shape, slots: int = 1):

@@ -10,7 +10,14 @@ data-URI result, same string keys: "human", "cat", "cow", ... as utils.py:145-19
 
 `FrameBatcher.submit_jpeg` asks for the JPEG file of the species view instead of its pixels.  Where the batch result
 lives decides the encoder: a view left on the device by the default runner is encoded there (K8, `jpeg.encode_jpeg`,
-the bytes of cv2.imencode) and only the compressed bytes come back; a NumPy result is encoded with cv2.imencode."""
+the bytes of cv2.imencode) and only the compressed bytes come back; a NumPy result is encoded with cv2.imencode.
+
+`FrameBatcher.submit_split_jpeg` asks for the JPEG file of the labelled split-compare frame of the request's input and
+its species view -- what the reference's CLI shows (main.py:41-48 `render_split_compare(img, out)`, with the defaults of
+`make_split_frame`).  Split requests share the species launch of their (key, shape) group with pixel and JPEG requests;
+on the device they are composed (K9, `split_compare_batch(..., labels=...)`) per distinct (labels, seam) from the input
+the runner already uploaded, and encoded by K8.  `process_split_image` wraps it as a data URI.  The reference server's
+`processsplitimage` (utils.py:202-336) is not restated here: this is the split frame defined above, not a drop-in."""
 from __future__ import annotations
 
 import base64
@@ -36,23 +43,33 @@ SERVER_KEYS: Dict[str, str] = {
 }
 
 
-def _device_runner(device=None) -> Callable[[str, np.ndarray], object]:
+class _DeviceRunner:
     """run(key, frames[k,H,W,3] uint8) -> the species view of every frame, a [k,H,W,3] uint8 CUDA tensor (index [1] of
-    `visualize`), enqueued on the current stream."""
-    from .engine import get_engine
-    species: Dict[str, object] = {}
+    `visualize`), enqueued on the current stream.  `upload_and_run` also returns the uploaded input, so split requests
+    compose from it without a second upload."""
 
-    def run(key: str, frames: np.ndarray) -> np.ndarray:
-        eng = get_engine(device)
+    def __init__(self, device=None):
+        self.device = device
+        self.species: Dict[str, object] = {}
+
+    def upload_and_run(self, key: str, frames: np.ndarray):
+        from .engine import get_engine
+        eng = get_engine(self.device)
         t = eng.torch
-        sp = species.get(key)
+        sp = self.species.get(key)
         if sp is None:
-            sp = species[key] = getattr(A, SERVER_KEYS[key])()
+            sp = self.species[key] = getattr(A, SERVER_KEYS[key])()
         with t.cuda.device(eng.device):
             pin = t.from_numpy(frames).pin_memory()
             dev = pin.to(eng.device, non_blocking=True)
-            return sp.visualize_batch(dev)[1]
-    return run
+            return dev, sp.visualize_batch(dev)[1]
+
+    def __call__(self, key: str, frames: np.ndarray):
+        return self.upload_and_run(key, frames)[1]
+
+
+def _device_runner(device=None) -> _DeviceRunner:
+    return _DeviceRunner(device)
 
 
 def _pixels(view, idx: List[int]) -> List[np.ndarray]:
@@ -87,6 +104,39 @@ def _jpegs(view, idx: List[int]) -> List[bytes]:
         return encode_jpeg(sel, 95)
 
 
+def _split_host(frame: np.ndarray, view: np.ndarray, labels: Tuple[str, str], seam: bool) -> bytes:
+    """The host route of a split request: slice copies, cv2 labels, cv2.imencode."""
+    import torch
+    from .renderers.video import draw_split_labels, split_compare_batch
+    comp = split_compare_batch(torch.from_numpy(frame[None]), torch.from_numpy(np.ascontiguousarray(view)[None]),
+                               draw_seam=seam)[0].numpy()
+    return _encode_host(draw_split_labels(comp, *labels))
+
+
+def _split_jpegs(frames: np.ndarray, dev_in, view, idx: List[int], labels: Tuple[str, str], seam: bool) -> List[bytes]:
+    """JPEG files of the labelled split frames (input | species view) of the frames `idx` of a batch."""
+    if isinstance(view, np.ndarray):
+        return [_split_host(frames[i], view[i], labels, seam) for i in idx]
+    import torch
+    from .jpeg import encode_jpeg
+    from .renderers.video import split_compare_batch
+    with torch.cuda.device(view.device):
+        if dev_in is None:
+            dev_in = torch.from_numpy(frames).pin_memory().to(view.device, non_blocking=True)
+        if len(idx) == view.shape[0]:
+            orig, sel = dev_in, view
+        else:
+            ix = torch.tensor(idx, device=view.device)
+            orig, sel = dev_in[ix], view[ix]
+        return encode_jpeg(split_compare_batch(orig, sel, draw_seam=seam, labels=labels), 95)
+
+
+def _check_labels(labels) -> Tuple[str, str]:
+    if not (isinstance(labels, (tuple, list)) and len(labels) == 2 and all(isinstance(x, str) for x in labels)):
+        raise TypeError(f"labels must be a pair of strings, got {labels!r}")
+    return (labels[0], labels[1])
+
+
 class FrameBatcher:
     """Collects (frame, species key) requests from any number of producers and runs them as device batches.
 
@@ -107,13 +157,27 @@ class FrameBatcher:
 
     def submit(self, frame: np.ndarray, animal: str) -> Future:
         """Future of the species view of `frame`, an HxWx3 uint8 array."""
-        return self._submit(frame, animal, False)
+        return self._submit(frame, animal, None)
 
     def submit_jpeg(self, frame: np.ndarray, animal: str) -> Future:
         """Future of the JPEG file (bytes) of the species view, the bytes cv2.imencode(".jpg", view) gives."""
-        return self._submit(frame, animal, True)
+        return self._submit(frame, animal, "jpeg")
 
-    def _submit(self, frame: np.ndarray, animal: str, jpeg: bool) -> Future:
+    def submit_split_jpeg(self, frame: np.ndarray, animal: str, labels: Tuple[str, str] = ("Original", "Transformed"),
+                          draw_seam: bool = True) -> Future:
+        """Future of the JPEG file (bytes) of the split-compare frame of `frame` and its species view: left half of
+        the input, right half of the view, the seam, and the two corner labels -- the bytes of
+        cv2.imencode(".jpg", draw_split_labels(split frame, *labels))."""
+        try:
+            kind = ("split", _check_labels(labels), bool(draw_seam))
+        except TypeError as e:
+            fut: Future = Future()
+            fut.set_exception(e)
+            return fut
+        return self._submit(frame, animal, kind)
+
+    def _submit(self, frame: np.ndarray, animal: str, kind) -> Future:
+        """kind: None (pixels), "jpeg", or ("split", labels, seam)."""
         fut: Future = Future()
         if animal != "human" and animal not in SERVER_KEYS:
             fut.set_exception(KeyError(f"no case implemented for {animal!r}"))             # utils.py:192-193 prints and fails later
@@ -122,18 +186,18 @@ class FrameBatcher:
             fut.set_exception(AssertionError("frame must be a HxWx3 uint8 array"))
             return fut
         if animal == "human":                                                               # utils.py:146-147
-            if not jpeg:
+            if kind is None:
                 fut.set_result(frame)
                 return fut
             try:
-                fut.set_result(_encode_host(frame))
+                fut.set_result(_encode_host(frame) if kind == "jpeg" else _split_host(frame, frame, kind[1], kind[2]))
             except Exception as e:          # noqa: BLE001
                 fut.set_exception(e)
             return fut
         with self._cv:
             if self._stop:
                 raise RuntimeError("FrameBatcher is closed")
-            self._q.append((animal, frame, fut, jpeg))
+            self._q.append((animal, frame, fut, kind))
             self._cv.notify()
         return fut
 
@@ -153,25 +217,40 @@ class FrameBatcher:
                 pending = list(self._q)
                 self._q.clear()
             groups: "OrderedDict[Tuple[str, Tuple[int, ...]], list]" = OrderedDict()
-            for animal, frame, fut, jpeg in pending:
-                groups.setdefault((animal, frame.shape), []).append((frame, fut, jpeg))
+            for animal, frame, fut, kind in pending:
+                groups.setdefault((animal, frame.shape), []).append((frame, fut, kind))
             for (animal, _shape), items in groups.items():
                 for a in range(0, len(items), self.max_batch):
                     part = items[a:a + self.max_batch]
                     try:
-                        out = self._run(animal, np.stack([f for f, _, _ in part]))
-                        self.batches.append((animal, len(part)))
-                        pix = [i for i, (_, _, jpeg) in enumerate(part) if not jpeg]
-                        jpg = [i for i, (_, _, jpeg) in enumerate(part) if jpeg]
-                        res = dict(zip(pix, _pixels(out, pix))) if pix else {}
-                        if jpg:
-                            res.update(zip(jpg, _jpegs(out, jpg)))
-                        for i, (_, fut, _) in enumerate(part):
-                            fut.set_result(res[i])
+                        self._run_part(animal, part)
                     except Exception as e:          # noqa: BLE001  (a failed batch fails its own requests, the loop lives on)
                         for _, fut, _ in part:
                             if not fut.done():
                                 fut.set_exception(e)
+
+    def _run_part(self, animal: str, part: list):
+        """One species launch for the requests `part` of one (key, shape) group, then each request's own result."""
+        batch = np.stack([f for f, _, _ in part])
+        splits: "OrderedDict[tuple, List[int]]" = OrderedDict()
+        for i, (_, _, kind) in enumerate(part):
+            if kind is not None and kind != "jpeg":
+                splits.setdefault(kind[1:], []).append(i)
+        upload_and_run = getattr(self._run, "upload_and_run", None)
+        if splits and upload_and_run is not None:
+            dev_in, out = upload_and_run(animal, batch)
+        else:
+            dev_in, out = None, self._run(animal, batch)
+        self.batches.append((animal, len(part)))
+        pix = [i for i, (_, _, kind) in enumerate(part) if kind is None]
+        jpg = [i for i, (_, _, kind) in enumerate(part) if kind == "jpeg"]
+        res = dict(zip(pix, _pixels(out, pix))) if pix else {}
+        if jpg:
+            res.update(zip(jpg, _jpegs(out, jpg)))
+        for (labels, seam), idx in splits.items():
+            res.update(zip(idx, _split_jpegs(batch, dev_in, out, idx, labels, seam)))
+        for i, (_, fut, _) in enumerate(part):
+            fut.set_result(res[i])
 
     def close(self):
         with self._cv:
@@ -206,4 +285,17 @@ def process_image(imagedata: bytes, animal: str, batcher: Optional[FrameBatcher]
     if img is None:
         raise ValueError("could not decode the image")
     enc = (batcher or default_batcher()).submit_jpeg(img, animal).result()
+    return "data:image/jpeg;base64," + base64.b64encode(enc).decode("utf-8")
+
+
+def process_split_image(imagedata: bytes, animal: str, labels: Tuple[str, str] = ("Original", "Transformed"),
+                        batcher: Optional[FrameBatcher] = None) -> str:
+    """JPEG bytes in, data URI of the JPEG of the labelled split-compare frame out (input on the left, species view on
+    the right, seam, corner labels; `FrameBatcher.submit_split_jpeg`).  Decoded BGR as cv2.imread gives it, like
+    `process_image`."""
+    import cv2
+    img = cv2.imdecode(np.frombuffer(imagedata, np.uint8), cv2.IMREAD_COLOR)
+    if img is None:
+        raise ValueError("could not decode the image")
+    enc = (batcher or default_batcher()).submit_split_jpeg(img, animal, labels).result()
     return "data:image/jpeg;base64," + base64.b64encode(enc).decode("utf-8")

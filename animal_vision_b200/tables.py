@@ -18,6 +18,7 @@ from __future__ import annotations
 
 import math
 from functools import lru_cache
+from typing import NamedTuple
 
 import numpy as np
 
@@ -532,3 +533,65 @@ def jpeg_header(H: int, W: int, quality: int) -> bytes:
     for tc, bits, vals in _JPEG_STD_HUFF:
         out += _jpeg_segment(0xC4, bytes([tc]) + bytes.fromhex(bits) + bytes.fromhex(vals))
     return out + _jpeg_segment(0xDA, bytes([3, 1, 0x00, 2, 0x11, 3, 0x11, 0, 63, 0]))
+
+
+# ----------------------------------------------------------------------------- split-compare labels (K9)
+SPLIT_LABEL_MARGIN = 16            # rows drawn below the lowest label rectangle; they must come out untouched
+SPLIT_CLASS_INDEX = np.uint16      # class map dtype (K9 reads uint16)
+
+
+class SplitLabelStencil(NamedTuple):
+    band_rows: int                 # rows [0, band_rows) hold every pixel the labels change
+    classes: np.ndarray            # [band_rows, W] SPLIT_CLASS_INDEX: table of each pixel, 0 = identity
+    luts: np.ndarray               # [n_classes, 256] uint8: byte b of a pixel of class c becomes luts[c, b]
+
+
+@lru_cache(maxsize=64)
+def split_label_stencil(H: int, W: int, left: str, right: str) -> SplitLabelStencil:
+    """`draw_split_labels(frame, left, right)` of an H x W frame as a per-pixel byte map.
+
+    Every step of the label drawing (addWeighted of a black overlay, anti-aliased putText towards two constant grey
+    colours) maps one byte of one pixel to one byte of the same pixel and channel, the same way for all three channels.
+    So the drawing is out[y, x, c] = F_(y,x)(in[y, x, c]), and F is found by drawing on constant canvases: draw k
+    carries the values 3k, 3k + 1, 3k + 2 in the three channels, so 86 draws give all 256 inputs.  Only the top rows
+    are drawn (the label rectangles' bottom row plus SPLIT_LABEL_MARGIN rows, with the geometry of the full frame), so
+    the cost grows with the band, not the frame; the margin rows must come out unchanged, which shows that no stroke
+    was clipped by the shorter canvas.  Pixels sharing a table share a class."""
+    from .renderers.video import draw_label_boxes, split_label_geometry
+    H, W = int(H), int(W)
+    if H < 1 or W < 1:
+        raise ValueError(f"split_label_stencil: frame size {H}x{W}")
+    boxes = split_label_geometry(H, W, left, right)
+    R = min(H, max(b.rect[3] for b in boxes) + 1 + SPLIT_LABEL_MARGIN)
+    lut = np.empty((258, R, W), np.uint8)                       # lut[v, y, x]: what the drawing makes of byte v
+    canvas = np.empty((R, W, 3), np.uint8)
+    for k in range(86):
+        canvas[:] = np.minimum(np.arange(3 * k, 3 * k + 3), 255).astype(np.uint8)
+        draw_label_boxes(canvas, boxes)
+        lut[3 * k:3 * k + 3] = canvas.transpose(2, 0, 1)
+    lut = lut[:256]
+    for v in (0, 1, 127, 128, 254, 255):                        # grey canvases: the channels must agree with the table
+        canvas[:] = v
+        draw_label_boxes(canvas, boxes)
+        if not (np.array_equal(canvas[..., 0], canvas[..., 1]) and np.array_equal(canvas[..., 0], canvas[..., 2])
+                and np.array_equal(canvas[..., 0], lut[v])):
+            raise ValueError("split_label_stencil: the label drawing treats the three channels differently "
+                             "(a label colour that is not grey); it has no per-pixel byte table")
+    changed = (lut != np.arange(256, dtype=np.uint8)[:, None, None]).any(axis=0)      # [R, W]
+    if R < H and changed[R - SPLIT_LABEL_MARGIN:].any():
+        raise ValueError("split_label_stencil: the labels reach the margin below their rectangles")
+    rows = np.flatnonzero(changed.any(axis=1))
+    band = int(rows[-1]) + 1 if rows.size else 0
+    rows256 = np.ascontiguousarray(lut[:, changed].T)                                 # [changed pixels, 256]
+    keys, inverse = np.unique(rows256.view(np.dtype((np.void, 256))).ravel(), return_inverse=True)
+    tabs = np.frombuffer(keys.tobytes(), np.uint8).reshape(-1, 256)
+    if tabs.shape[0] + 1 > int(np.iinfo(SPLIT_CLASS_INDEX).max) + 1:
+        raise ValueError(f"split_label_stencil: {tabs.shape[0] + 1} tables do not fit a {np.dtype(SPLIT_CLASS_INDEX)} "
+                         "class index")
+    classes = np.zeros((R, W), SPLIT_CLASS_INDEX)
+    classes[changed] = inverse.reshape(-1) + 1
+    luts = np.concatenate([np.arange(256, dtype=np.uint8)[None], tabs])
+    classes = np.ascontiguousarray(classes[:band])
+    classes.flags.writeable = False
+    luts.flags.writeable = False
+    return SplitLabelStencil(band, classes, luts)

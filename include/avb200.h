@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define AVB_VERSION 130            /* 0.1.3 */
+#define AVB_VERSION 140            /* 0.1.4 */
 
 #define AVB_OK 0
 #define AVB_E_ARG (-1)             /* bad argument (null pointer, non-positive size, unsupported radius ...) */
@@ -365,6 +365,18 @@ AVB_API int64_t avb_jpeg_workspace_bytes(int n, int H, int W);
 AVB_API int avb_jpeg_encode_u8(const uint8_t *in, int n, int H, int W, int64_t in_frame_stride, int64_t in_row_stride,
                                const uint8_t *header_host, int header_len, const uint8_t *qtables_host, uint8_t *out,
                                int64_t out_slot_stride, int64_t *out_lengths_dev, void *workspace_dev, avb_stream_t stream);
+
+/* ---- K9: labelled split-compare compose (csrc/k9_split.cu) ---------------------------------------------------
+ * make_split_frame (reference renderers/video.py:198-245) for n packed 8-bit 3-channel frames of H x W: columns
+ * [0, W/2) of out from left, [W/2, W) from right, column W/2 set to 255 when seam != 0; then, in rows [0, band_rows),
+ * every byte b of pixel (y, x) becomes luts_dev[classes_dev[y * W + x] * 256 + b] (class 0 is the identity table).
+ * The tables are the corner labels of draw_split_labels (animal_vision_b200/tables.py split_label_stencil); every class
+ * index must be below the number of tables.  Strides are in bytes; input frame strides may be 0 (one frame for all),
+ * output frames must not overlap, and out must not overlap either input.  band_rows = 0 takes no tables. */
+AVB_API int avb_split_compose_u8(const uint8_t *left, const uint8_t *right, uint8_t *out, int n, int H, int W,
+                                 int64_t left_frame_stride, int64_t left_row_stride, int64_t right_frame_stride,
+                                 int64_t right_row_stride, int64_t out_frame_stride, int64_t out_row_stride, int seam,
+                                 int band_rows, const uint16_t *classes_dev, const uint8_t *luts_dev, avb_stream_t stream);
 
 #ifdef __cplusplus
 }
