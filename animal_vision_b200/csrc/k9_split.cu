@@ -175,3 +175,76 @@ extern "C" int avb_split_compose_u8(const uint8_t *left, const uint8_t *right, u
     AVB_CUDA_OK(cudaGetLastError());
     return AVB_OK;
 }
+
+// The bytes of a composed split frame that can differ from its input frame, device -> host: rows [0, band_rows) whole,
+// and bytes [3 * (W / 2), 3W) of rows [band_rows, H) (the seam and the right half).  Everything else is the left half of
+// the input outside the label band, so fetching into the host frames that were uploaded turns them into their split
+// frames.  Pitched copies, two per frame, or two in all when both sides stack their frames as whole rows (one 3D copy
+// per piece).  The destination must be page-locked: a pageable one would make the copy synchronous and staged.
+namespace {
+
+// Frames lie `frame_stride / row_stride` whole rows apart, so a 3D copy with that slice height reaches every frame.
+bool stacked(int64_t frame_stride, int64_t row_stride, int H) {
+    return frame_stride % row_stride == 0 && frame_stride / row_stride >= H;
+}
+
+cudaError_t memory_type(const void *p, cudaMemoryType *type) {
+    cudaPointerAttributes at = {};
+    const cudaError_t e = cudaPointerGetAttributes(&at, p);
+    *type = at.type;
+    return e;
+}
+
+}  // namespace
+
+extern "C" int avb_split_fetch_u8(const uint8_t *src, uint8_t *dst_host, int n, int H, int W, int64_t src_frame_stride,
+                                  int64_t src_row_stride, int64_t dst_frame_stride, int64_t dst_row_stride, int band_rows,
+                                  avb_stream_t stream) {
+    AVB_REQUIRE(src && dst_host, "null frame pointer");
+    AVB_REQUIRE(n >= 1 && H >= 1 && W >= 1, "n, H and W must be positive");
+    AVB_REQUIRE(3LL * W <= (1LL << 30), "rows longer than 2^30 bytes");
+    AVB_REQUIRE(src_row_stride >= 3LL * W && dst_row_stride >= 3LL * W, "row strides must be at least 3 * W bytes");
+    AVB_REQUIRE(src_frame_stride >= 0, "negative frame stride");
+    AVB_REQUIRE(n == 1 || dst_frame_stride >= dst_row_stride * (H - 1) + 3LL * W, "destination frames overlap");
+    AVB_REQUIRE(band_rows >= 0 && band_rows <= H, "band_rows must lie in [0, H]");
+    const int64_t src_last = (n - 1) * src_frame_stride + (H - 1) * src_row_stride + 3LL * W - 1;
+    const int64_t dst_last = (n - 1) * dst_frame_stride + (H - 1) * dst_row_stride + 3LL * W - 1;
+    cudaMemoryType type;                      // first and last byte of each side
+    for (const uint8_t *p : {src, src + src_last}) {
+        AVB_CUDA_OK(memory_type(p, &type));
+        AVB_REQUIRE(type == cudaMemoryTypeDevice, "src must be device memory");
+    }
+    for (const uint8_t *p : {(const uint8_t *)dst_host, (const uint8_t *)dst_host + dst_last}) {
+        AVB_CUDA_OK(memory_type(p, &type));
+        AVB_REQUIRE(type == cudaMemoryTypeHost, "dst_host must be page-locked host memory (a pageable destination "
+                                                "makes the copy synchronous and staged)");
+    }
+    const int64_t row = 3LL * W, split = 3LL * (W / 2);
+    struct Piece {
+        int y0, rows;
+        int64_t x0, width;
+    };
+    const Piece pieces[2] = {{0, band_rows, 0, row}, {band_rows, H - band_rows, split, row - split}};
+    const bool one_copy = stacked(src_frame_stride, src_row_stride, H) && stacked(dst_frame_stride, dst_row_stride, H);
+    cudaStream_t st = (cudaStream_t)stream;
+    for (const Piece &p : pieces) {
+        if (p.rows == 0) continue;
+        if (one_copy) {
+            cudaMemcpy3DParms c = {};
+            c.srcPtr = make_cudaPitchedPtr((void *)src, src_row_stride, row, src_frame_stride / src_row_stride);
+            c.dstPtr = make_cudaPitchedPtr(dst_host, dst_row_stride, row, dst_frame_stride / dst_row_stride);
+            c.srcPos = c.dstPos = make_cudaPos(p.x0, p.y0, 0);
+            c.extent = make_cudaExtent(p.width, p.rows, n);
+            c.kind = cudaMemcpyDeviceToHost;
+            AVB_CUDA_OK(cudaMemcpy3DAsync(&c, st));
+        } else {
+            for (int f = 0; f < n; ++f) {
+                const int64_t so = f * src_frame_stride + p.y0 * src_row_stride + p.x0;
+                const int64_t doff = f * dst_frame_stride + p.y0 * dst_row_stride + p.x0;
+                AVB_CUDA_OK(cudaMemcpy2DAsync(dst_host + doff, dst_row_stride, src + so, src_row_stride, p.width, p.rows,
+                                              cudaMemcpyDeviceToHost, st));
+            }
+        }
+    }
+    return AVB_OK;
+}

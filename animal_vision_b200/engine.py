@@ -31,6 +31,11 @@ def get_engine(device=None) -> "Engine":
         return _engines[idx]
 
 
+def split_fetch_bytes(n: int, h: int, w: int, band_rows: int) -> int:
+    """Bytes Engine.split_fetch copies for n frames of h x w: the label band whole, then columns [w // 2, w)."""
+    return n * (band_rows * 3 * w + (h - band_rows) * (3 * w - 3 * (w // 2)))
+
+
 def _fptr(a: np.ndarray):
     return a.ctypes.data_as(C.c_void_p)
 
@@ -234,6 +239,24 @@ class Engine:
             None if cls is None else cls.data_ptr(), None if lut is None else lut.data_ptr(), self.stream_ptr())
         check(rc, "avb_split_compose_u8")
         self.launches += 1
+
+    @_on_device
+    def split_fetch(self, src, dst, band_rows: int) -> int:
+        """avb_split_fetch_u8 on the current stream: copy into the page-locked host frames `dst` the bytes of the composed
+        split frames `src` (CUDA, same shape) that can differ from the input frames -- rows [0, band_rows) and the columns
+        [W // 2, W) of the other rows.  With `dst` holding the frames `src` was composed from, `dst` becomes the split
+        frames.  Returns the bytes copied (split_fetch_bytes)."""
+        n, h, w, sfs, srs = self.check_frames(src, "src")
+        t = self.torch
+        if not (isinstance(dst, t.Tensor) and dst.device.type == "cpu" and dst.dtype == t.uint8
+                and tuple(dst.shape) == (n, h, w, 3) and dst.stride(3) == 1 and dst.stride(2) == 3):
+            raise AvbError("dst: expected a host uint8 tensor of src's shape with packed pixels")
+        if n == 0 or h == 0 or w == 0:
+            return 0
+        rc = self.lib.avb_split_fetch_u8(src.data_ptr(), dst.data_ptr(), n, h, w, sfs, srs, dst.stride(0), dst.stride(1),
+                                         int(band_rows), self.stream_ptr())
+        check(rc, "avb_split_fetch_u8")
+        return split_fetch_bytes(n, h, w, band_rows)
 
     # ------------------------------------------------------------------ NumPy shim staging
     @_on_device

@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define AVB_VERSION 140            /* 0.1.4 */
+#define AVB_VERSION 150            /* 0.1.5 */
 
 #define AVB_OK 0
 #define AVB_E_ARG (-1)             /* bad argument (null pointer, non-positive size, unsupported radius ...) */
@@ -377,6 +377,17 @@ AVB_API int avb_split_compose_u8(const uint8_t *left, const uint8_t *right, uint
                                  int64_t left_frame_stride, int64_t left_row_stride, int64_t right_frame_stride,
                                  int64_t right_row_stride, int64_t out_frame_stride, int64_t out_row_stride, int seam,
                                  int band_rows, const uint16_t *classes_dev, const uint8_t *luts_dev, avb_stream_t stream);
+
+/* The device -> host copy of the bytes of n composed split frames (`src`, device, e.g. avb_split_compose_u8's out) that
+ * can differ from their input frames: rows [0, band_rows) at full width, and bytes [3 * (W / 2), 3W) of rows
+ * [band_rows, H).  Fetched into the page-locked host frames that were uploaded as the compose's left input, it turns
+ * them into their split frames; n * (band_rows * 3W + (H - band_rows) * (3W - 3 * (W / 2))) bytes cross.  Pitched
+ * copies (cudaMemcpy3DAsync / cudaMemcpy2DAsync): two in all when both sides keep frame_stride a multiple of row_stride
+ * and at least H rows, else two per frame.  Strides are in bytes; destination frames must not overlap.  dst_host must be
+ * page-locked host memory and src device memory (cudaPointerGetAttributes of the first and last byte), else AVB_E_ARG. */
+AVB_API int avb_split_fetch_u8(const uint8_t *src, uint8_t *dst_host, int n, int H, int W, int64_t src_frame_stride,
+                               int64_t src_row_stride, int64_t dst_frame_stride, int64_t dst_row_stride, int band_rows,
+                               avb_stream_t stream);
 
 #ifdef __cplusplus
 }
