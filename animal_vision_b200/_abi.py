@@ -16,8 +16,9 @@ from . import _build
 _lock = threading.Lock()
 _lib = None
 
-AVB_VERSION = 150         # include/avb200.h AVB_VERSION
+AVB_VERSION = 160         # include/avb200.h AVB_VERSION
 AVB_JPEG_HEADER_MAX = 1024
+AVB_PNG_HEADER_LEN = 35
 AVB_NORM_DIV255 = 0
 AVB_NORM_AUTO = 1
 AVB_ENC_TABLE_MAX = 2048
@@ -67,6 +68,9 @@ SIGNATURES = {
     "avb_jpeg_bound_bytes": (_i64, [_i, _i]),
     "avb_jpeg_workspace_bytes": (_i64, [_i, _i, _i]),
     "avb_jpeg_encode_u8": (_i, [_p, _i, _i, _i, _i64, _i64, _p, _i, _p, _p, _i64, _p, _p, _p]),
+    "avb_png_bound_bytes": (_i64, [_i, _i]),
+    "avb_png_workspace_bytes": (_i64, [_i, _i, _i]),
+    "avb_png_encode_u8": (_i, [_p, _i, _i, _i, _i64, _i64, _p, _i, _p, _i64, _p, _p, _p]),
     "avb_split_compose_u8": (_i, [_p, _p, _p, _i, _i, _i, _i64, _i64, _i64, _i64, _i64, _i64, _i, _i, _p, _p, _p]),
     "avb_split_fetch_u8": (_i, [_p, _p, _i, _i, _i, _i64, _i64, _i64, _i64, _i, _p]),
 }

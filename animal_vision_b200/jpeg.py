@@ -8,7 +8,8 @@ from typing import List
 import numpy as np
 
 from . import tables
-from ._abi import AvbError, check
+from ._abi import AvbError
+from ._slots import encode_slots
 from .engine import _fptr, get_engine
 
 
@@ -30,27 +31,8 @@ def encode_jpeg(frames, quality: int = 95) -> List[bytes]:
     qt = np.ascontiguousarray(tables.jpeg_quant_tables(int(quality)))
     with torch.cuda.device(eng.device):
         lib = eng.lib
-        slot = int(lib.avb_jpeg_bound_bytes(h, w))
-        need = int(lib.avb_jpeg_workspace_bytes(n, h, w))
-        if slot <= 0 or need <= 0:
-            check(min(slot, need), "avb_jpeg_workspace_bytes")
-        key = ("jpeg", eng.stream_ptr())                    # per stream: encodes on different streams may overlap
-        bufs = eng._cache.get(key)
-        if bufs is None or bufs[0].numel() < need or bufs[1].numel() < n * slot or bufs[2].numel() < n:
-            eng._cache[key] = None
-            bufs = eng._cache[key] = (torch.empty(need, dtype=torch.uint8, device=eng.device),
-                                      torch.empty(n * slot, dtype=torch.uint8, device=eng.device),
-                                      torch.empty(n, dtype=torch.int64, device=eng.device))
-        ws, out, lengths = bufs
-        rc = lib.avb_jpeg_encode_u8(frames.data_ptr(), n, h, w, fs, rs, _fptr(header), int(header.size), _fptr(qt),
-                                    out.data_ptr(), slot, lengths.data_ptr(), ws.data_ptr(), eng.stream_ptr())
-        check(rc, "avb_jpeg_encode_u8")
-        eng.launches += 7
-        lens = lengths[:n].cpu().tolist()                   # waits for the encode
-        offs = np.concatenate([[0], np.cumsum(lens)]).astype(np.int64)
-        host = torch.empty(int(offs[-1]), dtype=torch.uint8).pin_memory()
-        for f in range(n):
-            host[int(offs[f]):int(offs[f + 1])].copy_(out[f * slot:f * slot + lens[f]], non_blocking=True)
-        torch.cuda.current_stream(eng.device).synchronize()
-        buf = host.numpy().tobytes()
-    return [buf[int(offs[f]):int(offs[f + 1])] for f in range(n)]
+        return encode_slots(
+            eng, "jpeg", n, int(lib.avb_jpeg_bound_bytes(h, w)), int(lib.avb_jpeg_workspace_bytes(n, h, w)),
+            lambda ws, out, slot, lengths: lib.avb_jpeg_encode_u8(
+                frames.data_ptr(), n, h, w, fs, rs, _fptr(header), int(header.size), _fptr(qt), out, slot, lengths, ws,
+                eng.stream_ptr()), 7)

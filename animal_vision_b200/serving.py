@@ -11,6 +11,7 @@ data-URI result, same string keys: "human", "cat", "cow", ... as utils.py:145-19
 `FrameBatcher.submit_jpeg` asks for the JPEG file of the species view instead of its pixels.  Where the batch result
 lives decides the encoder: a view left on the device by the default runner is encoded there (K8, `jpeg.encode_jpeg`,
 the bytes of cv2.imencode) and only the compressed bytes come back; a NumPy result is encoded with cv2.imencode.
+`FrameBatcher.submit_png` does the same with PNG (K10, `png.encode_png`), and `process_image_png` wraps it as a data URI.
 
 `FrameBatcher.submit_split_jpeg` asks for the JPEG file of the labelled split-compare frame of the request's input and
 its species view -- what the reference's CLI shows (main.py:41-48 `render_split_compare(img, out)`, with the defaults of
@@ -85,23 +86,28 @@ def _pixels(view, idx: List[int]) -> List[np.ndarray]:
         return [pin[k].numpy() for k in range(len(idx))]
 
 
-def _encode_host(frame: np.ndarray) -> bytes:
+_HOST_EXT = {"jpeg": ".jpg", "png": ".png"}       # encoded request kinds and cv2's extension for each
+
+
+def _encode_host(frame: np.ndarray, fmt: str = "jpeg") -> bytes:
     import cv2
-    ok, enc = cv2.imencode(".jpg", frame)
+    ok, enc = cv2.imencode(_HOST_EXT[fmt], frame)
     if not ok:
         raise ValueError("could not encode the result")
     return enc.tobytes()
 
 
-def _jpegs(view, idx: List[int]) -> List[bytes]:
-    """JPEG files (cv2.imencode's bytes, quality 95) of the frames `idx` of a batch result."""
+def _encoded(view, idx: List[int], fmt: str) -> List[bytes]:
+    """Files of the frames `idx` of a batch result, the bytes cv2.imencode gives with its defaults: JPEG at quality 95
+    (fmt "jpeg") or PNG (fmt "png")."""
     if isinstance(view, np.ndarray):
-        return [_encode_host(view[i]) for i in idx]
+        return [_encode_host(view[i], fmt) for i in idx]
     import torch
     from .jpeg import encode_jpeg
+    from .png import encode_png
     with torch.cuda.device(view.device):
         sel = view if len(idx) == view.shape[0] else view[torch.tensor(idx, device=view.device)]
-        return encode_jpeg(sel, 95)
+        return encode_jpeg(sel, 95) if fmt == "jpeg" else encode_png(sel)
 
 
 def _split_host(frame: np.ndarray, view: np.ndarray, labels: Tuple[str, str], seam: bool) -> bytes:
@@ -163,6 +169,10 @@ class FrameBatcher:
         """Future of the JPEG file (bytes) of the species view, the bytes cv2.imencode(".jpg", view) gives."""
         return self._submit(frame, animal, "jpeg")
 
+    def submit_png(self, frame: np.ndarray, animal: str) -> Future:
+        """Future of the PNG file (bytes) of the species view, the bytes cv2.imencode(".png", view) gives."""
+        return self._submit(frame, animal, "png")
+
     def submit_split_jpeg(self, frame: np.ndarray, animal: str, labels: Tuple[str, str] = ("Original", "Transformed"),
                           draw_seam: bool = True) -> Future:
         """Future of the JPEG file (bytes) of the split-compare frame of `frame` and its species view: left half of
@@ -177,7 +187,7 @@ class FrameBatcher:
         return self._submit(frame, animal, kind)
 
     def _submit(self, frame: np.ndarray, animal: str, kind) -> Future:
-        """kind: None (pixels), "jpeg", or ("split", labels, seam)."""
+        """kind: None (pixels), "jpeg", "png", or ("split", labels, seam)."""
         fut: Future = Future()
         if animal != "human" and animal not in SERVER_KEYS:
             fut.set_exception(KeyError(f"no case implemented for {animal!r}"))             # utils.py:192-193 prints and fails later
@@ -190,7 +200,7 @@ class FrameBatcher:
                 fut.set_result(frame)
                 return fut
             try:
-                fut.set_result(_encode_host(frame) if kind == "jpeg" else _split_host(frame, frame, kind[1], kind[2]))
+                fut.set_result(_encode_host(frame, kind) if kind in _HOST_EXT else _split_host(frame, frame, kind[1], kind[2]))
             except Exception as e:          # noqa: BLE001
                 fut.set_exception(e)
             return fut
@@ -234,7 +244,7 @@ class FrameBatcher:
         batch = np.stack([f for f, _, _ in part])
         splits: "OrderedDict[tuple, List[int]]" = OrderedDict()
         for i, (_, _, kind) in enumerate(part):
-            if kind is not None and kind != "jpeg":
+            if kind is not None and kind not in _HOST_EXT:
                 splits.setdefault(kind[1:], []).append(i)
         upload_and_run = getattr(self._run, "upload_and_run", None)
         if splits and upload_and_run is not None:
@@ -243,10 +253,11 @@ class FrameBatcher:
             dev_in, out = None, self._run(animal, batch)
         self.batches.append((animal, len(part)))
         pix = [i for i, (_, _, kind) in enumerate(part) if kind is None]
-        jpg = [i for i, (_, _, kind) in enumerate(part) if kind == "jpeg"]
         res = dict(zip(pix, _pixels(out, pix))) if pix else {}
-        if jpg:
-            res.update(zip(jpg, _jpegs(out, jpg)))
+        for fmt in _HOST_EXT:
+            idx = [i for i, (_, _, kind) in enumerate(part) if kind == fmt]
+            if idx:
+                res.update(zip(idx, _encoded(out, idx, fmt)))
         for (labels, seam), idx in splits.items():
             res.update(zip(idx, _split_jpegs(batch, dev_in, out, idx, labels, seam)))
         for i, (_, fut, _) in enumerate(part):
@@ -286,6 +297,17 @@ def process_image(imagedata: bytes, animal: str, batcher: Optional[FrameBatcher]
         raise ValueError("could not decode the image")
     enc = (batcher or default_batcher()).submit_jpeg(img, animal).result()
     return "data:image/jpeg;base64," + base64.b64encode(enc).decode("utf-8")
+
+
+def process_image_png(imagedata: bytes, animal: str, batcher: Optional[FrameBatcher] = None) -> str:
+    """`process_image` with a lossless result: image bytes in, data URI of the PNG of the species view out
+    (`FrameBatcher.submit_png`, the bytes of cv2.imencode(".png", view))."""
+    import cv2
+    img = cv2.imdecode(np.frombuffer(imagedata, np.uint8), cv2.IMREAD_COLOR)
+    if img is None:
+        raise ValueError("could not decode the image")
+    enc = (batcher or default_batcher()).submit_png(img, animal).result()
+    return "data:image/png;base64," + base64.b64encode(enc).decode("utf-8")
 
 
 def process_split_image(imagedata: bytes, animal: str, labels: Tuple[str, str] = ("Original", "Transformed"),

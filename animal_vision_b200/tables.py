@@ -535,6 +535,36 @@ def jpeg_header(H: int, W: int, quality: int) -> bytes:
     return out + _jpeg_segment(0xDA, bytes([3, 1, 0x00, 2, 0x11, 3, 0x11, 0, 63, 0]))
 
 
+# ----------------------------------------------------------------------------- PNG (K10)
+PNG_SIGNATURE = b"\x89PNG\r\n\x1a\n"
+
+
+def _png_chunk(kind: bytes, payload: bytes) -> bytes:
+    import zlib
+    return len(payload).to_bytes(4, "big") + kind + payload + zlib.crc32(kind + payload).to_bytes(4, "big")
+
+
+def png_header(H: int, W: int) -> bytes:
+    """Every byte of cv2.imencode(".png") that depends only on the frame size: the signature, the IHDR chunk (depth 8,
+    colour type 2, no interlace) and the two zlib header bytes that open the first IDAT payload.  zlib writes 78 01
+    (32K window, level 1); libpng's optimize_cmf then lowers the window to the smallest that holds the image data
+    when that data (H rows of 3W + 1 filtered bytes) is at most 16384 bytes."""
+    H, W = int(H), int(W)
+    if not (1 <= H <= 65535 and 1 <= W <= 65535):
+        raise ValueError(f"PNG frame size must lie in [1, 65535]^2, got {H}x{W}")
+    size = H * (3 * W + 1)
+    cmf, flg = 0x78, 0x01
+    if size <= 16384:
+        cinfo, half = 7, 1 << 14
+        while cinfo > 0 and size <= half:     # optimize_cmf: halve the window while the data still fits in half
+            half >>= 1
+            cinfo -= 1
+        cmf = (cinfo << 4) | 8
+        flg = 0x1F - (cmf << 8) % 0x1F
+    ihdr = W.to_bytes(4, "big") + H.to_bytes(4, "big") + bytes([8, 2, 0, 0, 0])
+    return PNG_SIGNATURE + _png_chunk(b"IHDR", ihdr) + bytes([cmf, flg])
+
+
 # ----------------------------------------------------------------------------- split-compare labels (K9)
 SPLIT_LABEL_MARGIN = 16            # rows drawn below the lowest label rectangle; they must come out untouched
 SPLIT_CLASS_INDEX = np.uint16      # class map dtype (K9 reads uint16)

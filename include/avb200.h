@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define AVB_VERSION 150            /* 0.1.5 */
+#define AVB_VERSION 160            /* 0.1.6 */
 
 #define AVB_OK 0
 #define AVB_E_ARG (-1)             /* bad argument (null pointer, non-positive size, unsupported radius ...) */
@@ -365,6 +365,24 @@ AVB_API int64_t avb_jpeg_workspace_bytes(int n, int H, int W);
 AVB_API int avb_jpeg_encode_u8(const uint8_t *in, int n, int H, int W, int64_t in_frame_stride, int64_t in_row_stride,
                                const uint8_t *header_host, int header_len, const uint8_t *qtables_host, uint8_t *out,
                                int64_t out_slot_stride, int64_t *out_lengths_dev, void *workspace_dev, avb_stream_t stream);
+
+/* ---- K10: PNG encode (csrc/k10_png.cu) -----------------------------------------------------------------
+ * The bytes of cv2.imencode(".png", frame) with OpenCV's defaults (libpng 1.6 + zlib: filter Sub, deflate level 1,
+ * strategy Z_RLE, memLevel 8, IDAT payloads of 8192 bytes) for n packed BGR uint8 frames of H x W, any byte strides.
+ * Stream-ordered on `stream`, never synchronises; everything after the frames (filter, parse, trees, emission,
+ * Adler-32, framing, CRC-32) runs on the device.
+ *   header_host     the signature, the IHDR chunk and the zlib CMF / FLG bytes (animal_vision_b200/tables.py
+ *                   png_header), exactly AVB_PNG_HEADER_LEN bytes
+ *   out             n slots of out_slot_stride >= avb_png_bound_bytes(H, W) bytes: frame f's file is written from
+ *                   out + f * out_slot_stride, its length to out_lengths_dev[f] (device int64)
+ *   workspace_dev   avb_png_workspace_bytes(n, H, W) bytes, 16-byte aligned
+ * H and W lie in [1, 65535]. */
+#define AVB_PNG_HEADER_LEN 35
+AVB_API int64_t avb_png_bound_bytes(int H, int W);
+AVB_API int64_t avb_png_workspace_bytes(int n, int H, int W);
+AVB_API int avb_png_encode_u8(const uint8_t *in, int n, int H, int W, int64_t in_frame_stride, int64_t in_row_stride,
+                              const uint8_t *header_host, int header_len, uint8_t *out, int64_t out_slot_stride,
+                              int64_t *out_lengths_dev, void *workspace_dev, avb_stream_t stream);
 
 /* ---- K9: labelled split-compare compose (csrc/k9_split.cu) ---------------------------------------------------
  * make_split_frame (reference renderers/video.py:198-245) for n packed 8-bit 3-channel frames of H x W: columns
