@@ -613,11 +613,11 @@ gauss_stream_kernel(const __grid_constant__ GaussCommon p, const __grid_constant
 // tensor pipe would become the bound of an otherwise CUDA-core kernel (measured mma.sync rate on B200:
 // 555 TFLOP/s, tools/micro/hmma_rate.cu; this kernel needs 0.13 TFLOP per 20 4K frames at 29 taps).
 //
-//   produce   as above (TMA-staged packed rows, LUT decode, 2x3 matrix) into a PLANAR F16 tile S[plane][part]
-//             [16 rows][x halo]; every value is split x = hi + lo (two f16) so the operand keeps 22 mantissa bits
+//   produce   as above (TMA-staged packed rows, LUT decode, 2x3 matrix) into a PLANAR F16 tile S[plane]
+//             [16 rows][x halo]
 //   H pass    D[16 rows x 8 cols] += S[16 rows x 16s..16s+15] * T_s,  T_s[k][n] = w[16s + k - n]: the Toeplitz
 //             fragments are pixel independent and live in registers for the whole kernel (6 words)
-//   ring      the H results (hi + lo again) of the last (D+1) blocks of 16 rows, D = ceil(2R/16)
+//   ring      the H results (f16 again) of the last (D+1) blocks of 16 rows, D = ceil(2R/16)
 //   V pass    D[16 out rows x 8 cols] += T'_s[16 x 16] * ring[block ob+s][16 rows x 8 cols] (ldmatrix.trans)
 //   encode    expand the two planes, table encode, packed bytes staged in shared memory, 128-bit stores.
 // Taps are rounded to f16 on the host with the rounding error diffused so that they still sum to 1 (flat
@@ -646,17 +646,10 @@ __device__ __forceinline__ uint32_t pack_h2(float a, float b) {
     const __half2 h = __floats2half2_rn(a, b);
     return *reinterpret_cast<const uint32_t *>(&h);
 }
-// x = hi + lo, both f16 (lo carries the rounding error of hi)
-__device__ __forceinline__ void split_h2(float a, float b, uint32_t &hi, uint32_t &lo) {
-    const __half2 h = __floats2half2_rn(a, b);
-    const float2 f = __half22float2(h);
-    hi = *reinterpret_cast<const uint32_t *>(&h);
-    lo = pack_h2(a - f.x, b - f.y);
-}
 
 template <int KSH>
 struct MmaCfg {
-    static constexpr int SP = 120 + 16 * KSH;     // S pitch in halves: 272 / 304 / 336 B = 17 / 19 / 21 x 16 B
+    static constexpr int SP = 120 + 16 * KSH;     // S pitch in halves: 304 / 336 B = 19 / 21 x 16 B
 };
 
 struct MmaGeom {
@@ -666,20 +659,19 @@ struct MmaGeom {
 };
 
 #ifndef M_MINB_SINGLE
-#define M_MINB_SINGLE 3     // single-f16 operands: 71 registers and ~72 KB of shared memory per CTA, three CTAs per SM
+#define M_MINB_SINGLE 3     // 71 registers and ~72 KB of shared memory per CTA, three CTAs per SM
 #endif
-template <int KSH, int D, bool SPLIT>
-__global__ void __launch_bounds__(M_THREADS, SPLIT ? 2 : M_MINB_SINGLE)
+template <int KSH, int D>
+__global__ void __launch_bounds__(M_THREADS, M_MINB_SINGLE)
 gauss_mma_kernel(const __grid_constant__ GaussCommon p, const __grid_constant__ DogProducer::Params pp, const __grid_constant__ MmaGeom geo) {
     constexpr int SP = MmaCfg<KSH>::SP;
-    constexpr int NP = SPLIT ? 2 : 1;             // operand parts (hi, lo)
     constexpr int KSV = D + 1;                    // k-steps of the V pass = ring depth in blocks
-    constexpr int S_PLANE = M_RB * SP;            // halves per (plane, part)
+    constexpr int S_PLANE = M_RB * SP;            // halves per plane
     constexpr int H_PLANE = KSV * M_RB * M_HP;
     extern __shared__ __align__(128) uint8_t smem_raw[];
-    __half *S = reinterpret_cast<__half *>(smem_raw);                     // [2][NP][16][SP]
-    __half *HR = S + 2 * NP * S_PLANE;                                     // [2][NP][KSV*16][M_HP]
-    uint8_t *stage = reinterpret_cast<uint8_t *>(HR + 2 * NP * H_PLANE);   // [16][400] encoded bytes of an output block
+    __half *S = reinterpret_cast<__half *>(smem_raw);                     // [2][16][SP]
+    __half *HR = S + 2 * S_PLANE;                                          // [2][KSV*16][M_HP]
+    uint8_t *stage = reinterpret_cast<uint8_t *>(HR + 2 * H_PLANE);        // [16][400] encoded bytes of an output block
     float *lut4 = reinterpret_cast<float *>(stage + M_RB * M_STAGE_PITCH); // [256][M_LUT_COPIES]
     uint32_t *enc_s = reinterpret_cast<uint32_t *>(lut4 + 256 * M_LUT_COPIES);
     uint8_t *rawt0 = reinterpret_cast<uint8_t *>(enc_s + G_ENC_SMEM);      // [2][16][M_RAW_PITCH] packed input rows (TMA double buffer)
@@ -700,7 +692,7 @@ gauss_mma_kernel(const __grid_constant__ GaussCommon p, const __grid_constant__ 
     for (int i = tid; i < 256 * M_LUT_COPIES; i += M_THREADS) lut4[i] = __ldg(pp.lut + (i / M_LUT_COPIES));
     copy_to_smem(enc_s, p.enc, min(G_ENC_SMEM, ENC_HEADER + (int)__ldg(p.enc + 2)));
     // the pad columns of S only ever meet zero Toeplitz entries, but they must hold finite numbers
-    for (int i = tid; i < 2 * NP * S_PLANE / 2; i += M_THREADS) reinterpret_cast<uint32_t *>(S)[i] = 0u;
+    for (int i = tid; i < S_PLANE; i += M_THREADS) reinterpret_cast<uint32_t *>(S)[i] = 0u;
     if (tid == 0) {
         gauss_mbar_init(&rbar[0], M_RB);
         gauss_mbar_init(&rbar[1], M_RB);
@@ -764,16 +756,11 @@ gauss_mma_kernel(const __grid_constant__ GaussCommon p, const __grid_constant__ 
     const int l_row = (lane & 7) + 8 * ((lane >> 3) & 1), l_hi = lane >> 4;
 
     auto store_px = [&](int r, int i, float o0, float o1) {
-        const __half h0 = __float2half_rn(o0), h1 = __float2half_rn(o1);
-        S[r * SP + i] = h0;
-        S[NP * S_PLANE + r * SP + i] = h1;
-        if (SPLIT) {
-            S[S_PLANE + r * SP + i] = __float2half_rn(o0 - __half2float(h0));
-            S[NP * S_PLANE + S_PLANE + r * SP + i] = __float2half_rn(o1 - __half2float(h1));
-        }
+        S[r * SP + i] = __float2half_rn(o0);
+        S[S_PLANE + r * SP + i] = __float2half_rn(o1);
     };
 
-    // ---- produce block ib: 16 rows x IN_W columns of the two planes as f16 (hi, lo)
+    // ---- produce block ib: 16 rows x IN_W columns of the two planes as f16
     auto produce = [&](int ib) {
         const int yb = y_start - R + ib * M_RB;
         if (staged) {
@@ -794,17 +781,9 @@ gauss_mma_kernel(const __grid_constant__ GaussCommon p, const __grid_constant__ 
                     px2(__byte_perm(w0, 0, 0x4443), __byte_perm(w1, 0, 0x4440), __byte_perm(w1, 0, 0x4441), a[1], b[1]);
                     px2(__byte_perm(w1, 0, 0x4442), __byte_perm(w1, 0, 0x4443), __byte_perm(w2, 0, 0x4440), a[2], b[2]);
                     px2(__byte_perm(w2, 0, 0x4441), __byte_perm(w2, 0, 0x4442), __byte_perm(w2, 0, 0x4443), a[3], b[3]);
-                    __half *d0 = S + r * SP + 4 * gq, *d1 = d0 + NP * S_PLANE;
-                    if (SPLIT) {
-                        uint2 hi, lo;
-                        split_h2(a[0], a[1], hi.x, lo.x); split_h2(a[2], a[3], hi.y, lo.y);
-                        *reinterpret_cast<uint2 *>(d0) = hi; *reinterpret_cast<uint2 *>(d0 + S_PLANE) = lo;
-                        split_h2(b[0], b[1], hi.x, lo.x); split_h2(b[2], b[3], hi.y, lo.y);
-                        *reinterpret_cast<uint2 *>(d1) = hi; *reinterpret_cast<uint2 *>(d1 + S_PLANE) = lo;
-                    } else {
-                        *reinterpret_cast<uint2 *>(d0) = make_uint2(pack_h2(a[0], a[1]), pack_h2(a[2], a[3]));
-                        *reinterpret_cast<uint2 *>(d1) = make_uint2(pack_h2(b[0], b[1]), pack_h2(b[2], b[3]));
-                    }
+                    __half *d0 = S + r * SP + 4 * gq, *d1 = d0 + S_PLANE;
+                    *reinterpret_cast<uint2 *>(d0) = make_uint2(pack_h2(a[0], a[1]), pack_h2(a[2], a[3]));
+                    *reinterpret_cast<uint2 *>(d1) = make_uint2(pack_h2(b[0], b[1]), pack_h2(b[2], b[3]));
                 }
             } else {
                 for (int idx = tid; idx < M_RB * IN_W; idx += M_THREADS) {
@@ -841,41 +820,30 @@ gauss_mma_kernel(const __grid_constant__ GaussCommon p, const __grid_constant__ 
             for (int e = 0; e < 2; ++e)
 #pragma unroll
                 for (int c = 0; c < 4; ++c) acc[e][c] = 0.f;
+            // half-fragments (16 rows x 8 columns) at columns 16 warp + 8 h, h = 0 .. 2 KSH
+            uint32_t hf[2 * KSH + 1][2];
+            const uint32_t base = S_sh + 2u * (uint32_t)(pl * S_PLANE + l_row * SP + 16 * warp);
 #pragma unroll
-            for (int part = 0; part < NP; ++part) {
-                // half-fragments (16 rows x 8 columns) at columns 16 warp + 8 h, h = 0 .. 2 KSH
-                uint32_t hf[2 * KSH + 1][2];
-                const uint32_t base = S_sh + 2u * (uint32_t)((pl * NP + part) * S_PLANE + l_row * SP + 16 * warp);
-#pragma unroll
-                for (int q = 0; q < KSH; ++q) {
-                    uint32_t r4[4];
-                    ldsm_x4(r4, base + 2u * (uint32_t)(16 * q + 8 * l_hi));
-                    hf[2 * q][0] = r4[0]; hf[2 * q][1] = r4[1]; hf[2 * q + 1][0] = r4[2]; hf[2 * q + 1][1] = r4[3];
-                }
-                {
-                    uint32_t r2[2];
-                    ldsm_x2(r2, base + 2u * (uint32_t)(16 * KSH));
-                    hf[2 * KSH][0] = r2[0]; hf[2 * KSH][1] = r2[1];
-                }
-#pragma unroll
-                for (int e = 0; e < 2; ++e)
-#pragma unroll
-                    for (int s = 0; s < KSH; ++s)
-                        mma16816(acc[e], hf[2 * s + e][0], hf[2 * s + e][1], hf[2 * s + e + 1][0], hf[2 * s + e + 1][1], th[2 * s], th[2 * s + 1]);
+            for (int q = 0; q < KSH; ++q) {
+                uint32_t r4[4];
+                ldsm_x4(r4, base + 2u * (uint32_t)(16 * q + 8 * l_hi));
+                hf[2 * q][0] = r4[0]; hf[2 * q][1] = r4[1]; hf[2 * q + 1][0] = r4[2]; hf[2 * q + 1][1] = r4[3];
+            }
+            {
+                uint32_t r2[2];
+                ldsm_x2(r2, base + 2u * (uint32_t)(16 * KSH));
+                hf[2 * KSH][0] = r2[0]; hf[2 * KSH][1] = r2[1];
             }
 #pragma unroll
+            for (int e = 0; e < 2; ++e)
+#pragma unroll
+                for (int s = 0; s < KSH; ++s)
+                    mma16816(acc[e], hf[2 * s + e][0], hf[2 * s + e][1], hf[2 * s + e + 1][0], hf[2 * s + e + 1][1], th[2 * s], th[2 * s + 1]);
+#pragma unroll
             for (int e = 0; e < 2; ++e) {
-                __half *d = HR + (pl * NP) * H_PLANE + (slot * M_RB + g) * M_HP + 8 * (2 * warp + e) + 2 * t;
-                if (SPLIT) {
-                    uint32_t hi, lo;
-                    split_h2(acc[e][0], acc[e][1], hi, lo);
-                    *reinterpret_cast<uint32_t *>(d) = hi; *reinterpret_cast<uint32_t *>(d + H_PLANE) = lo;
-                    split_h2(acc[e][2], acc[e][3], hi, lo);
-                    *reinterpret_cast<uint32_t *>(d + 8 * M_HP) = hi; *reinterpret_cast<uint32_t *>(d + 8 * M_HP + H_PLANE) = lo;
-                } else {
-                    *reinterpret_cast<uint32_t *>(d) = pack_h2(acc[e][0], acc[e][1]);
-                    *reinterpret_cast<uint32_t *>(d + 8 * M_HP) = pack_h2(acc[e][2], acc[e][3]);
-                }
+                __half *d = HR + pl * H_PLANE + (slot * M_RB + g) * M_HP + 8 * (2 * warp + e) + 2 * t;
+                *reinterpret_cast<uint32_t *>(d) = pack_h2(acc[e][0], acc[e][1]);
+                *reinterpret_cast<uint32_t *>(d + 8 * M_HP) = pack_h2(acc[e][2], acc[e][3]);
             }
         }
     };
@@ -890,16 +858,13 @@ gauss_mma_kernel(const __grid_constant__ GaussCommon p, const __grid_constant__ 
 #pragma unroll
                 for (int c = 0; c < 4; ++c) out[pl][e][c] = 0.f;
 #pragma unroll
-            for (int part = 0; part < NP; ++part) {
-#pragma unroll
-                for (int s = 0; s < KSV; ++s) {
-                    const int slot = (ob + s) % KSV;
-                    uint32_t b4[4];
-                    ldsm_x4_trans(b4, HR_sh + 2u * (uint32_t)((pl * NP + part) * H_PLANE + (slot * M_RB + l_row) * M_HP + 8 * (2 * warp + l_hi)));
-                    const uint32_t a1 = s > 0 ? tv[2 * s - 1] : 0u;
-                    mma16816(out[pl][0], tv[2 * s], a1, tv[2 * s + 1], tv[2 * s], b4[0], b4[1]);
-                    mma16816(out[pl][1], tv[2 * s], a1, tv[2 * s + 1], tv[2 * s], b4[2], b4[3]);
-                }
+            for (int s = 0; s < KSV; ++s) {
+                const int slot = (ob + s) % KSV;
+                uint32_t b4[4];
+                ldsm_x4_trans(b4, HR_sh + 2u * (uint32_t)(pl * H_PLANE + (slot * M_RB + l_row) * M_HP + 8 * (2 * warp + l_hi)));
+                const uint32_t a1 = s > 0 ? tv[2 * s - 1] : 0u;
+                mma16816(out[pl][0], tv[2 * s], a1, tv[2 * s + 1], tv[2 * s], b4[0], b4[1]);
+                mma16816(out[pl][1], tv[2 * s], a1, tv[2 * s + 1], tv[2 * s], b4[2], b4[3]);
             }
         }
         // fragment: (row g / g+8, columns 2t, 2t+1) of column tiles 2 warp, 2 warp + 1
@@ -1070,24 +1035,13 @@ static void quantize_taps_f16(float *taps, int ksize) {
     for (int i = 0; i < ksize; ++i) taps[i] = (float)q[i];
 }
 
-// AVB_GAUSS_MMA: 0 = CUDA-core kernel (gauss_stream_kernel) always; 1 = tensor-core kernel with hi+lo f16 operands from
-// radius 8 up (the round-2 default until the 1-LSB budget was spent: 4-9e-4 of the bytes differ from the reference);
-// 2 = single f16 operands from radius 8 up; 3 / 4 = modes 1 / 2 at every radius (tests);
-// 5 (DEFAULT) = single f16 operands from radius 5 up.  Single f16: ~0.05 LSB of systematic rounding, <= 1 LSB with 0.3-1.4 % of
-// the bytes differing (a flat region may flip by 1 LSB as a whole); the kernel then needs 71 registers and ~72 KB of shared
-// memory and runs three CTAs per SM -- measured, 20 4K frames, ms: Dog (29 taps) 1.13 -> 0.85, Raccoon (17) 0.99 -> 0.77,
-// Bear / Elephant (15) 1.03 -> 0.77, Wolf (13) / Fox / Lion (11) 0.91 -> 0.77 (the last three from the CUDA-core kernel).
+// A rank-2 matrix with radius 5..16 takes the tensor-core kernel.  Its single f16 operands cost ~0.05 LSB of systematic
+// rounding: <= 1 LSB, with 0.3-1.4 % of the bytes differing (a flat region may flip by 1 LSB as a whole).  Measured, 20 4K
+// frames, ms, against hi+lo f16 operands (Dog, Raccoon) or the CUDA-core kernel (the others): Dog (29 taps) 1.13 -> 0.85,
+// Raccoon (17) 0.99 -> 0.77, Bear / Elephant (15) 1.03 -> 0.77, Wolf (13) / Fox / Lion (11) 0.91 -> 0.77.
 // Squirrel (7 taps) would gain too (0.82 -> 0.75) but stays on the exact CUDA-core kernel: its narrow blur leaves the plateaus
 // of a checkerboard flat, and 8.6 % of that parity frame's bytes flip together (the 2 % gate of tests/test_gpu_mammals.py).
-// Read once per process.
-constexpr int G_MMA_MIN_RADIUS = 8, G_MMA_MIN_RADIUS_SINGLE = 5;
-static int gauss_mma_mode() {
-    static const int mode = [] {
-        const char *e = std::getenv("AVB_GAUSS_MMA");
-        return e ? std::atoi(e) : 5;
-    }();
-    return mode;
-}
+constexpr int G_MMA_MIN_RADIUS = 5;
 
 static int pick_seg_h_mma(int n, int H, int W, int d_blocks, int ctas_per_sm) {
     const long strips = (long)((W + G_TW - 1) / G_TW) * n;
@@ -1111,12 +1065,11 @@ static int pick_seg_h_mma(int n, int H, int W, int d_blocks, int ctas_per_sm) {
     return (seg_h + M_RB - 1) / M_RB * M_RB;
 }
 
-template <int KSH, int D, bool SPLIT>
+template <int KSH, int D>
 static int launch_gauss_mma(const GaussCommon &gc, const DogProducer::Params &pp, const MmaGeom &geo, cudaStream_t st) {
-    constexpr int NP = SPLIT ? 2 : 1;
-    const size_t smem = (size_t)2 * NP * M_RB * MmaCfg<KSH>::SP * 2 + (size_t)2 * NP * (D + 1) * M_RB * M_HP * 2 +
+    const size_t smem = (size_t)2 * M_RB * MmaCfg<KSH>::SP * 2 + (size_t)2 * (D + 1) * M_RB * M_HP * 2 +
                         (size_t)M_RB * M_STAGE_PITCH + (size_t)(256 * M_LUT_COPIES + G_ENC_SMEM) * 4 + 2 * (size_t)M_RB * M_RAW_PITCH;
-    auto kern = gauss_mma_kernel<KSH, D, SPLIT>;
+    auto kern = gauss_mma_kernel<KSH, D>;
     AVB_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     dim3 grid((gc.io.W + G_TW - 1) / G_TW, (gc.io.H + gc.seg_h - 1) / gc.seg_h, gc.io.n);
     AVB_TIMED(gc.fixup ? DogProducer::fixup_name() : DogProducer::name(), st);
@@ -1125,7 +1078,6 @@ static int launch_gauss_mma(const GaussCommon &gc, const DogProducer::Params &pp
     return AVB_OK;
 }
 
-template <bool SPLIT>
 static int dispatch_gauss_mma(int radius, GaussCommon gc, const DogProducer::Params &q, cudaStream_t st) {
     const int d = radius <= 8 ? 1 : 2;
     MmaGeom geo{};
@@ -1136,12 +1088,11 @@ static int dispatch_gauss_mma(int radius, GaussCommon gc, const DogProducer::Par
     for (int idx = 0; idx < M_RB * geo.groups; ++idx)                        // the multiply-shift division is exact on its range
         if ((int)(((uint32_t)idx * geo.div_groups) >> 16) != idx / geo.groups) { set_error("internal: group divider"); return AVB_E_UNSUPPORTED; }
     gc.radius = radius;
-    gc.seg_h = pick_seg_h_mma(gc.io.n, gc.io.H, gc.io.W, d, SPLIT ? 2 : M_MINB_SINGLE);
+    gc.seg_h = pick_seg_h_mma(gc.io.n, gc.io.H, gc.io.W, d, M_MINB_SINGLE);
     quantize_taps_f16(gc.taps, 2 * radius + 1);
-    if (radius <= 4) return launch_gauss_mma<1, 1, SPLIT>(gc, q, geo, st);
-    if (radius <= 8) return launch_gauss_mma<2, 1, SPLIT>(gc, q, geo, st);
-    if (radius <= 12) return launch_gauss_mma<2, 2, SPLIT>(gc, q, geo, st);
-    return launch_gauss_mma<3, 2, SPLIT>(gc, q, geo, st);
+    if (radius <= 8) return launch_gauss_mma<2, 1>(gc, q, geo, st);
+    if (radius <= 12) return launch_gauss_mma<2, 2>(gc, q, geo, st);
+    return launch_gauss_mma<3, 2>(gc, q, geo, st);
 }
 
 template <class Prod>
@@ -1158,17 +1109,14 @@ static int dispatch_gauss(int radius, GaussCommon &gc, typename Prod::Params &pp
         for (int i = 0; i < 6; ++i) q.M.m[i] = Q[i];
         q.M.m[6] = q.M.m[7] = q.M.m[8] = 0.f;
     }
-    if constexpr (std::is_same<Prod, DogProducer>::value) {
-        // measured (20 4K frames, ms, CUDA cores -> tensor cores hi+lo): 29 taps 1.45 -> 1.14, 17 taps 1.09 -> 1.00,
-        // 15 taps 1.04 -> 1.01, 7 taps 0.83 -> 0.97: below ~17 taps the FMAs saved do not pay for the f16 splitting
-        const int mode = gauss_mma_mode();
-        const int min_radius = mode == 5 ? G_MMA_MIN_RADIUS_SINGLE : (mode >= 3 ? 1 : G_MMA_MIN_RADIUS);   // modes 3 / 4: every radius (tests)
-        if (two && radius >= min_radius && radius <= 16 && mode != 0)
-            return (mode == 2 || mode == 4 || mode == 5) ? dispatch_gauss_mma<false>(radius, gc, q, st)
-                                                         : dispatch_gauss_mma<true>(radius, gc, q, st);
-    }
+    constexpr bool dog = std::is_same<Prod, DogProducer>::value;
+    if constexpr (dog)
+        if (two && radius >= G_MMA_MIN_RADIUS && radius <= 16) return dispatch_gauss_mma(radius, gc, q, st);
+    // a rank-2 Dog matrix from G_MMA_MIN_RADIUS up never gets here: no two-plane instantiation for it
     switch (radius) {
-#define AVB_CASE(RR) case RR: return two ? launch_gauss<RR, Prod, 2>(gc, q, st) : launch_gauss<RR, Prod, 3>(gc, q, st);
+#define AVB_CASE(RR) case RR: \
+        if constexpr (!(dog && RR >= G_MMA_MIN_RADIUS)) if (two) return launch_gauss<RR, Prod, 2>(gc, q, st); \
+        return launch_gauss<RR, Prod, 3>(gc, q, st);
         AVB_CASE(1) AVB_CASE(2) AVB_CASE(3) AVB_CASE(4) AVB_CASE(5) AVB_CASE(6) AVB_CASE(7) AVB_CASE(8)
         AVB_CASE(9) AVB_CASE(10) AVB_CASE(11) AVB_CASE(12) AVB_CASE(13) AVB_CASE(14) AVB_CASE(15) AVB_CASE(16)
 #undef AVB_CASE

@@ -93,7 +93,6 @@ struct UvParams {
     float mix_alpha;             // MAP_MIXED
     float *dbg_catches;          // optional [n][H][W][3] raw catches (test hook), else nullptr
     int aligned_in, aligned_out; // rows / frames 4-byte aligned -> 32-bit pixel-group accesses
-    int no_plane_map;            // AVB_UV_NO_PLANE_MAP=1: always take the second walk (A/B measurements)
     int strips_x, strips_y;
 };
 
@@ -296,13 +295,9 @@ __device__ __forceinline__ void strip_of(const UvParams &p, int task, int &xs, i
 // sqrt on the SFU (rsq + multiply, ~1 ulp): the opponent radius only feeds a percentile that is
 // computed from the very same values and a saturation ratio, both insensitive at the 1e-7 level.
 __device__ __forceinline__ float sqrt_sfu(float x) {
-#ifdef UV_SQRT_RN
-    return __fsqrt_rn(x);
-#else
     float r;
     asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
     return r;
-#endif
 }
 
 // atan2 without branches: octant reduction + the degree-17 odd minimax polynomial of Abramowitz &
@@ -495,7 +490,7 @@ __global__ void uv_prep_kernel(const __grid_constant__ UvParams p) {
 // the adapted, blurred catches themselves for the others -- when a lane's four pixels are one aligned float4 per plane and
 // one aligned 12-byte group of the output (any other geometry, and the matrix mapper, take the second walk, uv_map_kernel).
 __host__ __device__ __forceinline__ bool map_from_planes(const UvParams &p) {
-    return p.n_req > 0 && (p.io.W & 3) == 0 && p.aligned_out != 0 && !p.no_plane_map;
+    return p.n_req > 0 && (p.io.W & 3) == 0 && p.aligned_out != 0;
 }
 
 // ------------------------------------------------------------------ hist
@@ -1300,10 +1295,6 @@ extern "C" int avb_uv_map_u8(const uint8_t *in, uint8_t *out, int n, int H, int 
     p.dbg_catches = dbg_catches_dev;
     p.aligned_in = ((reinterpret_cast<uintptr_t>(in) | (uintptr_t)in_frame_stride | (uintptr_t)in_row_stride) & 3) == 0;
     p.aligned_out = ((reinterpret_cast<uintptr_t>(out) | (uintptr_t)out_frame_stride | (uintptr_t)out_row_stride) & 3) == 0;
-    {
-        static const bool off = [] { const char *e = std::getenv("AVB_UV_NO_PLANE_MAP"); return e && e[0] == '1'; }();
-        p.no_plane_map = off ? 1 : 0;
-    }
     const int SW = R ? 120 : 128;
     p.strips_x = (W + SW - 1) / SW;
     p.strips_y = (H + UV_RH - 1) / UV_RH;

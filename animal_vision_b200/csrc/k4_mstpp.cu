@@ -1019,7 +1019,8 @@ __global__ void __launch_bounds__(GEMM_THREADS) conv3_stream_kernel(const __grid
 // row h+1 never meets a reader of row h-3.  Measured dead end: the depthwise conv as 72 tcgen05.mma per row (N = 16,
 // diagonal 16x16 tap tiles, A descriptors shifted by dx * 16 B): correct, but an M = 128 MMA re-reads its 4 KB A tile from
 // shared memory in ~128 clk whatever N is -- 144 us per launch against 153 us for the three kernels it replaced.
-// Hidden widths above 128 (level 1) run as one pass per 128-channel chunk: chunk 0 writes x = xin + part0, chunk c adds
+// It serves the full-resolution level (Cp = 32, 124 hidden channels: one pass); the coarser levels measured faster as three
+// kernels.  Wider hidden maps run as one pass per 128-channel chunk: chunk 0 writes x = xin + part0, chunk c adds
 // part_c in place (stream order: the sum order is fixed, the forward stays bit-reproducible); LN(xin) is recomputed.
 struct FfnP {
     const float *xin;          // [B, H, W, CP] fp32: the residual stream after the attention block (LayerNorm input)
@@ -1700,11 +1701,6 @@ __device__ __forceinline__ void dwpos_tile(const DwPosP &p, int bx, int by, int 
         }
     }
 }
-__global__ void __launch_bounds__(256) dwpos_fused_kernel(const __grid_constant__ DwPosP p) {
-    pdl_wait();
-    __shared__ __align__(16) uint8_t smem[DP_SMEM];
-    dwpos_tile<256>(p, blockIdx.x, blockIdx.y, blockIdx.z, smem);
-}
 
 // ------------------------------------------------------------------------------------ tiled depthwise 3x3 (coarse-level FFN)
 // The row-walking dwconv_kernel above fetches every input pixel three times (left / centre / right neighbour) through
@@ -1781,95 +1777,15 @@ struct AttnStatP {
     long long *stats;    // [B][heads][32][32] fixed point (STAT_SCALE), zeroed
     int rows, Cp, heads, px_per_cta;
 };
-// 256 threads = 4 pixel groups x (8 x 8) threads, each thread a 4 x 4 register tile of G: per pixel
-// two LDS.128 feed 16 FMAs, so the kernel is bound by the FP32 pipe / HBM, not by shared memory.
-__global__ void __launch_bounds__(256) attn_stats_kernel(const __grid_constant__ AttnStatP p) {
-    pdl_wait();
-    constexpr int TP = 128;
-    __shared__ __align__(16) float qs[TP][32];
-    __shared__ __align__(16) float ks[TP][32];
-    const int tid = threadIdx.x;
-    const int grp = tid >> 6, t = tid & 63, ti = t >> 3, tj = t & 7;
-    const int head = blockIdx.y, b = blockIdx.z;
-    const int p0 = blockIdx.x * p.px_per_cta, p1 = min(p.rows, p0 + p.px_per_cta);
-    const int ld = 3 * p.Cp;
-    float acc[4][4], nk[4], nq[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        nk[i] = nq[i] = 0.f;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
-    }
-    // A head's 31 channels start at column 31*head of the q (and k) block: fetch the <= 5 aligned
-    // 8-channel chunks that cover them with 16-byte loads and scatter the members into the fp32 tile
-    const int lo8 = (head * NF) & ~7;
-    for (int e = tid; e < TP; e += 256) qs[e][31] = ks[e][31] = 0.f;
-    for (int t0 = p0; t0 < p1; t0 += TP) {
-        for (int e = tid; e < TP * 10; e += 256) {
-            const int px = e / 10, c = e - px * 10;
-            const int isk = c >= 5, col0 = lo8 + 8 * (c - 5 * isk);
-            if (col0 >= p.Cp) continue;
-            uint4 raw = make_uint4(0u, 0u, 0u, 0u);
-            if (t0 + px < p1) raw = __ldg(reinterpret_cast<const uint4 *>(p.qkv + ((long long)b * p.rows + t0 + px) * ld + isk * p.Cp + col0));
-            float *dst = isk ? ks[px] : qs[px];
-            const uint32_t w[4] = {raw.x, raw.y, raw.z, raw.w};
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-                const int ch = col0 + i - head * NF;
-                if ((unsigned)ch < (unsigned)NF) dst[ch] = __uint_as_float((i & 1) ? (w[i >> 1] & 0xffff0000u) : (w[i >> 1] << 16));
-            }
-        }
-        __syncthreads();
-#pragma unroll 4
-        for (int px = grp; px < TP; px += 4) {
-            const float4 kv = *reinterpret_cast<const float4 *>(&ks[px][4 * ti]);
-            const float4 qv = *reinterpret_cast<const float4 *>(&qs[px][4 * tj]);
-            const float ka[4] = {kv.x, kv.y, kv.z, kv.w}, qa[4] = {qv.x, qv.y, qv.z, qv.w};
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-#pragma unroll
-                for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(ka[i], qa[j], acc[i][j]);
-                nk[i] = fmaf(ka[i], ka[i], nk[i]);
-                nq[i] = fmaf(qa[i], qa[i], nq[i]);
-            }
-        }
-        __syncthreads();
-    }
-    // reduce the four pixel groups through shared memory (reusing the tiles), then one atomic per entry
-    float *red = &qs[0][0];                       // [4][32][32] floats = 16 KB = qs
-    float *rn = &ks[0][0];                        // [4][2][32]
-#pragma unroll
-    for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) red[(grp * 32 + 4 * ti + i) * 32 + 4 * tj + j] = acc[i][j];
-    if (tj == 0)
-#pragma unroll
-        for (int i = 0; i < 4; ++i) rn[(grp * 2 + 0) * 32 + 4 * ti + i] = nk[i];
-    if (ti == 0)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) rn[(grp * 2 + 1) * 32 + 4 * tj + j] = nq[j];
-    __syncthreads();
-    unsigned long long *out = reinterpret_cast<unsigned long long *>(p.stats) + ((long long)b * p.heads + head) * 1024;
-    for (int e = tid; e < 1024; e += 256) {
-        const int i = e >> 5, j = e & 31;
-        float v;
-        if (i < NF && j < NF) v = red[e] + red[1024 + e] + red[2048 + e] + red[3072 + e];
-        else if (i < NF) v = rn[i] + rn[64 + i] + rn[128 + i] + rn[192 + i];                  // [i][31] = |k_i|^2
-        else if (j < NF) v = rn[32 + j] + rn[96 + j] + rn[160 + j] + rn[224 + j];             // [31][j] = |q_j|^2
-        else v = 0.f;
-        atomicAdd(out + e, (unsigned long long)__double2ll_rn((double)v * STAT_SCALE));      // two's complement: negative sums wrap correctly
-    }
-}
-
-// ---- the same statistics on the tensor cores (round 2).  The CUDA-core kernel above issues 87 warp instructions per
-// pixel (a 4x4 register tile of G per thread: 47 us for the 250 K pixels of the full-resolution level, 11 % of a forward);
-// G = K^T Q over 16 pixels is ONE K-step of mma.sync.m16n8k16 (bf16 operands are exactly what q|k|v holds, f32
-// accumulate), i.e. ~1 warp instruction per pixel, which leaves the kernel bound by reading q and k once.
+// On the tensor cores (round 2): G = K^T Q over 16 pixels is ONE K-step of mma.sync.m16n8k16 (bf16 operands are exactly
+// what q|k|v holds, f32 accumulate), i.e. ~1 warp instruction per pixel, which leaves the statistics bound by reading q and
+// k once.  On the CUDA cores a 4x4 register tile of G per thread took 87 warp instructions per pixel (47 us for the 250 K
+// pixels of the full-resolution level, 11 % of a forward).
 // A head's 31 channels start at column 31*head: the (up to) five aligned 8-channel chunks covering them are staged as a
 // 40-wide bf16 window (zero padded to 48), G_window = K_w^T Q_w is 3 x 5 MMA tiles, the head's block is cut out at the
 // end; |k_i|^2 and |q_j|^2 are the diagonals of K_w^T K_w / Q_w^T Q_w (the 2 diagonal tiles of every 16-row block).
-// Both operands come straight from the [pixel][channel] rows with ldmatrix.trans.  Same fixed-point merge, same layout,
-// same geometry-only split as above: bit-reproducible and batch invariant.
+// Both operands come straight from the [pixel][channel] rows with ldmatrix.trans.  With the fixed-point merge and a split
+// of the pixels that depends on the geometry only, the statistics are bit-reproducible and batch invariant.
 constexpr int AS_TP = 64, AS_PITCH = 56;          // pixels per staging round; bf16 per staged row (112 B = 7 x 16 B: conflict-free ldmatrix)
 __device__ __forceinline__ void as_ldsm_x4_trans(uint32_t (&r)[4], uint32_t addr) {
     asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0,%1,%2,%3}, [%4];" : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
@@ -2005,11 +1921,6 @@ __device__ __forceinline__ void attn_stats_cta(const AttnStatP &p, int bx, int h
         atomicAdd(out + e, (unsigned long long)__double2ll_rn((double)v * STAT_SCALE));
     }
 }
-__global__ void __launch_bounds__(128) attn_stats_mma_kernel(const __grid_constant__ AttnStatP p) {
-    pdl_wait();
-    __shared__ __align__(16) AttnStatSmem S;
-    attn_stats_cta(p, blockIdx.x, blockIdx.y, blockIdx.z, S);
-}
 
 // attn = softmax_j(rescale * G_ij / (max(|k_i|,1e-12) max(|q_j|,1e-12)))  (:127-131), then
 // M[co][h*31+j] = sum_i Wproj[co][h*31+i] attn_h[i][j]  -> bf16 [B][Cp][Cp] (zero padded).
@@ -2018,62 +1929,11 @@ struct AttnFinP {
     bf16 *M;             // [B][Cp][Cp]
     int c, Cp, heads;
 };
-// grid (B, Cp / 32): every CTA redoes the (tiny) softmax and produces 32 rows of M from a Wproj slab
-// staged in shared memory with coalesced loads.
-__global__ void __launch_bounds__(1024) attn_finalize_kernel(const __grid_constant__ AttnFinP p) {
-    pdl_wait();
-    __shared__ float attn[4][31][32];
-    __shared__ float rq[4][32];              // 1 / max(|q_j|, 1e-12)
-    __shared__ float wslab[32][128];         // Wproj rows co0 .. co0+31 (c <= 124 columns)
-    const int b = blockIdx.x, co0 = blockIdx.y * 32, tid = threadIdx.x;
-    for (int e = tid; e < 32 * p.c; e += 1024) {
-        const int r = e / p.c, k = e - r * p.c;
-        wslab[r][k] = (co0 + r < p.c) ? __ldg(p.wproj + (long long)(co0 + r) * p.c + k) : 0.f;
-    }
-    if (tid < p.heads * 32) {
-        const int h = tid >> 5, j = tid & 31;
-        const long long *S = p.stats + ((long long)b * p.heads + h) * 1024;
-        rq[h][j] = j < NF ? 1.0f / fmaxf(sqrtf((float)((double)S[31 * 32 + j] * (1.0 / STAT_SCALE))), 1e-12f) : 0.f;
-    }
-    __syncthreads();
-    // softmax rows: one thread per (head, i)
-    if (tid < p.heads * NF) {
-        const int h = tid / NF, i = tid - h * NF;
-        const long long *S = p.stats + ((long long)b * p.heads + h) * 1024;
-        const float sc = __ldg(p.rescale + h) / fmaxf(sqrtf((float)((double)S[i * 32 + 31] * (1.0 / STAT_SCALE))), 1e-12f);
-        float row[NF], mx = -INFINITY;
-#pragma unroll
-        for (int j = 0; j < NF; ++j) {
-            row[j] = (float)((double)S[i * 32 + j] * (1.0 / STAT_SCALE)) * (sc * rq[h][j]);
-            mx = fmaxf(mx, row[j]);
-        }
-        float sum = 0.f;
-#pragma unroll
-        for (int j = 0; j < NF; ++j) { row[j] = __expf(row[j] - mx); sum += row[j]; }
-        const float inv = 1.0f / sum;
-#pragma unroll
-        for (int j = 0; j < NF; ++j) attn[h][i][j] = row[j] * inv;
-    }
-    __syncthreads();
-    bf16 *M = p.M + ((long long)b * p.Cp + co0) * p.Cp;
-    for (int e = tid; e < 32 * p.Cp; e += 1024) {
-        const int r = e / p.Cp, k = e - r * p.Cp;
-        float v = 0.f;
-        if (co0 + r < p.c && k < p.c) {
-            const int h = k / NF, j = k - h * NF;
-            const float *wrow = &wslab[r][h * NF];
-#pragma unroll
-            for (int i = 0; i < NF; ++i) v = fmaf(wrow[i], attn[h][i][j], v);
-        }
-        M[e] = __float2bfloat16_rn(v);
-    }
-}
-
 // ------------------------------------------------------------------------------------ attention side kernel
 // Everything between the q|k|v GEMM and the projection GEMM of an MSAB in ONE launch of heterogeneous CTAs (128 threads):
 //   blocks [0, nA)   statistics (attn_stats_cta); the LAST statistics CTA of an (image, head) -- a ticket counter behind
 //                    a __threadfence -- turns the finished sums into that head's softmax and its 31 columns of
-//                    M = Wproj . blockdiag(attn) (what attn_finalize_kernel did in a launch of its own)
+//                    M = Wproj . blockdiag(attn)
 //   blocks [nA, ..)  positional-embedding tiles (dwpos_tile), which depend on v only
 // The two parts are independent (one reads q|k and is bound by HBM, the other is CUDA-core work on v), so they overlap
 // on the SMs instead of running back to back, and two launches per block disappear.  Which CTA finalises is a race, what
@@ -2110,7 +1970,7 @@ __device__ __forceinline__ void attn_finalize_head(const AttnFinP &p, int b, int
     constexpr float INV_SCALE = (float)(1.0 / STAT_SCALE);
     if (tid < 32) rq[tid] = tid < NF ? 1.0f / fmaxf(sqrtf((float)__ldcg(S + 31 * 32 + tid) * INV_SCALE), 1e-12f) : 0.f;
     __syncthreads();
-    if (tid < NF) {          // softmax row i = tid (same arithmetic, same order as attn_finalize_kernel)
+    if (tid < NF) {          // softmax row i = tid
         const int i = tid;
         const float sc = __ldg(p.rescale + h) / fmaxf(sqrtf((float)__ldcg(S + i * 32 + 31) * INV_SCALE), 1e-12f);
         float row[NF], mx = -INFINITY;
@@ -2244,7 +2104,7 @@ struct MsabW {
     const float *pos0, *pos2, *ffn_dw;                            // device fp32 [9][Cp] / [9][Hp]
     const bf16 *wqkv, *ffn0, *ffn4;                               // device bf16
     const float *wqkv32;                                          // device fp32 [3*Cp][Cp] (tf32 TMA kernel)
-    const uint8_t *ffn_blob;                                      // fused FFN (Cp <= 64): per 128-channel hidden chunk W0 | W4
+    const uint8_t *ffn_blob;                                      // fused FFN (Cp == 32): per 128-channel hidden chunk W0 | W4
 };
 struct BodyW {
     const bf16 *embedding, *mapping;     // [32][9*32]
@@ -2350,7 +2210,7 @@ static bool pack_msab(Packer &pk, Cursor &cur, MsabW &m, int c) {
     { uint16_t *d = pk.b16((const void **)&m.ffn0, (size_t)Hp * Cp); put_dense(d, Cp, f0, 4 * c, c, 0, 0); }
     { uint16_t *d = pk.b16((const void **)&m.ffn4, (size_t)Cp * Hp); put_dense(d, Hp, f4, c, 4 * c, 0, 0); }
     m.ffn_blob = nullptr;
-    if (Cp <= 64) {
+    if (Cp == 32) {
         // operands of ffn_fused_kernel, chunk by chunk, in the kernel's shared-memory layout (canonical K-major, 16-byte
         // entries of 8 k values): W0 [Cp/8][128 n][8] bf16, W4 [16][Cp n][8] f16
         const int w0_el = (Cp / 8) * 128 * 8, w4_el = 16 * Cp * 8, chunk_el = w0_el + w4_el;
@@ -2598,13 +2458,12 @@ static bool launch_pw(Ctx &cx, const GemmP &p, const char *name) {
         // the tensor map cannot be built: unaligned views)
 #define TMA_CASE(BN_, KP_, EPI_) \
         if (!ln && p.K == KP_ && p.Np % BN_ == 0 && epi == (EPI_) && launch_tma_t<BN_, KP_, (EPI_)>(cx, p, name)) return true;
-        TMA_CASE(32, 32, PROJ) TMA_CASE(64, 64, PROJ) TMA_CASE(128, 128, PROJ) TMA_CASE(32, 128, EPI_RES1)
+        TMA_CASE(32, 32, PROJ) TMA_CASE(64, 64, PROJ) TMA_CASE(128, 128, PROJ)
 #undef TMA_CASE
         PW_CASE(32, 32, false, PROJ) PW_CASE(64, 64, false, PROJ) PW_CASE(128, 128, false, PROJ)
-        PW_CASE(32, 128, false, EPI_RES1)                                        // FFN out, full-resolution level
     } else {
         constexpr int FFN0 = EPI_GELU | EPI_OUTBF16, UP = EPI_BIAS | EPI_CONVT;
-        PW_CASE(128, 32, true, FFN0) PW_CASE(256, 64, true, FFN0) PW_CASE(256, 128, true, FFN0)
+        PW_CASE(256, 64, true, FFN0) PW_CASE(256, 128, true, FFN0)
         // q | k | v: fp32 activations through the TMA engine, tf32 tensor cores (thread-loader kernel as fall-back)
 #define TMA32_CASE(BN_, KP_, EPI_) \
         if (!ln && p.W32 && p.K == KP_ && p.Np % BN_ == 0 && epi == (EPI_) && launch_tma32_t<BN_, KP_, (EPI_)>(cx, p, name)) return true;
@@ -2692,8 +2551,7 @@ static void dwconv(Ctx &cx, const bf16 *in, int ldi, bf16 *out, int ldo, const f
     DwP p{in, ldi, out, ldo, w, cx.B, H, W, Cp, gelu_out, seg};
     const long long total = (long long)cx.B * ((H + seg - 1) / seg) * W * (Cp / DW_CPT);
     AVB_TIMED(name, cx.st);
-    static const bool walk = [] { const char *e = std::getenv("AVB_MSTPP_DW_WALK"); return e && e[0] == '1'; }();
-    if (!walk && Cp % DP_CB == 0 && (ldi & 7) == 0 && (reinterpret_cast<uintptr_t>(in) & 15) == 0) {
+    if (Cp % DP_CB == 0 && (ldi & 7) == 0 && (reinterpret_cast<uintptr_t>(in) & 15) == 0) {
         launch_pdl(dwconv_tile_kernel, dim3((W + DP_TX - 1) / DP_TX, (H + DP_TY - 1) / DP_TY, cx.B * (Cp / DP_CB)), dim3(256), 0, cx.st, p);
         return;
     }
@@ -2732,8 +2590,7 @@ static void msab(Ctx &cx, const MsabW &m, float *x, int H, int W, Workspace &ws)
         p.zero_n = (int)(reinterpret_cast<float *>(ws.stats) - reinterpret_cast<float *>(ws.tickets)) + 2 * cx.B * m.heads * 1024;
         launch_gemm<false, MODE_PW>(cx, p, "k4_gemm_qkv");
     }
-    static const bool attn_unmerged = [] { const char *e = std::getenv("AVB_MSTPP_ATTN_UNMERGED"); return e && e[0] == '1'; }();
-    if (!attn_unmerged) {
+    {
         // statistics (+ softmax / M by the last CTA of every head) and the positional embedding in one launch
         AttnSideP p{};
         p.st = AttnStatP{ws.qkv, ws.stats, rows, Cp, m.heads, 0};
@@ -2751,44 +2608,11 @@ static void msab(Ctx &cx, const MsabW &m, float *x, int H, int W, Workspace &ws)
         const long long total = (long long)p.nA + (long long)p.gx * p.gy * cx.B * (Cp / DP_CB);
         AVB_TIMED("k4_attn_side", cx.st);
         launch_pdl(attn_side_kernel, dim3((unsigned)total), dim3(128), 0, cx.st, p);
-    } else {
-    // Gram + norms over all pixels
-    {
-        AttnStatP p{ws.qkv, ws.stats, rows, Cp, m.heads, 0};
-        // the split depends on the patch geometry only, never on the batch size: a patch gives the same bits
-        // whether it runs alone, in a batch, or in one of several concurrent forwards
-        int ctas = std::max(1, std::min((rows + 255) / 256, sm_count() * 4 / std::max(1, m.heads)));
-        p.px_per_cta = ((rows + ctas - 1) / ctas + 127) / 128 * 128;
-        ctas = (rows + p.px_per_cta - 1) / p.px_per_cta;
-        AVB_TIMED("k4_attn_stats", cx.st);
-        static const bool cuda_core_stats = [] { const char *e = std::getenv("AVB_MSTPP_STATS_CUDA_CORES"); return e && e[0] == '1'; }();
-        if (cuda_core_stats) {
-            launch_pdl(attn_stats_kernel, dim3(ctas, m.heads, cx.B), dim3(256), 0, cx.st, p);
-        } else {
-            // the tensor-core kernel streams: two CTAs per SM over all heads, each a long double-buffered run of pixels
-            ctas = std::max(1, std::min((rows + 255) / 256, sm_count() * 2 / std::max(1, m.heads)));
-            p.px_per_cta = ((rows + ctas - 1) / ctas + 127) / 128 * 128;
-            ctas = (rows + p.px_per_cta - 1) / p.px_per_cta;
-            launch_pdl(attn_stats_mma_kernel, dim3(ctas, m.heads, cx.B), dim3(128), 0, cx.st, p);
-        }
     }
-    {
-        AttnFinP p{ws.stats, m.rescale, m.wproj_f32, ws.M, m.c, Cp, m.heads};
-        AVB_TIMED("k4_attn_finalize", cx.st);
-        launch_pdl(attn_finalize_kernel, dim3(cx.B, Cp / 32), dim3(1024), 0, cx.st, p);
-    }
-    // pos_emb(v): dw3x3 -> GELU -> dw3x3
-    {
-        DwPosP p{ws.qkv + 2 * Cp, 3 * Cp, ws.p2, Cp, m.pos0, m.pos2, cx.B, H, W, Cp};
-        AVB_TIMED("k4_dw_pos", cx.st);
-        launch_pdl(dwpos_fused_kernel, dim3((W + DP_TX - 1) / DP_TX, (H + DP_TY - 1) / DP_TY, cx.B * (Cp / DP_CB)), dim3(256), 0, cx.st, p);
-    }
-    }
-    // the fused feed-forward kernel reads halo rows of its input while neighbouring CTAs write the output: the
-    // attention block then leaves its result in ws.xt and the feed-forward block brings it back to x
-    static const bool ffn_unfused = [] { const char *e = std::getenv("AVB_MSTPP_FFN_UNFUSED"); return e && e[0] == '1'; }();
-    static const int ffn_fused_max_cp = [] { const char *e = std::getenv("AVB_MSTPP_FFN_FUSED_MAXCP"); return e ? atoi(e) : 32; }();
-    const bool ffn_fused = !ffn_unfused && m.ffn_blob != nullptr && (Cp == 32 || Cp == 64) && Cp <= ffn_fused_max_cp;
+    // the full-resolution level (Cp == 32) runs its feed-forward block as one fused kernel, the coarser levels as three.
+    // The fused kernel reads halo rows of its input while neighbouring CTAs write the output: the attention block then
+    // leaves its result in ws.xt and the feed-forward block brings it back to x
+    const bool ffn_fused = Cp == 32;
     // x = v M^T + b + pos + x
     {
         GemmP p = gemm_defaults();
@@ -2797,8 +2621,7 @@ static void msab(Ctx &cx, const MsabW &m, float *x, int H, int W, Workspace &ws)
         launch_gemm<true, MODE_PW>(cx, p, "k4_gemm_attn_proj");
     }
     if (ffn_fused) {
-        if (Cp == 32) ffn_fused_launch<32>(cx, m, ws.xt, x, H, W);
-        else ffn_fused_launch<64>(cx, m, ws.xt, x, H, W);
+        ffn_fused_launch<32>(cx, m, ws.xt, x, H, W);
         return;
     }
     // FFN: x = W4 GELU(dw(GELU(W0 LN(x)))) + x; the LayerNorm runs inside the FFN-in GEMM's loader

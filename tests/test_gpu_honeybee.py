@@ -119,3 +119,29 @@ def test_bee_degenerate_frames_keep_exact_percentiles():
         _, ref = uv.honeybee_visualize(fr)
         _, out = HoneyBee().visualize(fr)
         _cmp(out, ref, "degenerate")
+
+
+def test_plane_route_equals_the_second_walk():
+    """The map pass of a mapper with percentiles reads the planes of the hist pass when the output is 4-byte aligned and
+    W % 4 == 0, and walks the frame a second time otherwise (map_from_planes in csrc/k3_uv.cu).  Both routes give identical
+    bytes: every case runs once into a packed output and once into a view that starts one pixel (3 bytes) into a wider
+    buffer, which always takes the walk."""
+    import torch
+    from animal_vision_b200.animals import HoneyBee
+    g = torch.Generator().manual_seed(5)
+    for n, h, w in ((3, 270, 480), (1, 123, 236), (2, 64, 1100), (1, 37, 50)):
+        fr = torch.randint(0, 256, (n, h, w, 3), dtype=torch.uint8, generator=g).cuda()
+        fr[0, : h // 2] //= 3
+        wide = torch.zeros((n, h, w + 24, 3), dtype=torch.uint8, device="cuda")
+        wide[:, :, 8:8 + w] = fr
+        cases = [(kw, fr) for kw in ({}, {"adaptation": "gray_world"}, {"blur_sigma_px": None}, {"blur_sigma_px": 0.6},
+                                     {"adaptation": None}, {"mapping_mode": "falsecolor"}, {"mapping_mode": "uv_purple_yellow"},
+                                     {"mapping_mode": "falsecolor_uv_mixed"},
+                                     {"mapping_mode": "falsecolor", "adaptation": "gray_world", "blur_sigma_px": 0.6})]
+        cases.append(({}, wide[:, :, 8:8 + w]))            # strided input rows
+        for kw, src in cases:
+            bee = HoneyBee(**kw)
+            _, packed = bee.visualize_batch(src)
+            shifted = torch.empty((n, h, w + 1, 3), dtype=torch.uint8, device="cuda")[:, :, 1:]
+            bee.visualize_batch(src, shifted)
+            assert torch.equal(packed, shifted), ((n, h, w), kw, src.is_contiguous())

@@ -36,7 +36,8 @@ def test_against_reference_golden(model, golden):
     assert mx <= TOL and l2 <= TOL, f"max-abs rel {mx:.3e}, rel-L2 {l2:.3e}"
 
 
-@pytest.mark.parametrize("shape", [(1, 64, 72), (2, 40, 88), (3, 17, 33), (1, 130, 94), (1, 24, 200), (2, 9, 300)])
+@pytest.mark.parametrize("shape", [(1, 64, 72), (2, 40, 88), (3, 17, 33), (1, 130, 94), (1, 24, 200), (2, 9, 300),
+                                   (2, 24, 200), (1, 130, 260)])
 def test_against_oracle_shapes_and_batches(model, shape):
     """Batches: the attention statistics are per image, so images must not see each other."""
     net, sd = model
