@@ -6,7 +6,7 @@
 //             block (strip + halo columns, REFLECT_101 halo rows resolved per row) are staged by the
 //             TMA engine: one cp.async.bulk per row into a double-buffered raw byte tile, completion
 //             on an mbarrier, issued one block ahead -- no thread waits on a global load.  The LUT
-//             producer then decodes 4 pixels (12 bytes) per thread, the cat warp producer gathers its
+//             kernel then decodes 4 pixels (12 bytes) per thread, the cat warp kernel gathers its
 //             bilinear taps from the tile; unaligned frames and image-border strips go pixel by pixel;
 //   H pass    8 outputs per thread from an (8+2R)-wide register window (LDS.128), taps from the
 //             kernel-parameter constant bank;
@@ -23,13 +23,12 @@
 // third fewer FMAs), the 3x2 expansion happens in the encode phase.  Full-rank matrices take the
 // three-plane instantiation.
 //
-// The producer is a policy: DogProducer (LUT decode + 3x3; animals/dog.py:35-48) or CatProducer
-// (binocular wide-FOV gather + blend + pow decode + 3x3; animals/cat_widevision_utils.py:46-99,
-// animals/cat.py:95-101).
+// Two kernels share the H pass, V pass and encode: gauss_stream_kernel produces with DogProducer (LUT
+// decode + 3x3; animals/dog.py:35-48), cat_warp_kernel with the binocular wide-FOV gather + blend + pow
+// decode + 3x3 (animals/cat_widevision_utils.py:46-99, animals/cat.py:95-101).
 #include <algorithm>
 #include <cmath>
 #include <cstdlib>
-#include <type_traits>
 
 #include <cuda_fp16.h>
 
@@ -79,8 +78,6 @@ struct DogProducer {
         const float *lut;  // 256-entry decode LUT (device)
     };
     static constexpr int SMEM_FLOATS = 256;
-    static constexpr bool VEC = true;      // has a 4-pixel vector path (three packed 32-bit words -> 4 px)
-    static constexpr bool GATHER = false;
     static constexpr int RAW_PITCH = 528;  // bytes per row of the raw tile: 33 chunks of 16 B
     const float *lut_s;
     const uint8_t *src;
@@ -98,7 +95,6 @@ struct DogProducer {
         for (int i = 0; i < 9; ++i) m[i] = pp.M.m[i];
         seen = 0;
     }
-    __device__ __forceinline__ bool all_black(int, int) const { return false; }
     __device__ __forceinline__ void px(uint32_t b0, uint32_t b1, uint32_t b2, float &o0, float &o1, float &o2) const {
         const float l0 = lut_s[b0], l1 = lut_s[b1], l2 = lut_s[b2];
         o0 = m[0] * l0 + m[1] * l1 + m[2] * l2;
@@ -121,167 +117,6 @@ struct DogProducer {
         seen |= b0 | b1 | b2;
         px(b0, b1, b2, o0, o1, o2);
     }
-    template <bool WORDS>
-    __device__ __forceinline__ void at_row(const Column &, const uint8_t *, float &, float &, float &) {}
-    __device__ __forceinline__ void span(const Column &, int &, int &, int &) const {}
-};
-
-struct CatProducer {
-    static const char *name() { return "k2_gauss_cat_warp"; }
-    static const char *fixup_name() { return "k2_gauss_cat_warp_fixup"; }
-    struct Params {
-        Mat3 M;             // RGB->LMS, L/M merge, LMS->RGB collapsed into one 3x3 (host, float64 -> f32)
-        const float *xl, *xr, *wl, *wr;  // per-column tables, length W (device)
-        const float *ws, *rws;           // per column: wl + wr + 1e-8 (float32) and its correctly rounded reciprocal
-        const uint32_t *frame_flags;     // per frame: != 0 when some byte >= 2 (written by frame_flags_kernel)
-        int norm_mode;                   // AVB_NORM_DIV255: always /255; AVB_NORM_AUTO: /255 iff flag set
-    };
-    static constexpr int SMEM_FLOATS = 256;
-    static constexpr bool VEC = false;
-    static constexpr bool GATHER = true;   // source columns of a strip are staged in shared memory, taps gather from there
-    static constexpr int RAW_PITCH = 960;  // 16 B slack + 58 chunks of 16 B + slack: (128 + 2*16) columns x 2.1 source px x 3 B + alignment slack
-    const float *norm_s;
-    const uint8_t *src;
-    int64_t rs;
-    int W;
-    float m[9];
-    const float *xl, *xr, *wl, *wr, *ws, *rws;
-    uint32_t seen;
-
-    __device__ __forceinline__ void init(const Params &pp, float *smem, const uint8_t *frame, int64_t row_stride,
-                                         int /*H*/, int W_, int frame_idx) {
-        // normalised byte values exactly as NumPy makes them: float32(v) / float32(255), or, when the
-        // frame max is <= 1 (get_normalized_image's other branch), the byte itself clipped to [0,1]
-        const bool div255 = pp.norm_mode == AVB_NORM_DIV255 || __ldg(pp.frame_flags + frame_idx) != 0;
-        for (int i = threadIdx.x; i < 256; i += blockDim.x)
-            smem[i] = div255 ? __fdiv_rn((float)i, 255.0f) : fminf((float)i, 1.0f);
-        norm_s = smem;
-        src = frame;
-        rs = row_stride;
-        W = W_;
-#pragma unroll
-        for (int i = 0; i < 9; ++i) m[i] = pp.M.m[i];
-        xl = pp.xl; xr = pp.xr; wl = pp.wl; wr = pp.wr; ws = pp.ws; rws = pp.rws;
-        seen = 0;
-    }
-    __device__ __forceinline__ void decode4(uint32_t, uint32_t, uint32_t, float4 &, float4 &, float4 &) {}
-    __device__ __forceinline__ void px(uint32_t, uint32_t, uint32_t, float &, float &, float &) const {}
-    // every column of [xa, xb) has zero weight in both eye views: the strip is black
-    __device__ __forceinline__ bool all_black(int xa, int xb) const {
-        bool any = false;
-        for (int x = xa + (int)threadIdx.x; x < xb; x += blockDim.x) {
-            const int xc = reflect101(x, W);
-            any |= (__ldg(wl + xc) != 0.0f) || (__ldg(wr + xc) != 0.0f);
-        }
-        return !__syncthreads_or(any);
-    }
-    // ---- per-column state (every map of cat_widevision_utils.py:61-96 depends on the column only):
-    // which eye view is live, its two source columns and bilinear weights, the blend denominator.
-    // cv::remap INTER_LINEAR: map coordinate quantised to 1/32 px, two taps, border constant 0.
-    struct Tap { int ix; float w0, f; bool ok0, ok1; };
-    struct Column { float wL, wR, s, r; Tap L, R; };
-    __device__ __forceinline__ Tap make_tap(float xs) const {
-        Tap t;
-        const int sx = __float2int_rn(xs * 32.0f);
-        t.ix = sx >> 5;
-        t.f = (float)(sx & 31) * (1.0f / 32.0f);
-        t.w0 = 1.0f - t.f;
-        t.ok0 = (unsigned)t.ix < (unsigned)W;
-        t.ok1 = (unsigned)(t.ix + 1) < (unsigned)W;
-        return t;
-    }
-    __device__ __forceinline__ Column column(int x) const {
-        Column c;
-        c.wL = __ldg(wl + x); c.wR = __ldg(wr + x);
-        c.s = __ldg(ws + x); c.r = __ldg(rws + x);
-        c.L = make_tap(__ldg(xl + x));
-        c.R = make_tap(__ldg(xr + x));
-        return c;
-    }
-    __device__ __forceinline__ void gather(const uint8_t *row, const Tap &t, float &c0, float &c1, float &c2) {
-        float a0 = 0.f, a1 = 0.f, a2 = 0.f, b0 = 0.f, b1 = 0.f, b2 = 0.f;
-        const uint8_t *q = row + 3 * t.ix;
-        if (t.ok0) {
-            const uint32_t u0 = q[0], u1 = q[1], u2 = q[2];
-            seen |= u0 | u1 | u2;
-            a0 = norm_s[u0]; a1 = norm_s[u1]; a2 = norm_s[u2];
-        }
-        if (t.ok1) {
-            const uint32_t u0 = q[3], u1 = q[4], u2 = q[5];
-            seen |= u0 | u1 | u2;
-            b0 = norm_s[u0]; b1 = norm_s[u1]; b2 = norm_s[u2];
-        }
-        c0 = __fadd_rn(__fmul_rn(a0, t.w0), __fmul_rn(b0, t.f));
-        c1 = __fadd_rn(__fmul_rn(a1, t.w0), __fmul_rn(b1, t.f));
-        c2 = __fadd_rn(__fmul_rn(a2, t.w0), __fmul_rn(b2, t.f));
-    }
-    // same taps from a 4-byte aligned row (the shared raw tile): the two source pixels are 6
-    // contiguous bytes = three 32-bit loads + two funnel shifts instead of six byte loads.  Out of
-    // image taps (border constant 0) are masked after the fact; the tile has slack on both sides.
-    __device__ __forceinline__ void gather_words(const uint8_t *row, const Tap &t, float &c0, float &c1, float &c2) {
-        const int ob = 3 * t.ix;
-        const uint32_t *w = reinterpret_cast<const uint32_t *>(row + (ob & ~3));
-        const int sh = (ob & 3) * 8;
-        const uint32_t w0 = w[0], w1 = w[1], w2 = w[2];
-        const uint32_t lo = __funnelshift_r(w0, w1, sh), hi = __funnelshift_r(w1, w2, sh);
-        float a0 = norm_s[lo & 0xffu], a1 = norm_s[(lo >> 8) & 0xffu], a2 = norm_s[(lo >> 16) & 0xffu];
-        float b0 = norm_s[lo >> 24], b1 = norm_s[hi & 0xffu], b2 = norm_s[(hi >> 8) & 0xffu];
-        if (!t.ok0) { a0 = a1 = a2 = 0.f; }
-        if (!t.ok1) { b0 = b1 = b2 = 0.f; }
-        c0 = __fadd_rn(__fmul_rn(a0, t.w0), __fmul_rn(b0, t.f));
-        c1 = __fadd_rn(__fmul_rn(a1, t.w0), __fmul_rn(b1, t.f));
-        c2 = __fadd_rn(__fmul_rn(a2, t.w0), __fmul_rn(b2, t.f));
-    }
-    static __device__ __forceinline__ float decode(float v) {
-        // animals/animal_utils.py:5-11 on float32; the power goes through the SFU (ex2(2.4 lg2 x),
-        // ~5e-7 relative: far inside the 1-LSB budget of the uint8 result)
-        // (arguments stay in [0.09, 1] and exponents in [-8.4, 0]: the .ftz SFU forms are exact enough
-        // and need no denormal scaling code around them)
-        float l, e;
-        asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(l) : "f"((v + 0.055f) * (1.0f / 1.055f)));
-        asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(2.4f * l));
-        return v <= 0.04045f ? v * (1.0f / 12.92f) : e;
-    }
-    // source-column span this output column touches, and which eye views are live
-    __device__ __forceinline__ void span(const Column &c, int &lo, int &hi, int &mode) const {
-        if (c.wL != 0.0f) { lo = min(lo, c.L.ix); hi = max(hi, c.L.ix + 1); mode |= 1; }
-        if (c.wR != 0.0f) { lo = min(lo, c.R.ix); hi = max(hi, c.R.ix + 1); mode |= 2; }
-        if (c.wL != 0.0f && c.wR != 0.0f) mode |= 4;
-    }
-    __device__ __forceinline__ void at(const Column &c, int y, float &o0, float &o1, float &o2) {
-        at_row<false>(c, src + (int64_t)y * rs, o0, o1, o2);
-    }
-    // `row` addresses source column ix at row[3*ix] (a global row, or the shared raw tile rebased;
-    // WORDS: the row is 4-byte aligned and readable a few bytes past either end of the span)
-    template <bool WORDS>
-    __device__ __forceinline__ void at_row(const Column &c, const uint8_t *row, float &o0, float &o1, float &o2) {
-        if (c.wL == 0.0f && c.wR == 0.0f) {     // outside both eye views: (0*wL + 0*wR)/ws = 0 -> decode(0) = 0
-            o0 = o1 = o2 = 0.f;
-            return;
-        }
-        float l0 = 0.f, l1 = 0.f, l2 = 0.f, r0 = 0.f, r1 = 0.f, r2 = 0.f;
-        // a zero weight multiplies a finite sample: skipping the gather leaves the sum unchanged
-        if (WORDS) {
-            if (c.wL != 0.0f) gather_words(row, c.L, l0, l1, l2);
-            if (c.wR != 0.0f) gather_words(row, c.R, r0, r1, r2);
-        } else {
-            if (c.wL != 0.0f) gather(row, c.L, l0, l1, l2);
-            if (c.wR != 0.0f) gather(row, c.R, r0, r1, r2);
-        }
-        // (left*wL + right*wR) / (wL + wR + 1e-8), the quotient correctly rounded from the
-        // per-column reciprocal (one Newton step on the quotient)
-        const float n0 = __fadd_rn(__fmul_rn(l0, c.wL), __fmul_rn(r0, c.wR));
-        const float n1 = __fadd_rn(__fmul_rn(l1, c.wL), __fmul_rn(r1, c.wR));
-        const float n2 = __fadd_rn(__fmul_rn(l2, c.wL), __fmul_rn(r2, c.wR));
-        float q0 = __fmul_rn(n0, c.r), q1 = __fmul_rn(n1, c.r), q2 = __fmul_rn(n2, c.r);
-        q0 = fmaf(fmaf(-q0, c.s, n0), c.r, q0);
-        q1 = fmaf(fmaf(-q1, c.s, n1), c.r, q1);
-        q2 = fmaf(fmaf(-q2, c.s, n2), c.r, q2);
-        const float s0 = decode(__saturatef(q0)), s1 = decode(__saturatef(q1)), s2 = decode(__saturatef(q2));
-        o0 = m[0] * s0 + m[1] * s1 + m[2] * s2;
-        o1 = m[3] * s0 + m[4] * s1 + m[5] * s2;
-        o2 = m[6] * s0 + m[7] * s1 + m[8] * s2;
-    }
 };
 
 // ------------------------------------------------------------------------------------ bulk-copy (TMA) helpers
@@ -302,7 +137,98 @@ __device__ __forceinline__ void gauss_mbar_wait(uint64_t *bar, uint32_t parity) 
                      : "=r"(ok) : "r"(a), "r"(parity) : "memory");
 }
 
-// ------------------------------------------------------------------------------------ kernel
+// ------------------------------------------------------------------------------------ phases shared by both kernels
+// H pass: thread -> (plane ch, row h_r, 8-px group h_xg); 8 outputs from a WIN-wide register window
+template <int R>
+__device__ __forceinline__ void gauss_hpass(const GaussCommon &p, const float *S, float *X, int ch, int h_r, int h_xg) {
+    using C = GaussCfg<R>;
+    const float4 *w4 = reinterpret_cast<const float4 *>(&S[ch * C::S_PLANE + h_r * C::S_PITCH + h_xg * 8]);
+    float v[4 * C::NW4];
+#pragma unroll
+    for (int q = 0; q < C::NW4; ++q) {
+        const float4 t = w4[q];
+        v[4 * q] = t.x; v[4 * q + 1] = t.y; v[4 * q + 2] = t.z; v[4 * q + 3] = t.w;
+    }
+    float acc[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) acc[j] = 0.f;
+#pragma unroll
+    for (int k = 0; k <= 2 * R; ++k) {
+        const float tk = p.taps[k];
+#pragma unroll
+        for (int j = 0; j < 8; ++j) acc[j] = fmaf(tk, v[j + k], acc[j]);
+    }
+    float4 *d4 = reinterpret_cast<float4 *>(&X[ch * C::X_PLANE + h_r * C::X_PITCH + h_xg * 8]);
+    d4[0] = make_float4(acc[0], acc[1], acc[2], acc[3]);
+    d4[1] = make_float4(acc[4], acc[5], acc[6], acc[7]);
+}
+
+// V pass, one input row at a time: finish the oldest output row, advance the rest.  Thread -> (plane ch, column v_x).
+// Input row i (0-based in the segment) completes output row y_start + i - 2R.
+template <int R>
+__device__ __forceinline__ void gauss_vpass(const GaussCommon &p, const float *X, float *Y, int ch, int v_x, float (&A)[2 * R]) {
+    using C = GaussCfg<R>;
+    const float *col = X + ch * C::X_PLANE + v_x;
+    float *ycol = Y + ch * C::X_PLANE + v_x;
+#pragma unroll
+    for (int r = 0; r < G_RB; ++r) {
+        const float h = col[r * C::X_PITCH];
+        ycol[r * C::X_PITCH] = fmaf(p.taps[2 * R], h, A[0]);
+#pragma unroll
+        for (int m = 0; m < 2 * R - 1; ++m) A[m] = fmaf(p.taps[2 * R - 1 - m], h, A[m + 1]);
+        A[2 * R - 1] = p.taps[0] * h;
+    }
+}
+
+// expand (two-plane mode) + encode + store: a task is 4 consecutive pixels of one row (12 bytes = three 32-bit
+// stores); input row i = 8*ib + r -> output row y_start + i - 2R
+template <int R, int NCH, int THREADS>
+__device__ __forceinline__ void gauss_encode_store(const GaussCommon &p, const EncTable &enc, const float *Y, uint8_t *dst_frame,
+                                                   int ib, int y_start, int y_end, int x0, bool out4) {
+    using C = GaussCfg<R>;
+    const int W = p.io.W;
+    const int oy0 = y_start + ib * G_RB - 2 * R;
+    for (int t = threadIdx.x; t < G_RB * (G_TW / 4); t += THREADS) {
+        const int r = t >> 5, g4 = t & 31;
+        const int oy = oy0 + r;
+        if (oy < y_start || oy >= y_end) continue;
+        const int xo = x0 + 4 * g4;
+        if (xo >= W) continue;
+        const float4 a4 = *reinterpret_cast<const float4 *>(&Y[0 * C::X_PLANE + r * C::X_PITCH + 4 * g4]);
+        const float4 b4 = *reinterpret_cast<const float4 *>(&Y[1 * C::X_PLANE + r * C::X_PITCH + 4 * g4]);
+        float4 c4 = make_float4(0.f, 0.f, 0.f, 0.f);
+        if (NCH == 3) c4 = *reinterpret_cast<const float4 *>(&Y[2 * C::X_PLANE + r * C::X_PITCH + 4 * g4]);
+        const float av[4] = {a4.x, a4.y, a4.z, a4.w}, bv[4] = {b4.x, b4.y, b4.z, b4.w}, cv[4] = {c4.x, c4.y, c4.z, c4.w};
+        uint32_t by[12];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            float r0, r1, r2;
+            if (NCH == 2) {
+                r0 = fmaf(p.P[1], bv[j], p.P[0] * av[j]);
+                r1 = fmaf(p.P[3], bv[j], p.P[2] * av[j]);
+                r2 = fmaf(p.P[5], bv[j], p.P[4] * av[j]);
+            } else {
+                r0 = av[j]; r1 = bv[j]; r2 = cv[j];
+            }
+            by[3 * j] = encode_u8(enc, r0);
+            by[3 * j + 1] = encode_u8(enc, r1);
+            by[3 * j + 2] = encode_u8(enc, r2);
+        }
+        uint8_t *o = dst_frame + (int64_t)oy * p.io.out_rs + (int64_t)xo * 3;
+        if (out4 && xo + 3 < W) {
+            uint32_t *o32 = reinterpret_cast<uint32_t *>(o);
+#pragma unroll
+            for (int q = 0; q < 3; ++q) o32[q] = by[4 * q] | (by[4 * q + 1] << 8) | (by[4 * q + 2] << 16) | (by[4 * q + 3] << 24);
+        } else {
+            const int nb = 3 * min(4, W - xo);
+#pragma unroll
+            for (int q = 0; q < 12; ++q)
+                if (q < nb) o[q] = (uint8_t)by[q];
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------ LUT kernel
 #ifndef G_MINB
 #define G_MINB 2
 #endif
@@ -311,16 +237,12 @@ __device__ __forceinline__ void gauss_mbar_wait(uint64_t *bar, uint32_t parity) 
 #endif
 // two-plane CTAs (256 threads) fit three per SM up to radius 14 (72 registers with the TMA-staged tiles);
 // three-plane CTAs (384 threads) keep the earlier split
-#ifndef G_MINB4_R
-#define G_MINB4_R 4
-#endif
-// the cat's gather producer at radius <= 4 (its 9-tap blur): four CTAs per SM, 64 registers (measured, 20 4K frames: 1.169 -> 1.135 ms)
-template <int R, int NCH, bool GATHER = false>
-struct GaussOcc { static constexpr int MIN_BLOCKS = (GATHER && NCH == 2 && R <= G_MINB4_R) ? 4 : ((R <= (NCH == 2 ? G_MINB3_R : 8)) ? 3 : G_MINB); };
+template <int R, int NCH>
+struct GaussOcc { static constexpr int MIN_BLOCKS = (R <= (NCH == 2 ? G_MINB3_R : 8)) ? 3 : G_MINB; };
 
-template <int R, class Prod, int NCH>
-__global__ void __launch_bounds__(G_THREADS_PER_PLANE * NCH, GaussOcc<R, NCH, Prod::GATHER>::MIN_BLOCKS)
-gauss_stream_kernel(const __grid_constant__ GaussCommon p, const __grid_constant__ typename Prod::Params pp) {
+template <int R, int NCH>
+__global__ void __launch_bounds__(G_THREADS_PER_PLANE * NCH, GaussOcc<R, NCH>::MIN_BLOCKS)
+gauss_stream_kernel(const __grid_constant__ GaussCommon p, const __grid_constant__ DogProducer::Params pp) {
     using C = GaussCfg<R>;
     constexpr int THREADS = G_THREADS_PER_PLANE * NCH;
     extern __shared__ __align__(16) uint8_t smem_raw[];
@@ -328,22 +250,21 @@ gauss_stream_kernel(const __grid_constant__ GaussCommon p, const __grid_constant
     float *X = S + NCH * C::S_PLANE;                           // [NCH][RB][X_PITCH] horizontally blurred rows
     float *Y = X + NCH * C::X_PLANE;                           // [NCH][RB][X_PITCH] fully blurred rows
     float *prod_smem = Y + NCH * C::X_PLANE;
-    uint32_t *enc_s = reinterpret_cast<uint32_t *>(prod_smem + Prod::SMEM_FLOATS);
+    uint32_t *enc_s = reinterpret_cast<uint32_t *>(prod_smem + DogProducer::SMEM_FLOATS);
     uint8_t *rawt0 = reinterpret_cast<uint8_t *>(enc_s + G_ENC_SMEM);              // [2][RB][RAW_PITCH] packed input rows (TMA double buffer)
-    constexpr int RAW_PITCH = Prod::RAW_PITCH;
+    constexpr int RAW_PITCH = DogProducer::RAW_PITCH;
     __shared__ __align__(8) uint64_t rbar[2];                                       // completion of the bulk copies of each buffer
-    __shared__ int gat[3];                                                          // gather producer: span lo, hi, eye mode
 
     const int frame = blockIdx.z;
     if (p.fixup && p.flags[frame] != 0) return;
 
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int tid = threadIdx.x, lane = tid & 31;
     const int H = p.io.H, W = p.io.W;
     const int x0 = blockIdx.x * G_TW;
     const int y_start = blockIdx.y * p.seg_h;
     const int y_end = min(H, y_start + p.seg_h);
 
-    Prod prod;
+    DogProducer prod;
     const uint8_t *src_frame = p.io.in + (int64_t)frame * p.io.in_fs;
     prod.init(pp, prod_smem, src_frame, p.io.in_rs, H, W, frame);
     copy_to_smem(enc_s, p.enc, min(G_ENC_SMEM, ENC_HEADER + (int)__ldg(p.enc + 2)));
@@ -351,46 +272,15 @@ gauss_stream_kernel(const __grid_constant__ GaussCommon p, const __grid_constant
     const EncTable enc = enc_view(enc_s);
 
     uint8_t *dst_frame = p.io.out + (int64_t)frame * p.io.out_fs;
-    const bool vec_ok = (x0 + G_TW <= W) && ((p.io.out_rs & 15) == 0) && ((p.io.out_fs & 15) == 0) &&
-                        ((reinterpret_cast<uintptr_t>(p.io.out) & 15) == 0);
     const bool out4 = ((p.io.out_rs & 3) == 0) && ((p.io.out_fs & 3) == 0) && ((reinterpret_cast<uintptr_t>(p.io.out) & 3) == 0);
 
-    // a strip whose producer is identically zero (the cat's blind middle third) encodes to byte 0
-    if (prod.all_black(x0 - R, x0 + G_TW + R)) {
-        const int nbytes = min(G_TW, W - x0) * 3;
-        for (int y = y_start + warp; y < y_end; y += THREADS / 32) {
-            uint8_t *row = dst_frame + (int64_t)y * p.io.out_rs + (int64_t)x0 * 3;
-            if (vec_ok) {
-                if (lane < G_TW * 3 / 16) reinterpret_cast<uint4 *>(row)[lane] = make_uint4(0u, 0u, 0u, 0u);
-            } else {
-                for (int b = lane; b < nbytes; b += 32) row[b] = 0;
-            }
-        }
-        return;
-    }
-
-    // Raw tile: the packed bytes [a0, a0 + 16*n_chunks) of 8 input rows, fetched with 16-byte loads
-    // one block ahead.  LUT producer: the strip plus its halo (and the over-read of the last 4-pixel
-    // group); gather producer: the source columns the strip's taps touch (single live eye view).
+    // Raw tile: the packed bytes [a0, a0 + 16*n_chunks) of 8 input rows -- the strip plus its halo (and the
+    // over-read of the last 4-pixel group) -- fetched with 16-byte loads one block ahead.
     const bool in16 = ((p.io.in_rs & 15) == 0) && ((p.io.in_fs & 15) == 0) && ((reinterpret_cast<uintptr_t>(p.io.in) & 15) == 0);
-    int a_byte = 3 * (x0 - R);                       // first byte of the produced span (LUT producer)
-    int a0 = a_byte & ~15;
-    int n_chunks = (a_byte - a0 + 12 * C::GROUPS + 15) >> 4;
-    bool vec_in = Prod::VEC && x0 - R >= 0 && a0 + 16 * n_chunks <= 3 * W && in16;
-    if (Prod::GATHER) {
-        if (tid == 0) { gat[0] = 0x7fffffff; gat[1] = -1; gat[2] = 0; }
-        __syncthreads();
-        int lo = 0x7fffffff, hi = -1, mode = 0;
-        for (int i = tid; i < C::IN_W; i += THREADS) prod.span(prod.column(reflect101(x0 - R + i, W)), lo, hi, mode);
-        if (mode) { atomicMin(&gat[0], lo); atomicMax(&gat[1], hi); atomicOr(&gat[2], mode); }
-        __syncthreads();
-        const int ixlo = max(gat[0], 0), ixhi = min(gat[1], W - 1);
-        a0 = (3 * ixlo) & ~15;
-        n_chunks = (3 * (ixhi + 1) - a0 + 15) >> 4;
-        vec_in = (gat[2] == 1 || gat[2] == 2) && in16 && n_chunks > 0 && 16 * n_chunks + 32 <= RAW_PITCH &&
-                 a0 + 16 * n_chunks <= (int)p.io.in_rs;
-    }
-    vec_in = vec_in && 16 * n_chunks + (Prod::GATHER ? 32 : 0) <= RAW_PITCH;
+    const int a_byte = 3 * (x0 - R);                 // first byte of the produced span
+    const int a0 = a_byte & ~15;
+    const int n_chunks = (a_byte - a0 + 12 * C::GROUPS + 15) >> 4;
+    const bool vec_in = x0 - R >= 0 && a0 + 16 * n_chunks <= 3 * W && in16 && 16 * n_chunks <= RAW_PITCH;
 
     const int n_in_rows = (y_end - y_start) + 2 * R;
     const int n_in_blocks = (n_in_rows + G_RB - 1) / G_RB;
@@ -414,7 +304,7 @@ gauss_stream_kernel(const __grid_constant__ GaussCommon p, const __grid_constant
     auto raw_issue = [&](int yb_, int buf) {
         if (tid < G_RB) {
             const uint8_t *g = src_frame + (int64_t)reflect101(yb_ + tid, H) * p.io.in_rs + a0;
-            gauss_bulk_load(rawt0 + buf * (G_RB * RAW_PITCH) + (Prod::GATHER ? 16 : 0) + tid * RAW_PITCH, g, 16u * (uint32_t)n_chunks, &rbar[buf]);
+            gauss_bulk_load(rawt0 + buf * (G_RB * RAW_PITCH) + tid * RAW_PITCH, g, 16u * (uint32_t)n_chunks, &rbar[buf]);
         }
     };
     uint32_t rphase = 0;                             // bit b: parity the next wait on buffer b expects
@@ -431,73 +321,46 @@ gauss_stream_kernel(const __grid_constant__ GaussCommon p, const __grid_constant
             gauss_mbar_wait(&rbar[buf], (rphase >> buf) & 1u);
             rphase ^= 1u << buf;
             if (ib + 1 < n_in_blocks) raw_issue(yb + G_RB, buf ^ 1);
-            if (Prod::GATHER) {
-                // taps gather from the shared raw tile: a task is one column x 4 rows.  The 2 * IN_W tasks
-                // do not divide by the thread count: the tasks beyond the first THREADS are split into
-                // single pixels, so the second round costs one pixel per thread instead of four
-                constexpr int NT = 2 * C::IN_W, REM = NT > THREADS ? NT - THREADS : 0;
-                static_assert((G_RB / 2) * REM <= THREADS, "second producer round must fit one pass");
-                auto gather_px = [&](const typename Prod::Column &col, int i, int r) {
-                    float o0, o1, o2;
-                    prod.template at_row<true>(col, rawt + 16 + r * RAW_PITCH - a0, o0, o1, o2);
-                    S[0 * C::S_PLANE + r * C::S_PITCH + i] = o0;
-                    S[1 * C::S_PLANE + r * C::S_PITCH + i] = o1;
-                    if (NCH == 3) S[2 * C::S_PLANE + r * C::S_PITCH + i] = o2;
-                };
-                if (tid < NT) {
-                    const int half = tid / C::IN_W, i = tid - half * C::IN_W;
-                    const typename Prod::Column col = prod.column(reflect101(x0 - R + i, W));
-#pragma unroll
-                    for (int rr = 0; rr < G_RB / 2; ++rr) gather_px(col, i, half * (G_RB / 2) + rr);
+            // a task is a group of 4 pixels; the tasks beyond the first THREADS are split into single
+            // pixels (second round: one pixel per thread instead of four)
+            constexpr int NTG = G_RB * C::GROUPS, REMG_ALL = NTG > THREADS ? NTG - THREADS : 0;
+            // (measured: splitting pays while the remainder is small; with 56 left-over groups -- 29 taps --
+            // the byte-granular second round costs as much as it saves)
+            constexpr int REMG = REMG_ALL <= 32 ? REMG_ALL : 0;
+            const int sh = (a_byte - a0) & 3, w_off = (a_byte - a0) >> 2;
+            if (REMG > 0 && tid < 4 * REMG) {
+                const int idx = NTG - REMG + (tid >> 2), j = tid & 3;
+                const int r = idx / C::GROUPS, g = idx - r * C::GROUPS;
+                const uint8_t *q = rawt + r * RAW_PITCH + (a_byte - a0) + 3 * (4 * g + j);
+                const uint32_t b0 = q[0], b1 = q[1], b2 = q[2];
+                prod.seen |= b0 | b1 | b2;
+                float o0, o1, o2;
+                prod.px(b0, b1, b2, o0, o1, o2);
+                S[0 * C::S_PLANE + r * C::S_PITCH + 4 * g + j] = o0;
+                S[1 * C::S_PLANE + r * C::S_PITCH + 4 * g + j] = o1;
+                if (NCH == 3) S[2 * C::S_PLANE + r * C::S_PITCH + 4 * g + j] = o2;
+            }
+            for (int idx = tid; idx < NTG - REMG; idx += THREADS) {
+                const int r = idx / C::GROUPS, g = idx - r * C::GROUPS;
+                const uint32_t *q = reinterpret_cast<const uint32_t *>(rawt + r * RAW_PITCH) + w_off + 3 * g;
+                uint32_t w0 = q[0], w1 = q[1], w2 = q[2];
+                if (sh) {
+                    const uint32_t w3 = q[3];
+                    w0 = __funnelshift_r(w0, w1, 8 * sh);
+                    w1 = __funnelshift_r(w1, w2, 8 * sh);
+                    w2 = __funnelshift_r(w2, w3, 8 * sh);
                 }
-                if (REM > 0 && tid < (G_RB / 2) * REM) {
-                    const int idx = THREADS + tid / (G_RB / 2), rr = tid % (G_RB / 2);
-                    const int half = idx / C::IN_W, i = idx - half * C::IN_W;
-                    gather_px(prod.column(reflect101(x0 - R + i, W)), i, half * (G_RB / 2) + rr);
-                }
-            } else {
-                // a task is a group of 4 pixels; the tasks beyond the first THREADS are split into single
-                // pixels (second round: one pixel per thread instead of four)
-                constexpr int NTG = G_RB * C::GROUPS, REMG_ALL = NTG > THREADS ? NTG - THREADS : 0;
-                // (measured: splitting pays while the remainder is small; with 56 left-over groups -- 29 taps --
-                // the byte-granular second round costs as much as it saves)
-                constexpr int REMG = REMG_ALL <= 32 ? REMG_ALL : 0;
-                const int sh = (a_byte - a0) & 3, w_off = (a_byte - a0) >> 2;
-                if (REMG > 0 && tid < 4 * REMG) {
-                    const int idx = NTG - REMG + (tid >> 2), j = tid & 3;
-                    const int r = idx / C::GROUPS, g = idx - r * C::GROUPS;
-                    const uint8_t *q = rawt + r * RAW_PITCH + (a_byte - a0) + 3 * (4 * g + j);
-                    const uint32_t b0 = q[0], b1 = q[1], b2 = q[2];
-                    prod.seen |= b0 | b1 | b2;
-                    float o0, o1, o2;
-                    prod.px(b0, b1, b2, o0, o1, o2);
-                    S[0 * C::S_PLANE + r * C::S_PITCH + 4 * g + j] = o0;
-                    S[1 * C::S_PLANE + r * C::S_PITCH + 4 * g + j] = o1;
-                    if (NCH == 3) S[2 * C::S_PLANE + r * C::S_PITCH + 4 * g + j] = o2;
-                }
-                for (int idx = tid; idx < NTG - REMG; idx += THREADS) {
-                    const int r = idx / C::GROUPS, g = idx - r * C::GROUPS;
-                    const uint32_t *q = reinterpret_cast<const uint32_t *>(rawt + r * RAW_PITCH) + w_off + 3 * g;
-                    uint32_t w0 = q[0], w1 = q[1], w2 = q[2];
-                    if (sh) {
-                        const uint32_t w3 = q[3];
-                        w0 = __funnelshift_r(w0, w1, 8 * sh);
-                        w1 = __funnelshift_r(w1, w2, 8 * sh);
-                        w2 = __funnelshift_r(w2, w3, 8 * sh);
-                    }
-                    float4 c0, c1, c2;
-                    prod.decode4(w0, w1, w2, c0, c1, c2);
-                    *reinterpret_cast<float4 *>(&S[0 * C::S_PLANE + r * C::S_PITCH + 4 * g]) = c0;
-                    *reinterpret_cast<float4 *>(&S[1 * C::S_PLANE + r * C::S_PITCH + 4 * g]) = c1;
-                    if (NCH == 3) *reinterpret_cast<float4 *>(&S[2 * C::S_PLANE + r * C::S_PITCH + 4 * g]) = c2;
-                }
+                float4 c0, c1, c2;
+                prod.decode4(w0, w1, w2, c0, c1, c2);
+                *reinterpret_cast<float4 *>(&S[0 * C::S_PLANE + r * C::S_PITCH + 4 * g]) = c0;
+                *reinterpret_cast<float4 *>(&S[1 * C::S_PLANE + r * C::S_PITCH + 4 * g]) = c1;
+                if (NCH == 3) *reinterpret_cast<float4 *>(&S[2 * C::S_PLANE + r * C::S_PITCH + 4 * g]) = c2;
             }
         } else {
-            // pixel-by-pixel producer (image borders, unaligned frames, the cat warp): a task is one
-            // column x 4 rows, so per-column state (table loads, tap geometry) is set up once per 4 px
+            // pixel-by-pixel producer (image borders, unaligned frames): a task is one column x 4 rows
             for (int idx = tid; idx < 2 * C::IN_W; idx += THREADS) {
                 const int half = idx / C::IN_W, i = idx - half * C::IN_W;
-                const typename Prod::Column col = prod.column(reflect101(x0 - R + i, W));
+                const DogProducer::Column col = prod.column(reflect101(x0 - R + i, W));
 #pragma unroll
                 for (int rr = 0; rr < G_RB / 2; ++rr) {
                     const int r = half * (G_RB / 2) + rr;
@@ -510,90 +373,11 @@ gauss_stream_kernel(const __grid_constant__ GaussCommon p, const __grid_constant
             }
         }
         __syncthreads();
-
-        // ---- horizontal pass: 8 outputs per thread from a WIN-wide register window
-        {
-            const float4 *w4 = reinterpret_cast<const float4 *>(&S[ch * C::S_PLANE + h_r * C::S_PITCH + h_xg * 8]);
-            float v[4 * C::NW4];
-#pragma unroll
-            for (int q = 0; q < C::NW4; ++q) {
-                const float4 t = w4[q];
-                v[4 * q] = t.x; v[4 * q + 1] = t.y; v[4 * q + 2] = t.z; v[4 * q + 3] = t.w;
-            }
-            float acc[8];
-#pragma unroll
-            for (int j = 0; j < 8; ++j) acc[j] = 0.f;
-#pragma unroll
-            for (int k = 0; k <= 2 * R; ++k) {
-                const float tk = p.taps[k];
-#pragma unroll
-                for (int j = 0; j < 8; ++j) acc[j] = fmaf(tk, v[j + k], acc[j]);
-            }
-            float4 *d4 = reinterpret_cast<float4 *>(&X[ch * C::X_PLANE + h_r * C::X_PITCH + h_xg * 8]);
-            d4[0] = make_float4(acc[0], acc[1], acc[2], acc[3]);
-            d4[1] = make_float4(acc[4], acc[5], acc[6], acc[7]);
-        }
+        gauss_hpass<R>(p, S, X, ch, h_r, h_xg);
         __syncthreads();
-
-        // ---- vertical pass, one input row at a time: finish the oldest output row, advance the rest.
-        // Input row i (0-based in the segment) completes output row y_start + i - 2R.
-        {
-            const float *col = X + ch * C::X_PLANE + v_x;
-            float *ycol = Y + ch * C::X_PLANE + v_x;
-#pragma unroll
-            for (int r = 0; r < G_RB; ++r) {
-                const float h = col[r * C::X_PITCH];
-                ycol[r * C::X_PITCH] = fmaf(p.taps[2 * R], h, A[0]);
-#pragma unroll
-                for (int m = 0; m < 2 * R - 1; ++m) A[m] = fmaf(p.taps[2 * R - 1 - m], h, A[m + 1]);
-                A[2 * R - 1] = p.taps[0] * h;
-            }
-        }
+        gauss_vpass<R>(p, X, Y, ch, v_x, A);
         __syncthreads();
-
-        // ---- expand (two-plane mode) + encode + store: a task is 4 consecutive pixels of one row
-        // (12 bytes = three 32-bit stores); input row i = 8*ib + r -> output row y_start + i - 2R
-        {
-            const int oy0 = y_start + ib * G_RB - 2 * R;
-            for (int t = tid; t < G_RB * (G_TW / 4); t += THREADS) {
-                const int r = t >> 5, g4 = t & 31;
-                const int oy = oy0 + r;
-                if (oy < y_start || oy >= y_end) continue;
-                const int xo = x0 + 4 * g4;
-                if (xo >= W) continue;
-                const float4 a4 = *reinterpret_cast<const float4 *>(&Y[0 * C::X_PLANE + r * C::X_PITCH + 4 * g4]);
-                const float4 b4 = *reinterpret_cast<const float4 *>(&Y[1 * C::X_PLANE + r * C::X_PITCH + 4 * g4]);
-                float4 c4 = make_float4(0.f, 0.f, 0.f, 0.f);
-                if (NCH == 3) c4 = *reinterpret_cast<const float4 *>(&Y[2 * C::X_PLANE + r * C::X_PITCH + 4 * g4]);
-                const float av[4] = {a4.x, a4.y, a4.z, a4.w}, bv[4] = {b4.x, b4.y, b4.z, b4.w}, cv[4] = {c4.x, c4.y, c4.z, c4.w};
-                uint32_t by[12];
-#pragma unroll
-                for (int j = 0; j < 4; ++j) {
-                    float r0, r1, r2;
-                    if (NCH == 2) {
-                        r0 = fmaf(p.P[1], bv[j], p.P[0] * av[j]);
-                        r1 = fmaf(p.P[3], bv[j], p.P[2] * av[j]);
-                        r2 = fmaf(p.P[5], bv[j], p.P[4] * av[j]);
-                    } else {
-                        r0 = av[j]; r1 = bv[j]; r2 = cv[j];
-                    }
-                    by[3 * j] = encode_u8(enc, r0);
-                    by[3 * j + 1] = encode_u8(enc, r1);
-                    by[3 * j + 2] = encode_u8(enc, r2);
-                }
-                uint8_t *o = dst_frame + (int64_t)oy * p.io.out_rs + (int64_t)xo * 3;
-                if (out4 && xo + 3 < W) {
-                    uint32_t *o32 = reinterpret_cast<uint32_t *>(o);
-#pragma unroll
-                    for (int q = 0; q < 3; ++q) o32[q] = by[4 * q] | (by[4 * q + 1] << 8) | (by[4 * q + 2] << 16) | (by[4 * q + 3] << 24);
-                } else {
-                    const int nb = 3 * min(4, W - xo);
-#pragma unroll
-                    for (int q = 0; q < 12; ++q)
-                        if (q < nb) o[q] = (uint8_t)by[q];
-                }
-            }
-        }
+        gauss_encode_store<R, NCH, THREADS>(p, enc, Y, dst_frame, ib, y_start, y_end, x0, out4);
         // hazards: the next produce writes rawt / S (H pass done); X is rewritten after the next
         // produce barrier (V pass done); Y is rewritten after the next H-pass barrier (encode done).
     }
@@ -929,14 +713,14 @@ gauss_mma_kernel(const __grid_constant__ GaussCommon p, const __grid_constant__ 
     }
 }
 
-template <int R, class Prod, int NCH>
-static int launch_gauss(const GaussCommon &gc, const typename Prod::Params &pp, cudaStream_t st) {
+template <int R, int NCH>
+static int launch_gauss(const GaussCommon &gc, const DogProducer::Params &pp, cudaStream_t st) {
     using C = GaussCfg<R>;
-    const size_t smem = (size_t)(NCH * C::S_PLANE + 2 * NCH * C::X_PLANE + Prod::SMEM_FLOATS + G_ENC_SMEM) * 4 + 2 * (size_t)G_RB * Prod::RAW_PITCH;
-    auto kern = gauss_stream_kernel<R, Prod, NCH>;
+    const size_t smem = (size_t)(NCH * C::S_PLANE + 2 * NCH * C::X_PLANE + DogProducer::SMEM_FLOATS + G_ENC_SMEM) * 4 + 2 * (size_t)G_RB * DogProducer::RAW_PITCH;
+    auto kern = gauss_stream_kernel<R, NCH>;
     AVB_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     dim3 grid((gc.io.W + G_TW - 1) / G_TW, (gc.io.H + gc.seg_h - 1) / gc.seg_h, gc.io.n);
-    AVB_TIMED(gc.fixup ? Prod::fixup_name() : Prod::name(), st);
+    AVB_TIMED(gc.fixup ? DogProducer::fixup_name() : DogProducer::name(), st);
     kern<<<grid, G_THREADS_PER_PLANE * NCH, smem, st>>>(gc, pp);
     AVB_CUDA_OK(cudaGetLastError());
     return AVB_OK;
@@ -1095,28 +879,21 @@ static int dispatch_gauss_mma(int radius, GaussCommon gc, const DogProducer::Par
     return launch_gauss_mma<3, 2>(gc, q, geo, st);
 }
 
-template <class Prod>
-static int dispatch_gauss(int radius, GaussCommon &gc, typename Prod::Params &pp, cudaStream_t st) {
-#ifndef G_CAT_SEG_SLOTS
-#define G_CAT_SEG_SLOTS 3
-#endif
-    gc.seg_h = pick_seg_h(gc.io.n, gc.io.H, gc.io.W, radius, (Prod::GATHER && radius <= G_MINB4_R) ? G_CAT_SEG_SLOTS : (radius <= G_MINB3_R ? 3 : G_MINB));
+static int dispatch_gauss(int radius, GaussCommon &gc, const DogProducer::Params &pp, cudaStream_t st) {
+    gc.seg_h = pick_seg_h(gc.io.n, gc.io.H, gc.io.W, radius, radius <= G_MINB3_R ? 3 : G_MINB);
     float Q[6];
-    const float T[9] = {pp.M.m[0], pp.M.m[1], pp.M.m[2], pp.M.m[3], pp.M.m[4], pp.M.m[5], pp.M.m[6], pp.M.m[7], pp.M.m[8]};
-    const bool two = rank2_factor(T, Q, gc.P);
-    typename Prod::Params q = pp;
+    const bool two = rank2_factor(pp.M.m, Q, gc.P);
+    DogProducer::Params q = pp;
     if (two) {
         for (int i = 0; i < 6; ++i) q.M.m[i] = Q[i];
         q.M.m[6] = q.M.m[7] = q.M.m[8] = 0.f;
     }
-    constexpr bool dog = std::is_same<Prod, DogProducer>::value;
-    if constexpr (dog)
-        if (two && radius >= G_MMA_MIN_RADIUS && radius <= 16) return dispatch_gauss_mma(radius, gc, q, st);
-    // a rank-2 Dog matrix from G_MMA_MIN_RADIUS up never gets here: no two-plane instantiation for it
+    if (two && radius >= G_MMA_MIN_RADIUS && radius <= 16) return dispatch_gauss_mma(radius, gc, q, st);
+    // a rank-2 matrix from G_MMA_MIN_RADIUS up never gets here: no two-plane instantiation for it
     switch (radius) {
 #define AVB_CASE(RR) case RR: \
-        if constexpr (!(dog && RR >= G_MMA_MIN_RADIUS)) if (two) return launch_gauss<RR, Prod, 2>(gc, q, st); \
-        return launch_gauss<RR, Prod, 3>(gc, q, st);
+        if constexpr (RR < G_MMA_MIN_RADIUS) if (two) return launch_gauss<RR, 2>(gc, q, st); \
+        return launch_gauss<RR, 3>(gc, q, st);
         AVB_CASE(1) AVB_CASE(2) AVB_CASE(3) AVB_CASE(4) AVB_CASE(5) AVB_CASE(6) AVB_CASE(7) AVB_CASE(8)
         AVB_CASE(9) AVB_CASE(10) AVB_CASE(11) AVB_CASE(12) AVB_CASE(13) AVB_CASE(14) AVB_CASE(15) AVB_CASE(16)
 #undef AVB_CASE
@@ -1161,11 +938,11 @@ extern "C" int avb_dichromat_blur_u8(const uint8_t *in, uint8_t *out, int n, int
         gc.flags = flags_dev;
     }
     gc.fixup = 0;
-    if (int e = dispatch_gauss<DogProducer>(ksize / 2, gc, pp, st)) return e;
+    if (int e = dispatch_gauss(ksize / 2, gc, pp, st)) return e;
     if (norm_mode == AVB_NORM_AUTO) {
         gc.fixup = 1;
         pp.lut = dec_raw_dev;
-        if (int e = dispatch_gauss<DogProducer>(ksize / 2, gc, pp, st)) return e;
+        if (int e = dispatch_gauss(ksize / 2, gc, pp, st)) return e;
     }
     return AVB_OK;
 }
@@ -1202,6 +979,310 @@ __global__ void __launch_bounds__(256) frame_flags_kernel(FrameIO io, uint32_t *
     if (__any_sync(0xffffffffu, (seen & 0xfefefefeu) != 0) && (threadIdx.x & 31) == 0) flags[frame] = 1u;
 }
 
+// ------------------------------------------------------------------------------------ cat warp kernel
+// Binocular wide-FOV gather + blend + pow decode + 3x3 (animals/cat_widevision_utils.py:46-99, animals/cat.py:95-101)
+// -> separable Gaussian -> encode, in the strip / 8-row-block shape of gauss_stream_kernel and with its H pass, V pass
+// and encode.  Every map of the warp depends on the column only, so each CTA first turns the per-column tables into
+// one record per produced column in shared memory: the live eye view (a single one for every column of the default
+// geometry), the byte offset of its left tap, the two bilinear weights and the eye weight, the blend denominator and
+// its reciprocal.  A producer task is then one column x 8 rows.  Measured on a B200 at 1000 W, 20 4K frames:
+// 1.135 ms with the producer policy of gauss_stream_kernel (tables and tap geometry per 4 rows, both eyes' terms of the
+// blend), 0.993 ms here.
+//
+// cv::remap INTER_LINEAR: map coordinate quantised to 1/32 px, two taps, border constant 0.  A tap outside the
+// image gets weight 0 in the record instead of a zeroed sample: both products are +0 (samples are finite and >= 0),
+// so the sums are unchanged; its offset is clamped to [-1, W-1] so that it still reads bytes of the staged span.
+// A single live eye drops the other eye's terms of the blend: the skipped product is +0 added to a value >= +0.
+struct CatParams {
+    Mat3 M;             // RGB->LMS, L/M merge, LMS->RGB collapsed into one 3x3 (host, float64 -> f32)
+    const float *xl, *xr, *wl, *wr;  // per-column tables, length W (device)
+    const float *ws, *rws;           // per column: wl + wr + 1e-8 (float32) and its correctly rounded reciprocal
+    const uint32_t *frame_flags;     // per frame: != 0 when some byte >= 2 (written by frame_flags_kernel)
+    int norm_mode;                   // AVB_NORM_DIV255: always /255; AVB_NORM_AUTO: /255 iff flag set
+};
+
+constexpr int CAT_RAW_PITCH = 960;   // 16 B slack + 58 chunks of 16 B + slack: (128 + 2*16) columns x 2.1 source px x 3 B + alignment slack
+
+// record of one tap pair: {byte offset of the left tap (int bits), weight of the left tap, of the right tap, eye weight}
+__device__ __forceinline__ float4 cat_tap(float xs, float w_eye, int W, int &lo, int &hi) {
+    const int sx = __float2int_rn(xs * 32.0f);
+    const int ix = sx >> 5;
+    const float f = (float)(sx & 31) * (1.0f / 32.0f);
+    const float w0 = 1.0f - f;
+    const int ixc = min(max(ix, -1), W - 1);
+    lo = min(lo, ixc);
+    hi = max(hi, ixc + 1);
+    return make_float4(__int_as_float(3 * ixc), (unsigned)ix < (unsigned)W ? w0 : 0.f, (unsigned)(ix + 1) < (unsigned)W ? f : 0.f, w_eye);
+}
+
+// the two taps of one eye view, from a 4-byte aligned row (the shared raw tile, readable a few bytes past either end
+// of the span): the two source pixels are 6 contiguous bytes = three 32-bit loads + two funnel shifts
+__device__ __forceinline__ void cat_gather_words(const float *norm_s, const uint8_t *q, float w0, float f, float &c0, float &c1, float &c2) {
+    const uint32_t *w = reinterpret_cast<const uint32_t *>(reinterpret_cast<uintptr_t>(q) & ~(uintptr_t)3);
+    const uint32_t sh = (uint32_t)(reinterpret_cast<uintptr_t>(q) & 3) * 8;
+    const uint32_t v0 = w[0], v1 = w[1], v2 = w[2];
+    const uint32_t lo = __funnelshift_r(v0, v1, sh), hi = __funnelshift_r(v1, v2, sh);
+    const float a0 = norm_s[lo & 0xffu], a1 = norm_s[(lo >> 8) & 0xffu], a2 = norm_s[(lo >> 16) & 0xffu];
+    const float b0 = norm_s[lo >> 24], b1 = norm_s[hi & 0xffu], b2 = norm_s[(hi >> 8) & 0xffu];
+    c0 = __fadd_rn(__fmul_rn(a0, w0), __fmul_rn(b0, f));
+    c1 = __fadd_rn(__fmul_rn(a1, w0), __fmul_rn(b1, f));
+    c2 = __fadd_rn(__fmul_rn(a2, w0), __fmul_rn(b2, f));
+}
+// same from a global row: only taps inside the image (weight != 0) are read
+__device__ __forceinline__ void cat_gather_bytes(const float *norm_s, const uint8_t *q, float w0, float f, float &c0, float &c1, float &c2) {
+    float a0 = 0.f, a1 = 0.f, a2 = 0.f, b0 = 0.f, b1 = 0.f, b2 = 0.f;
+    if (w0 != 0.0f) { a0 = norm_s[q[0]]; a1 = norm_s[q[1]]; a2 = norm_s[q[2]]; }
+    if (f != 0.0f) { b0 = norm_s[q[3]]; b1 = norm_s[q[4]]; b2 = norm_s[q[5]]; }
+    c0 = __fadd_rn(__fmul_rn(a0, w0), __fmul_rn(b0, f));
+    c1 = __fadd_rn(__fmul_rn(a1, w0), __fmul_rn(b1, f));
+    c2 = __fadd_rn(__fmul_rn(a2, w0), __fmul_rn(b2, f));
+}
+
+__device__ __forceinline__ float cat_decode(float v) {
+    // animals/animal_utils.py:5-11 on float32; the power goes through the SFU (ex2(2.4 lg2 x),
+    // ~5e-7 relative: far inside the 1-LSB budget of the uint8 result)
+    // (arguments stay in [0.09, 1] and exponents in [-8.4, 0]: the .ftz SFU forms are exact enough
+    // and need no denormal scaling code around them)
+    float l, e;
+    asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(l) : "f"((v + 0.055f) * (1.0f / 1.055f)));
+    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(2.4f * l));
+    return v <= 0.04045f ? v * (1.0f / 12.92f) : e;
+}
+
+// blend numerators n -> quotient n / (wL + wR + 1e-8), correctly rounded from the per-column reciprocal (one Newton
+// step on the quotient) -> decode -> 3x3 (rows 0, 1 of Q in two-plane mode)
+__device__ __forceinline__ void cat_finish(const float (&m)[9], float n0, float n1, float n2, float s, float r, float &o0, float &o1, float &o2) {
+    float q0 = __fmul_rn(n0, r), q1 = __fmul_rn(n1, r), q2 = __fmul_rn(n2, r);
+    q0 = fmaf(fmaf(-q0, s, n0), r, q0);
+    q1 = fmaf(fmaf(-q1, s, n1), r, q1);
+    q2 = fmaf(fmaf(-q2, s, n2), r, q2);
+    const float s0 = cat_decode(__saturatef(q0)), s1 = cat_decode(__saturatef(q1)), s2 = cat_decode(__saturatef(q2));
+    o0 = m[0] * s0 + m[1] * s1 + m[2] * s2;
+    o1 = m[3] * s0 + m[4] * s1 + m[5] * s2;
+    o2 = m[6] * s0 + m[7] * s1 + m[8] * s2;
+}
+
+#ifndef CAT_MINB4_R
+#define CAT_MINB4_R 4
+#endif
+// two planes at radius <= 4 (the cat's own 9-tap blur): four CTAs per SM -- 60 registers, no spill, 55 KB of shared
+// memory per CTA (CUDA 12.9)
+template <int R, int NCH>
+struct CatOcc { static constexpr int MIN_BLOCKS = (NCH == 2 && R <= CAT_MINB4_R) ? 4 : GaussOcc<R, NCH>::MIN_BLOCKS; };
+
+template <int R, int NCH>
+__global__ void __launch_bounds__(G_THREADS_PER_PLANE * NCH, CatOcc<R, NCH>::MIN_BLOCKS)
+cat_warp_kernel(const __grid_constant__ GaussCommon p, const __grid_constant__ CatParams pp) {
+    using C = GaussCfg<R>;
+    constexpr int THREADS = G_THREADS_PER_PLANE * NCH;
+    static_assert(C::IN_W <= THREADS, "one column record per thread");
+    extern __shared__ __align__(16) uint8_t smem_raw[];
+    float *S = reinterpret_cast<float *>(smem_raw);            // [NCH][RB][S_PITCH] produced rows (+x halo)
+    float *X = S + NCH * C::S_PLANE;                           // [NCH][RB][X_PITCH] horizontally blurred rows
+    float *Y = X + NCH * C::X_PLANE;                           // [NCH][RB][X_PITCH] fully blurred rows
+    float *norm_s = Y + NCH * C::X_PLANE;                      // [256] normalised byte values
+    uint32_t *enc_s = reinterpret_cast<uint32_t *>(norm_s + 256);
+    float4 *rec_a = reinterpret_cast<float4 *>(enc_s + G_ENC_SMEM);                 // [IN_W] live eye (left eye if both live)
+    float4 *rec_b = rec_a + C::IN_W;                                                 // [IN_W] right eye if both live, else weight 0
+    float2 *rec_s = reinterpret_cast<float2 *>(rec_b + C::IN_W);                     // [IN_W] blend denominator, its reciprocal
+    uint8_t *rawt0 = reinterpret_cast<uint8_t *>(rec_s + C::IN_W);                   // [2][RB][RAW_PITCH] packed input rows (TMA double buffer)
+    constexpr int RAW_PITCH = CAT_RAW_PITCH;
+    __shared__ __align__(8) uint64_t rbar[2];                                       // completion of the bulk copies of each buffer
+    __shared__ int span[3];                                                         // source columns the strip's taps touch: lo, hi; eye mode
+
+    const int frame = blockIdx.z;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int H = p.io.H, W = p.io.W;
+    const int x0 = blockIdx.x * G_TW;
+    const int y_start = blockIdx.y * p.seg_h;
+    const int y_end = min(H, y_start + p.seg_h);
+    const uint8_t *src_frame = p.io.in + (int64_t)frame * p.io.in_fs;
+
+    // normalised byte values exactly as NumPy makes them: float32(v) / float32(255), or, when the
+    // frame max is <= 1 (get_normalized_image's other branch), the byte itself clipped to [0,1]
+    const bool div255 = pp.norm_mode == AVB_NORM_DIV255 || __ldg(pp.frame_flags + frame) != 0;
+    for (int i = tid; i < 256; i += THREADS) norm_s[i] = div255 ? __fdiv_rn((float)i, 255.0f) : fminf((float)i, 1.0f);
+    copy_to_smem(enc_s, p.enc, min(G_ENC_SMEM, ENC_HEADER + (int)__ldg(p.enc + 2)));
+    if (tid == 0) {
+        span[0] = 0x7fffffff; span[1] = -1; span[2] = 0;
+        gauss_mbar_init(&rbar[0], G_RB);
+        gauss_mbar_init(&rbar[1], G_RB);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+    if (tid < C::IN_W) {
+        const int x = reflect101(x0 - R + tid, W);
+        const float wL = __ldg(pp.wl + x), wR = __ldg(pp.wr + x);
+        int lo = 0x7fffffff, hi = -1, mode = 0;
+        float4 a = make_float4(0.f, 0.f, 0.f, 0.f), b = a;
+        if (wL != 0.0f) { a = cat_tap(__ldg(pp.xl + x), wL, W, lo, hi); mode |= 1; }
+        if (wR != 0.0f) {
+            const float4 t = cat_tap(__ldg(pp.xr + x), wR, W, lo, hi);
+            if (mode) { b = t; mode |= 4; } else { a = t; }
+            mode |= 2;
+        }
+        rec_a[tid] = a;
+        rec_b[tid] = b;
+        rec_s[tid] = make_float2(__ldg(pp.ws + x), __ldg(pp.rws + x));
+        if (mode) { atomicMin(&span[0], lo); atomicMax(&span[1], hi); atomicOr(&span[2], mode); }
+    }
+    __syncthreads();
+    const EncTable enc = enc_view(enc_s);
+    uint8_t *dst_frame = p.io.out + (int64_t)frame * p.io.out_fs;
+
+    // a strip outside both eye views (the blind middle third) is identically zero and encodes to byte 0
+    if (span[2] == 0) {
+        const bool vec_ok = (x0 + G_TW <= W) && ((p.io.out_rs & 15) == 0) && ((p.io.out_fs & 15) == 0) &&
+                            ((reinterpret_cast<uintptr_t>(p.io.out) & 15) == 0);
+        const int nbytes = min(G_TW, W - x0) * 3;
+        for (int y = y_start + warp; y < y_end; y += THREADS / 32) {
+            uint8_t *row = dst_frame + (int64_t)y * p.io.out_rs + (int64_t)x0 * 3;
+            if (vec_ok) {
+                if (lane < G_TW * 3 / 16) reinterpret_cast<uint4 *>(row)[lane] = make_uint4(0u, 0u, 0u, 0u);
+            } else {
+                for (int b = lane; b < nbytes; b += 32) row[b] = 0;
+            }
+        }
+        return;
+    }
+
+    // Raw tile: the packed bytes [a0, a0 + 16*n_chunks) of 8 input rows -- the source columns the strip's taps touch
+    // -- fetched with 16-byte loads one block ahead, 16 bytes into each tile row.  Strips with a single live eye view
+    // only; the others (and unaligned frames) gather from global memory.
+    const bool out4 = ((p.io.out_rs & 3) == 0) && ((p.io.out_fs & 3) == 0) && ((reinterpret_cast<uintptr_t>(p.io.out) & 3) == 0);
+    const bool in16 = ((p.io.in_rs & 15) == 0) && ((p.io.in_fs & 15) == 0) && ((reinterpret_cast<uintptr_t>(p.io.in) & 15) == 0);
+    const int ixlo = max(span[0], 0), ixhi = min(span[1], W - 1);
+    const int a0 = (3 * ixlo) & ~15;
+    const int n_chunks = (3 * (ixhi + 1) - a0 + 15) >> 4;
+    const bool vec_in = (span[2] == 1 || span[2] == 2) && in16 && n_chunks > 0 && 16 * n_chunks + 32 <= RAW_PITCH &&
+                        a0 + 16 * n_chunks <= (int)p.io.in_rs;
+
+    const int n_in_rows = (y_end - y_start) + 2 * R;
+    const int n_in_blocks = (n_in_rows + G_RB - 1) / G_RB;
+
+    const int ch = tid >> 7;                         // 128 threads per plane
+    const int h_r = tid & 7, h_xg = (tid & 127) >> 3;
+    const int v_x = tid & 127;
+    float A[2 * R];                                  // partial sums of the 2R output rows in flight
+#pragma unroll
+    for (int i = 0; i < 2 * R; ++i) A[i] = 0.f;
+    float m[9];
+#pragma unroll
+    for (int i = 0; i < 9; ++i) m[i] = pp.M.m[i];
+
+    auto raw_issue = [&](int yb_, int buf) {
+        if (tid < G_RB) {
+            const uint8_t *g = src_frame + (int64_t)reflect101(yb_ + tid, H) * p.io.in_rs + a0;
+            gauss_bulk_load(rawt0 + buf * (G_RB * RAW_PITCH) + 16 + tid * RAW_PITCH, g, 16u * (uint32_t)n_chunks, &rbar[buf]);
+        }
+    };
+    uint32_t rphase = 0;                             // bit b: parity the next wait on buffer b expects
+    if (vec_in) raw_issue(y_start - R, 0);
+
+    auto store = [&](int r, int i, float o0, float o1, float o2) {
+        S[0 * C::S_PLANE + r * C::S_PITCH + i] = o0;
+        S[1 * C::S_PLANE + r * C::S_PITCH + i] = o1;
+        if (NCH == 3) S[2 * C::S_PLANE + r * C::S_PITCH + i] = o2;
+    };
+
+    for (int ib = 0; ib < n_in_blocks; ++ib) {
+        const int yb = y_start - R + ib * G_RB;      // first input row of this block
+        // ---- produce RB rows x IN_W columns of linear-light values: a task is one column x 8 rows
+        if (vec_in) {
+            // the packed rows of this block were requested one block ahead: wait for the copies, then put
+            // the next block's copies in flight (its buffer was last read two barriers ago)
+            const int buf = ib & 1;
+            gauss_mbar_wait(&rbar[buf], (rphase >> buf) & 1u);
+            rphase ^= 1u << buf;
+            if (ib + 1 < n_in_blocks) raw_issue(yb + G_RB, buf ^ 1);
+            if (tid < C::IN_W) {
+                const float4 a = rec_a[tid];
+                if (a.w == 0.0f) {                   // outside both eye views: (0*wL + 0*wR)/ws = 0 -> decode(0) = 0
+#pragma unroll
+                    for (int r = 0; r < G_RB; ++r) store(r, tid, 0.f, 0.f, 0.f);
+                } else {
+                    const float2 sr = rec_s[tid];
+                    const uint8_t *q = rawt0 + buf * (G_RB * RAW_PITCH) + 16 + (__float_as_int(a.x) - a0);
+#pragma unroll
+                    for (int r = 0; r < G_RB; ++r) {
+                        float c0, c1, c2, o0, o1, o2;
+                        cat_gather_words(norm_s, q + r * RAW_PITCH, a.y, a.z, c0, c1, c2);
+                        cat_finish(m, __fmul_rn(c0, a.w), __fmul_rn(c1, a.w), __fmul_rn(c2, a.w), sr.x, sr.y, o0, o1, o2);
+                        store(r, tid, o0, o1, o2);
+                    }
+                }
+            }
+        } else {
+            // unaligned frames, strips that see both eye views: gather from global memory
+            if (tid < C::IN_W) {
+                const float4 a = rec_a[tid], b = rec_b[tid];
+                const float2 sr = rec_s[tid];
+                for (int r = 0; r < G_RB; ++r) {
+                    float o0 = 0.f, o1 = 0.f, o2 = 0.f;
+                    if (a.w != 0.0f) {
+                        const uint8_t *row = src_frame + (int64_t)reflect101(yb + r, H) * p.io.in_rs;
+                        float l0, l1, l2;
+                        cat_gather_bytes(norm_s, row + __float_as_int(a.x), a.y, a.z, l0, l1, l2);
+                        float n0 = __fmul_rn(l0, a.w), n1 = __fmul_rn(l1, a.w), n2 = __fmul_rn(l2, a.w);
+                        if (b.w != 0.0f) {
+                            float r0, r1, r2;
+                            cat_gather_bytes(norm_s, row + __float_as_int(b.x), b.y, b.z, r0, r1, r2);
+                            n0 = __fadd_rn(n0, __fmul_rn(r0, b.w));
+                            n1 = __fadd_rn(n1, __fmul_rn(r1, b.w));
+                            n2 = __fadd_rn(n2, __fmul_rn(r2, b.w));
+                        }
+                        cat_finish(m, n0, n1, n2, sr.x, sr.y, o0, o1, o2);
+                    }
+                    store(r, tid, o0, o1, o2);
+                }
+            }
+        }
+        __syncthreads();
+        gauss_hpass<R>(p, S, X, ch, h_r, h_xg);
+        __syncthreads();
+        gauss_vpass<R>(p, X, Y, ch, v_x, A);
+        __syncthreads();
+        gauss_encode_store<R, NCH, THREADS>(p, enc, Y, dst_frame, ib, y_start, y_end, x0, out4);
+    }
+}
+
+template <int R, int NCH>
+static int launch_cat(const GaussCommon &gc, const CatParams &pp, cudaStream_t st) {
+    using C = GaussCfg<R>;
+    const size_t smem = (size_t)(NCH * C::S_PLANE + 2 * NCH * C::X_PLANE + 256 + G_ENC_SMEM) * 4 + (size_t)C::IN_W * (16 + 16 + 8) +
+                        2 * (size_t)G_RB * CAT_RAW_PITCH;
+    auto kern = cat_warp_kernel<R, NCH>;
+    AVB_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    dim3 grid((gc.io.W + G_TW - 1) / G_TW, (gc.io.H + gc.seg_h - 1) / gc.seg_h, gc.io.n);
+    AVB_TIMED("k2_gauss_cat_warp", st);
+    kern<<<grid, G_THREADS_PER_PLANE * NCH, smem, st>>>(gc, pp);
+    AVB_CUDA_OK(cudaGetLastError());
+    return AVB_OK;
+}
+
+static int dispatch_cat(int radius, GaussCommon &gc, const CatParams &pp, cudaStream_t st) {
+#ifndef G_CAT_SEG_SLOTS
+#define G_CAT_SEG_SLOTS 3
+#endif
+    gc.seg_h = pick_seg_h(gc.io.n, gc.io.H, gc.io.W, radius, radius <= CAT_MINB4_R ? G_CAT_SEG_SLOTS : (radius <= G_MINB3_R ? 3 : G_MINB));
+    float Q[6];
+    const bool two = rank2_factor(pp.M.m, Q, gc.P);
+    CatParams q = pp;
+    if (two) {
+        for (int i = 0; i < 6; ++i) q.M.m[i] = Q[i];
+        q.M.m[6] = q.M.m[7] = q.M.m[8] = 0.f;
+    }
+    switch (radius) {
+#define AVB_CASE(RR) case RR: return two ? launch_cat<RR, 2>(gc, q, st) : launch_cat<RR, 3>(gc, q, st);
+        AVB_CASE(1) AVB_CASE(2) AVB_CASE(3) AVB_CASE(4) AVB_CASE(5) AVB_CASE(6) AVB_CASE(7) AVB_CASE(8)
+        AVB_CASE(9) AVB_CASE(10) AVB_CASE(11) AVB_CASE(12) AVB_CASE(13) AVB_CASE(14) AVB_CASE(15) AVB_CASE(16)
+#undef AVB_CASE
+        default:
+            set_error("gaussian radius %d unsupported (ksize must be odd, 3..33)", radius);
+            return AVB_E_UNSUPPORTED;
+    }
+}
+
 // Centre zoom (cat_widevision_utils.py:11-29): crop + cv2.resize(INTER_LINEAR) on uint8, restated
 // in OpenCV's 11-bit fixed point so the result is bit-exact.  tab = W x int4 {xi0, xi1, xw0, xw1}
 // then H x int4 {yi0, yi1, yw0, yw1} (source indices already include the crop origin).
@@ -1225,7 +1306,9 @@ __device__ __forceinline__ void zoom_taps(const uint32_t *row32, int xi0, int la
 #endif
 constexpr int ZOOM_ROWS = ZOOM_ROWS_N;
 #ifndef ZOOM_MINB
-#define ZOOM_MINB 6      // 85 registers, 24 warps per SM (measured, 20 4K frames: 4 -> 0.471 ms, 6 -> 0.406, 8 -> 0.464)
+// 24 warps per SM (measured, 20 4K frames: 4 -> 0.471 ms, 6 -> 0.406, 8 -> 0.464).  CUDA 12.9 fits it in 80 registers with
+// 112 B of spill stores; five CTAs per SM (96 registers, no spill) measured slower on a B200 at 1000 W: 0.437 against 0.409 ms
+#define ZOOM_MINB 6
 #endif
 __global__ void __launch_bounds__(128, ZOOM_MINB) center_zoom_kernel(FrameIO io, const int32_t *__restrict__ tab, int aligned_out, int aligned_in) {
     const int W = io.W, H = io.H;
@@ -1372,21 +1455,21 @@ extern "C" int avb_cat_u8(const uint8_t *in, uint8_t *out_human, uint8_t *out_ca
             gc.flags = flags_dev;
         }
         gc.fixup = 0;
-        if (int e = dispatch_gauss<DogProducer>(ksize / 2, gc, dp, st)) return e;
+        if (int e = dispatch_gauss(ksize / 2, gc, dp, st)) return e;
         if (norm_mode == AVB_NORM_AUTO) {
             gc.fixup = 1;
             dp.lut = dec_raw_dev;
-            if (int e = dispatch_gauss<DogProducer>(ksize / 2, gc, dp, st)) return e;
+            if (int e = dispatch_gauss(ksize / 2, gc, dp, st)) return e;
         }
         return AVB_OK;
     }
-    gc.flags = nullptr;   // the producer does not see every pixel: normalisation comes from frame_flags_kernel
+    gc.flags = nullptr;   // the warp does not see every pixel: normalisation comes from frame_flags_kernel
     gc.fixup = 0;
-    CatProducer::Params pp{};
+    CatParams pp{};
     for (int i = 0; i < 9; ++i) pp.M.m[i] = m_host[i];
     pp.xl = warp_dev; pp.xr = warp_dev + W; pp.wl = warp_dev + 2 * W; pp.wr = warp_dev + 3 * W;
     pp.ws = warp_dev + 4 * W; pp.rws = warp_dev + 5 * W;
     pp.frame_flags = flags_dev;
     pp.norm_mode = norm_mode;
-    return dispatch_gauss<CatProducer>(ksize / 2, gc, pp, st);
+    return dispatch_cat(ksize / 2, gc, pp, st);
 }

@@ -15,7 +15,7 @@ import sys
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 # substring of the CUDA kernel name -> name used by AVB_TIMED / bench.py
-NAMES = [("DogProducer", "k2_gauss_dichromat"), ("CatProducer", "k2_gauss_cat_warp"), ("center_zoom", "cat_center_zoom"),
+NAMES = [("DogProducer", "k2_gauss_dichromat"), ("cat_warp_kernel", "k2_gauss_cat_warp"), ("center_zoom", "cat_center_zoom"),
          ("tcblur", "k2_tcblur"), ("frame_flags", "frame_flags"),
          ("uv_stats", "k3_uv_stats"), ("uv_hist", "k3_uv_hist"), ("uv_compact", "k3_uv_compact"), ("uv_map", "k3_uv_map"),
          ("uv_prep", "k3_uv_prep"), ("uv_scan", "k3_uv_scan"), ("uv_select", "k3_uv_select"), ("uv_fused", "k3_uv_fused"),
