@@ -16,7 +16,7 @@ from . import _build
 _lock = threading.Lock()
 _lib = None
 
-AVB_VERSION = 160         # include/avb200.h AVB_VERSION
+AVB_VERSION = 170         # include/avb200.h AVB_VERSION
 AVB_JPEG_HEADER_MAX = 1024
 AVB_PNG_HEADER_LEN = 35
 AVB_NORM_DIV255 = 0
@@ -68,6 +68,8 @@ SIGNATURES = {
     "avb_jpeg_bound_bytes": (_i64, [_i, _i]),
     "avb_jpeg_workspace_bytes": (_i64, [_i, _i, _i]),
     "avb_jpeg_encode_u8": (_i, [_p, _i, _i, _i, _i64, _i64, _p, _i, _p, _p, _i64, _p, _p, _p]),
+    "avb_jpeg_encode_rgb_u8": (_i, [_p, _i, _i, _i, _i64, _i64, _p, _i, _p, _p, _i64, _p, _p, _p]),
+    "avb_mjpeg_pack_u8": (_i, [_p, _i64, _p, _i, _p, _p, _p]),
     "avb_png_bound_bytes": (_i64, [_i, _i]),
     "avb_png_workspace_bytes": (_i64, [_i, _i, _i]),
     "avb_png_encode_u8": (_i, [_p, _i, _i, _i, _i64, _i64, _p, _i, _p, _i64, _p, _p, _p]),

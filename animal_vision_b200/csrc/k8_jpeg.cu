@@ -1,7 +1,7 @@
 // K8 -- batched baseline JPEG encoder, byte-identical to cv2.imencode(".jpg") with OpenCV's defaults
 // (libjpeg-turbo: 4:2:0, standard Huffman tables, no restart interval).  Every stage is integer arithmetic, so
 // the device restates libjpeg bit for bit (oracle/jpeg.py is the NumPy statement of the same stages):
-//   jpeg_transform  one CTA per strip of 8 MCUs (16 x 128 px): BGR gather with edge replication, jccolor.c
+//   jpeg_transform  one CTA per strip of 8 MCUs (16 x 128 px): BGR (or RGB) gather with edge replication, jccolor.c
 //                   fixed-point YCbCr, jcsample.c h2v2 (bias 1, 2), jfdctint.c islow, jcdctmgr.c quantisation,
 //                   jccoefct.c dummy blocks; writes zigzag int16 coefficients, quantised DCs and per-block
 //                   code lengths (the DC code of blocks 0 / Cb / Cr waits for the previous MCU's DCs)
@@ -179,6 +179,8 @@ __device__ __forceinline__ void fdct8(const int *d, int *o) {
     o[1] = descale(t7 + z1 + z4, SH);
 }
 
+// RGB: the frames hold R, G, B (avb_jpeg_encode_rgb_u8); everything after the gather is shared
+template <bool RGB>
 __global__ void __launch_bounds__(TF_THREADS) jpeg_transform_kernel(const uint8_t *__restrict__ in, int64_t fs, int64_t rs,
                                                                      Geo g, QDiv qd, Work w) {
     __shared__ uint8_t sY[16][128], sCb[16][128], sCr[16][128], sC[2][8][64];
@@ -194,7 +196,7 @@ __global__ void __launch_bounds__(TF_THREADS) jpeg_transform_kernel(const uint8_
         const int r = p >> 7, c = p & 127;
         const int gy = min(my * 16 + r, g.H - 1), gx = min(mx0 * 16 + c, g.W - 1);
         const uint8_t *px = fin + gy * rs + gx * 3;
-        const int b = px[0], gg = px[1], rr = px[2];              // BGR
+        const int b = px[RGB ? 2 : 0], gg = px[1], rr = px[RGB ? 0 : 2];
         sY[r][c] = (uint8_t)((19595 * rr + 38470 * gg + 7471 * b + 32768) >> 16);
         sCb[r][c] = (uint8_t)((-11059 * rr - 21709 * gg + 32768 * b + (128 << 16) + 32767) >> 16);
         sCr[r][c] = (uint8_t)((32768 * rr - 27439 * gg - 5329 * b + (128 << 16) + 32767) >> 16);
@@ -552,24 +554,35 @@ extern "C" int64_t avb_jpeg_workspace_bytes(int n, int H, int W) {
     return carve(geometry(H, W), n, nullptr, nullptr);
 }
 
-extern "C" int avb_jpeg_encode_u8(const uint8_t *in, int n, int H, int W, int64_t in_frame_stride, int64_t in_row_stride,
-                                  const uint8_t *header_host, int header_len, const uint8_t *qtables_host, uint8_t *out,
-                                  int64_t out_slot_stride, int64_t *out_lengths_dev, void *workspace_dev,
-                                  avb_stream_t stream) {
-    AVB_REQUIRE(in && header_host && qtables_host && out && out_lengths_dev && workspace_dev, "null pointer");
-    AVB_REQUIRE(n >= 1 && n <= 65535 && dims_ok(H, W), "n must lie in [1, 65535], H and W in [1, 65535]");
-    AVB_REQUIRE(in_row_stride >= 3LL * W && (n == 1 || in_frame_stride >= in_row_stride * (H - 1) + 3LL * W),
+namespace {
+
+// AVB_REQUIRE with the name of the entry point that was called
+#define K8_REQUIRE(cond, msg)                   \
+    do {                                        \
+        if (!(cond)) {                          \
+            avb::set_error("%s: %s", fn, msg);  \
+            return AVB_E_ARG;                   \
+        }                                       \
+    } while (0)
+
+template <bool RGB>
+int encode(const char *fn, const uint8_t *in, int n, int H, int W, int64_t in_frame_stride, int64_t in_row_stride,
+           const uint8_t *header_host, int header_len, const uint8_t *qtables_host, uint8_t *out, int64_t out_slot_stride,
+           int64_t *out_lengths_dev, void *workspace_dev, avb_stream_t stream) {
+    K8_REQUIRE(in && header_host && qtables_host && out && out_lengths_dev && workspace_dev, "null pointer");
+    K8_REQUIRE(n >= 1 && n <= 65535 && dims_ok(H, W), "n must lie in [1, 65535], H and W in [1, 65535]");
+    K8_REQUIRE(in_row_stride >= 3LL * W && (n == 1 || in_frame_stride >= in_row_stride * (H - 1) + 3LL * W),
                 "input strides overlap");
-    AVB_REQUIRE(header_len >= 2 && header_len <= AVB_JPEG_HEADER_MAX, "header_len must lie in [2, AVB_JPEG_HEADER_MAX]");
-    AVB_REQUIRE(out_slot_stride >= avb_jpeg_bound_bytes(H, W), "output slot smaller than avb_jpeg_bound_bytes(H, W)");
-    AVB_REQUIRE(((uintptr_t)workspace_dev & 15) == 0, "workspace must be 16-byte aligned");
+    K8_REQUIRE(header_len >= 2 && header_len <= AVB_JPEG_HEADER_MAX, "header_len must lie in [2, AVB_JPEG_HEADER_MAX]");
+    K8_REQUIRE(out_slot_stride >= avb_jpeg_bound_bytes(H, W), "output slot smaller than avb_jpeg_bound_bytes(H, W)");
+    K8_REQUIRE(((uintptr_t)workspace_dev & 15) == 0, "workspace must be 16-byte aligned");
     const Geo g = geometry(H, W);
-    AVB_REQUIRE(g.mh <= 65535, "too many MCU rows");
+    K8_REQUIRE(g.mh <= 65535, "too many MCU rows");
     QDiv qd;
     for (int t = 0; t < 2; ++t)
         for (int zz = 0; zz < 64; ++zz) {
             const int q = qtables_host[t * 64 + zz];
-            AVB_REQUIRE(q >= 1, "quantiser entries must lie in [1, 255]");
+            K8_REQUIRE(q >= 1, "quantiser entries must lie in [1, 255]");
         }
     static const uint8_t zigzag[64] = {0,  1,  8,  16, 9,  2,  3,  10, 17, 24, 32, 25, 18, 11, 4,  5,  12, 19, 26, 33, 40, 48,
                                        41, 34, 27, 20, 13, 6,  7,  14, 21, 28, 35, 42, 49, 56, 57, 50, 43, 36, 29, 22, 15, 23,
@@ -584,8 +597,8 @@ extern "C" int avb_jpeg_encode_u8(const uint8_t *in, int n, int H, int W, int64_
     const int grid = avb::sm_count() * 4;
     {
         AVB_TIMED("jpeg_transform", st);
-        jpeg_transform_kernel<<<dim3((g.mw + STRIP - 1) / STRIP, g.mh, n), TF_THREADS, 0, st>>>(in, in_frame_stride,
-                                                                                              in_row_stride, g, qd, w);
+        jpeg_transform_kernel<RGB><<<dim3((g.mw + STRIP - 1) / STRIP, g.mh, n), TF_THREADS, 0, st>>>(in, in_frame_stride,
+                                                                                                   in_row_stride, g, qd, w);
     }
     {
         AVB_TIMED("jpeg_mcu_scan", st);
@@ -613,4 +626,24 @@ extern "C" int avb_jpeg_encode_u8(const uint8_t *in, int n, int H, int W, int64_
     }
     AVB_CUDA_OK(cudaGetLastError());
     return AVB_OK;
+}
+
+#undef K8_REQUIRE
+
+}  // namespace
+
+extern "C" int avb_jpeg_encode_u8(const uint8_t *in, int n, int H, int W, int64_t in_frame_stride, int64_t in_row_stride,
+                                  const uint8_t *header_host, int header_len, const uint8_t *qtables_host, uint8_t *out,
+                                  int64_t out_slot_stride, int64_t *out_lengths_dev, void *workspace_dev,
+                                  avb_stream_t stream) {
+    return encode<false>(__func__, in, n, H, W, in_frame_stride, in_row_stride, header_host, header_len, qtables_host,
+                         out, out_slot_stride, out_lengths_dev, workspace_dev, stream);
+}
+
+extern "C" int avb_jpeg_encode_rgb_u8(const uint8_t *in, int n, int H, int W, int64_t in_frame_stride,
+                                      int64_t in_row_stride, const uint8_t *header_host, int header_len,
+                                      const uint8_t *qtables_host, uint8_t *out, int64_t out_slot_stride,
+                                      int64_t *out_lengths_dev, void *workspace_dev, avb_stream_t stream) {
+    return encode<true>(__func__, in, n, H, W, in_frame_stride, in_row_stride, header_host, header_len, qtables_host,
+                        out, out_slot_stride, out_lengths_dev, workspace_dev, stream);
 }

@@ -1,4 +1,4 @@
-"""Device JPEG encode (K8, include/avb200.h avb_jpeg_encode_u8): the bytes of
+"""Device JPEG encode (K8, include/avb200.h avb_jpeg_encode_u8 / avb_jpeg_encode_rgb_u8): the bytes of
 `cv2.imencode(".jpg", frame, [cv2.IMWRITE_JPEG_QUALITY, quality])` for a batch of frames, computed on the GPU.
 Only the compressed bytes cross to the host."""
 from __future__ import annotations
@@ -13,26 +13,53 @@ from ._slots import encode_slots
 from .engine import _fptr, get_engine
 
 
-def encode_jpeg(frames, quality: int = 95) -> List[bytes]:
-    """frames: CUDA uint8 tensor [N,H,W,3] in the channel order cv2.imencode expects (BGR), packed pixels, any row
-    and frame strides.  Runs on the current stream; returns one JPEG file per frame."""
+JPEG_LAUNCHES = 7                 # kernels one K8 encode launches (csrc/k8_jpeg.cu)
+
+
+def check_quality(quality, what: str = "encode_jpeg") -> int:
+    if isinstance(quality, bool) or not isinstance(quality, (int, np.integer)) or not 1 <= int(quality) <= 100:
+        raise AvbError(f"{what}: quality must be an integer in [1, 100], got {quality!r}")
+    return int(quality)
+
+
+class JpegLauncher:
+    """K8 for frames of one shape and quality: the header and quantiser tables built once, the sizes of the slots and
+    the workspace, and `launch` of n frames on the current stream."""
+
+    def __init__(self, lib, h: int, w: int, quality: int, rgb: bool):
+        if not (1 <= h <= 65535 and 1 <= w <= 65535):
+            raise AvbError(f"encode_jpeg: frame size {h}x{w} outside [1, 65535]^2")
+        self.lib, self.h, self.w = lib, h, w
+        self.header = np.frombuffer(tables.jpeg_header(h, w, quality), np.uint8)
+        self.qt = np.ascontiguousarray(tables.jpeg_quant_tables(quality))
+        self.fn = lib.avb_jpeg_encode_rgb_u8 if rgb else lib.avb_jpeg_encode_u8
+        self.name = "avb_jpeg_encode_rgb_u8" if rgb else "avb_jpeg_encode_u8"
+        self.slot = int(lib.avb_jpeg_bound_bytes(h, w))
+
+    def workspace_bytes(self, n: int) -> int:
+        return int(self.lib.avb_jpeg_workspace_bytes(n, self.h, self.w))
+
+    def launch(self, frames_ptr: int, n: int, fs: int, rs: int, ws: int, out: int, slot: int, lengths: int,
+               stream: int) -> int:
+        return self.fn(frames_ptr, n, self.h, self.w, fs, rs, _fptr(self.header), int(self.header.size), _fptr(self.qt),
+                       out, slot, lengths, ws, stream)
+
+
+def encode_jpeg(frames, quality: int = 95, *, rgb: bool = False) -> List[bytes]:
+    """frames: CUDA uint8 tensor [N,H,W,3] in the channel order cv2.imencode expects (BGR), or in RGB order with
+    `rgb=True` (the bytes of cv2.imencode of `frame[..., ::-1]`); packed pixels, any row and frame strides.  Runs on the
+    current stream; returns one JPEG file per frame."""
     import torch
     if not (isinstance(frames, torch.Tensor) and frames.is_cuda):
         raise AvbError("encode_jpeg: expected a CUDA uint8 tensor [N,H,W,3]")
-    if isinstance(quality, bool) or not isinstance(quality, (int, np.integer)) or not 1 <= int(quality) <= 100:
-        raise AvbError(f"encode_jpeg: quality must be an integer in [1, 100], got {quality!r}")
+    quality = check_quality(quality)
     eng = get_engine(frames.device)
     n, h, w, fs, rs = eng.check_frames(frames)
     if n == 0:
         return []
-    if not (1 <= h <= 65535 and 1 <= w <= 65535):
-        raise AvbError(f"encode_jpeg: frame size {h}x{w} outside [1, 65535]^2")
-    header = np.frombuffer(tables.jpeg_header(h, w, int(quality)), np.uint8)
-    qt = np.ascontiguousarray(tables.jpeg_quant_tables(int(quality)))
+    k8 = JpegLauncher(eng.lib, h, w, quality, bool(rgb))
     with torch.cuda.device(eng.device):
-        lib = eng.lib
         return encode_slots(
-            eng, "jpeg", n, int(lib.avb_jpeg_bound_bytes(h, w)), int(lib.avb_jpeg_workspace_bytes(n, h, w)),
-            lambda ws, out, slot, lengths: lib.avb_jpeg_encode_u8(
-                frames.data_ptr(), n, h, w, fs, rs, _fptr(header), int(header.size), _fptr(qt), out, slot, lengths, ws,
-                eng.stream_ptr()), 7)
+            eng, "jpeg", n, k8.slot, k8.workspace_bytes(n),
+            lambda ws, out, slot, lengths: k8.launch(frames.data_ptr(), n, fs, rs, ws, out, slot, lengths,
+                                                     eng.stream_ptr()), JPEG_LAUNCHES)

@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define AVB_VERSION 160            /* 0.1.6 */
+#define AVB_VERSION 170            /* 0.1.7 */
 
 #define AVB_OK 0
 #define AVB_E_ARG (-1)             /* bad argument (null pointer, non-positive size, unsupported radius ...) */
@@ -365,6 +365,22 @@ AVB_API int64_t avb_jpeg_workspace_bytes(int n, int H, int W);
 AVB_API int avb_jpeg_encode_u8(const uint8_t *in, int n, int H, int W, int64_t in_frame_stride, int64_t in_row_stride,
                                const uint8_t *header_host, int header_len, const uint8_t *qtables_host, uint8_t *out,
                                int64_t out_slot_stride, int64_t *out_lengths_dev, void *workspace_dev, avb_stream_t stream);
+/* The same for frames in RGB order: the bytes of cv2.imencode(".jpg", frame[..., ::-1], [IMWRITE_JPEG_QUALITY, q]).
+ * Arguments as avb_jpeg_encode_u8. */
+AVB_API int avb_jpeg_encode_rgb_u8(const uint8_t *in, int n, int H, int W, int64_t in_frame_stride,
+                                   int64_t in_row_stride, const uint8_t *header_host, int header_len,
+                                   const uint8_t *qtables_host, uint8_t *out, int64_t out_slot_stride,
+                                   int64_t *out_lengths_dev, void *workspace_dev, avb_stream_t stream);
+
+/* ---- K11: Motion-JPEG AVI records (csrc/k11_mjpeg.cu) ----------------------------------------------------------
+ * Packs n encoded files, file f at slots + f * slot_stride and lengths_dev[f] bytes long (device int64, e.g. the slots
+ * and lengths of avb_jpeg_encode_u8), contiguously into `out` as AVI '00dc' chunks: the fourcc, a little-endian u32
+ * size, the file, then zero bytes up to a multiple of 4 (the size counts them, as OpenCV's AVI writer does).  Record f
+ * starts at out + out_offsets_dev[f] (device int64); out_offsets_dev[n] is the bytes written.  `out` holds at least
+ * n * (8 + ((slot_stride + 3) & ~3)) bytes; a length outside [0, slot_stride] is clamped to it.  slots is 4-byte, out
+ * 16-byte aligned; n lies in [1, 65535]. */
+AVB_API int avb_mjpeg_pack_u8(const uint8_t *slots, int64_t slot_stride, const int64_t *lengths_dev, int n, uint8_t *out,
+                              int64_t *out_offsets_dev, avb_stream_t stream);
 
 /* ---- K10: PNG encode (csrc/k10_png.cu) -----------------------------------------------------------------
  * The bytes of cv2.imencode(".png", frame) with OpenCV's defaults (libpng 1.6 + zlib: filter Sub, deflate level 1,
