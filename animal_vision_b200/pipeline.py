@@ -7,9 +7,8 @@ from / to pinned host memory.  No collective, no host synchronisation inside the
 """
 from __future__ import annotations
 
+from contextlib import contextmanager
 from typing import List, Optional, Protocol, Sequence, Tuple
-
-import numpy as np
 
 from ._abi import check
 from .engine import get_engine
@@ -58,49 +57,69 @@ class HostBatchPipeline:
         t = self.eng.torch
         return [t.empty(tuple(frames.shape), dtype=t.uint8).pin_memory() for _ in range(n_out)]
 
+    @contextmanager
+    def _draining(self):
+        """Runs the enclosed code on the pipeline's device, then waits for all four streams, also when that code raises,
+        so no copy from or into the caller's host memory outlives the call."""
+        with self.eng.torch.cuda.device(self.eng.device):
+            try:
+                yield
+            finally:
+                for s in (self.s_rec, self.s_out, self.s_run, self.s_in):
+                    s.synchronize()
+
+    def _chunks(self, jobs):
+        """The chunk loop of every entry point.  jobs: (job, n_buf) with job[1] its frames_host [N,H,W,3].  Per chunk
+        of `chunk` frames, in job and frame order: takes the next of the `depth` slots of (chunk shape, n_buf) buffers
+        (slot numbers start at 0 on each call and run on across jobs); if the slot was used before, makes s_in and s_run
+        wait for its release event; uploads frames_host[a:b] on s_in and makes s_run wait for that upload (e_in).  Then
+        yields (job, a, b, the device input, the n_buf device buffers, the slot's event cell, the slot number), each
+        buffer cut to b - a frames.  The caller enqueues the chunk's work after e_in and sets the cell [0] to the event
+        that frees the slot.  A chunk is prepared only when the caller asks for it, so it sees a release event set after
+        the previous yield (run_split_jpeg sets it only when it retires a chunk)."""
+        t = self.eng.torch
+        slot_i = 0
+        for job, n_buf in jobs:
+            src = job[1]
+            n = src.shape[0]
+            for a in range(0, n, self.chunk):
+                b = min(n, a + self.chunk)
+                k = slot_i % self.depth
+                d_in, d_outs, ev = self._slot_bufs((self.chunk,) + tuple(src.shape[1:]), n_buf)[k]
+                slot_i += 1
+                if ev[0] is not None:                    # slot reused: its last copy out must be done
+                    self.s_in.wait_event(ev[0])
+                    self.s_run.wait_event(ev[0])
+                with t.cuda.stream(self.s_in):
+                    d_in[: b - a].copy_(src[a:b], non_blocking=True)
+                    e_in = self.s_in.record_event()
+                self.s_run.wait_event(e_in)
+                yield job, a, b, d_in[: b - a], [d[: b - a] for d in d_outs], ev, k
+
+    def _visualize(self, species, d_in, bufs):
+        """visualize_batch of d_in into slot buffers: (bufs[0], bufs[1]) for a two-output species (n_outputs), else its
+        view into bufs[-1]."""
+        species.visualize_batch(d_in, out=(bufs[0], bufs[1]) if self.n_outputs(species) == 2 else bufs[-1])
+
     def run(self, jobs: Sequence[Tuple[object, object, List[object]]]):
         """jobs: (species, frames_host, outs_host) with frames_host / outs_host pinned uint8
         tensors [N,H,W,3] (outs_host: one tensor per species output, see n_outputs).
-        Enqueues everything, then waits once.  Returns (h2d_bytes, d2h_bytes)."""
+        Enqueues everything, then waits once, also when a job fails mid-way, so no copy from or into the caller's
+        tensors is left in flight.  Returns (h2d_bytes, d2h_bytes)."""
         t = self.eng.torch
         h2d = d2h = 0
-        slot_i = 0
-        with t.cuda.device(self.eng.device):
-            for species, src, outs in jobs:
-                n = src.shape[0]
-                n_out = len(outs)
-                for a in range(0, n, self.chunk):
-                    b = min(n, a + self.chunk)
-                    shape = (self.chunk,) + tuple(src.shape[1:])
-                    slots = self._slot_bufs(shape, n_out)
-                    d_in, d_outs, ev = slots[slot_i % self.depth]
-                    slot_i += 1
-                    if ev[0] is not None:                    # slot reused: its last D2H must be done
-                        self.s_in.wait_event(ev[0])
-                        self.s_run.wait_event(ev[0])
-                    with t.cuda.stream(self.s_in):
-                        d_in[: b - a].copy_(src[a:b], non_blocking=True)
-                        e_in = t.cuda.Event()
-                        e_in.record(self.s_in)
-                    with t.cuda.stream(self.s_run):
-                        self.s_run.wait_event(e_in)
-                        if n_out == 2:
-                            species.visualize_batch(d_in[: b - a], out=(d_outs[0][: b - a], d_outs[1][: b - a]))
-                        else:
-                            species.visualize_batch(d_in[: b - a], out=d_outs[0][: b - a])
-                        e_run = t.cuda.Event()
-                        e_run.record(self.s_run)
-                    with t.cuda.stream(self.s_out):
-                        self.s_out.wait_event(e_run)
-                        for d, o in zip(d_outs, outs):
-                            o[a:b].copy_(d[: b - a], non_blocking=True)
-                        e_out = t.cuda.Event()
-                        e_out.record(self.s_out)
-                    ev[0] = e_out
-                    h2d += (b - a) * int(np.prod(src.shape[1:]))
-                    d2h += n_out * (b - a) * int(np.prod(src.shape[1:]))
-            self.s_out.synchronize()
-            self.s_run.synchronize()
+        with self._draining():
+            for (species, _, outs), a, b, d_in, bufs, ev, _ in self._chunks((job, len(job[2])) for job in jobs):
+                with t.cuda.stream(self.s_run):
+                    self._visualize(species, d_in, bufs)
+                    e_run = self.s_run.record_event()
+                with t.cuda.stream(self.s_out):
+                    self.s_out.wait_event(e_run)
+                    for d, o in zip(bufs, outs):
+                        o[a:b].copy_(d, non_blocking=True)
+                    ev[0] = self.s_out.record_event()
+                h2d += d_in.numel()
+                d2h += len(outs) * d_in.numel()
         return h2d, d2h
 
     def _split_plan(self, jobs, labels, what: str):
@@ -135,49 +154,22 @@ class HostBatchPipeline:
         t = self.eng.torch
         plan = self._split_plan(jobs, labels, "run_split")
         h2d = d2h = 0
-        slot_i = 0
-        with t.cuda.device(self.eng.device):
-            try:
-                for species, src, stencil in plan:
-                    n = src.shape[0]
-                    band = 0 if stencil is None else stencil[0]
-                    for a in range(0, n, self.chunk):
-                        b = min(n, a + self.chunk)
-                        # two buffers per slot for every species: [0] the split frame (and, first, the scratch
-                        # baseline of a two-output species, which the compose overwrites), [1] the view
-                        slots = self._slot_bufs((self.chunk,) + tuple(src.shape[1:]), 2)
-                        d_in, (d_split, d_view), ev = slots[slot_i % self.depth]
-                        slot_i += 1
-                        if ev[0] is not None:                    # slot reused: its last D2H must be done
-                            self.s_in.wait_event(ev[0])
-                            self.s_run.wait_event(ev[0])
-                        with t.cuda.stream(self.s_in):
-                            d_in[: b - a].copy_(src[a:b], non_blocking=True)
-                            e_in = t.cuda.Event()
-                            e_in.record(self.s_in)
-                        with t.cuda.stream(self.s_run):
-                            self.s_run.wait_event(e_in)
-                            if self.n_outputs(species) == 2:
-                                species.visualize_batch(d_in[: b - a], out=(d_split[: b - a], d_view[: b - a]))
-                            else:
-                                species.visualize_batch(d_in[: b - a], out=d_view[: b - a])
-                            self.eng.split_compose(d_in[: b - a], d_view[: b - a], d_split[: b - a], bool(draw_seam),
-                                                   stencil)
-                            e_run = t.cuda.Event()
-                            e_run.record(self.s_run)
-                        # The fetch writes src[a:b], the frames the H2D above reads: it waits for e_run, recorded
-                        # after the compose on s_run, which waited for e_in, recorded after that H2D.  No other
-                        # chunk reads these frames (jobs do not overlap, checked above).
-                        with t.cuda.stream(self.s_out):
-                            self.s_out.wait_event(e_run)
-                            d2h += self.eng.split_fetch(d_split[: b - a], src[a:b], band)
-                            e_out = t.cuda.Event()
-                            e_out.record(self.s_out)
-                        ev[0] = e_out
-                        h2d += (b - a) * int(np.prod(src.shape[1:]))
-            finally:
-                for s in (self.s_out, self.s_run, self.s_in):
-                    s.synchronize()
+        with self._draining():
+            # two buffers per slot for every species: [0] the split frame (and, first, the scratch baseline of a
+            # two-output species, which the compose overwrites), [1] the view
+            for (species, src, stencil), a, b, d_in, (d_split, d_view), ev, _ in self._chunks((j, 2) for j in plan):
+                with t.cuda.stream(self.s_run):
+                    self._visualize(species, d_in, (d_split, d_view))
+                    self.eng.split_compose(d_in, d_view, d_split, bool(draw_seam), stencil)
+                    e_run = self.s_run.record_event()
+                # The fetch writes src[a:b], the frames the chunk's H2D reads: it waits for e_run, recorded after the
+                # compose on s_run, which waited for e_in, recorded after that H2D (_chunks).  No other chunk reads
+                # these frames (jobs do not overlap, checked above).
+                with t.cuda.stream(self.s_out):
+                    self.s_out.wait_event(e_run)
+                    d2h += self.eng.split_fetch(d_split, src[a:b], 0 if stencil is None else stencil[0])
+                    ev[0] = self.s_out.record_event()
+                h2d += d_in.numel()
         return h2d, d2h
 
     def _jpeg_bufs(self, h: int, w: int, k8):
@@ -232,7 +224,6 @@ class HostBatchPipeline:
             if hw not in k8s:
                 k8s[hw] = JpegLauncher(eng.lib, *hw, quality, rgb=True)
         h2d = d2h = 0
-        slot_i = 0
         pending = []                      # enqueued chunks whose records are not yet copied, oldest first
         staged = []                       # at most one (copy event, staging, bytes, lengths) not yet handed to `out`
         retired = 0
@@ -263,57 +254,33 @@ class HostBatchPipeline:
                 hand_over()
             staged.append((e_out, staging, total, lengths))
 
-        with t.cuda.device(eng.device):
-            try:
-                for species, src, stencil in plan:
-                    n_all, h, w = src.shape[0], src.shape[1], src.shape[2]
-                    k8 = k8s[(h, w)]
-                    fs, rs = h * w * 3, w * 3
-                    for a in range(0, n_all, self.chunk):
-                        b = min(n_all, a + self.chunk)
-                        n = b - a
-                        slots = self._slot_bufs((self.chunk,) + tuple(src.shape[1:]), 2)
-                        d_in, (d_split, d_view), ev = slots[slot_i % self.depth]
-                        ws, jslots, packed, meta, meta_host = self._jpeg_bufs(h, w, k8)[slot_i % self.depth]
-                        slot_i += 1
-                        if ev[0] is not None:                    # slot reused: its last D2H must be done
-                            self.s_in.wait_event(ev[0])
-                            self.s_run.wait_event(ev[0])
-                        with t.cuda.stream(self.s_in):
-                            d_in[:n].copy_(src[a:b], non_blocking=True)
-                            e_in = t.cuda.Event()
-                            e_in.record(self.s_in)
-                        with t.cuda.stream(self.s_run):
-                            self.s_run.wait_event(e_in)
-                            if self.n_outputs(species) == 2:
-                                species.visualize_batch(d_in[:n], out=(d_split[:n], d_view[:n]))
-                            else:
-                                species.visualize_batch(d_in[:n], out=d_view[:n])
-                            eng.split_compose(d_in[:n], d_view[:n], d_split[:n], bool(draw_seam), stencil)
-                            # meta: [0, n] the record offsets (K11), [n + 1, 2n] the JPEG lengths (K8)
-                            st = eng.stream_ptr()
-                            check(k8.launch(d_split.data_ptr(), n, fs, rs, ws.data_ptr(), jslots.data_ptr(), k8.slot,
-                                            meta[n + 1:].data_ptr(), st), k8.name)
-                            check(eng.lib.avb_mjpeg_pack_u8(jslots.data_ptr(), k8.slot, meta[n + 1:].data_ptr(), n,
-                                                            packed.data_ptr(), meta.data_ptr(), st), "avb_mjpeg_pack_u8")
-                            eng.launches += JPEG_LAUNCHES + 1
-                            e_run = t.cuda.Event()
-                            e_run.record(self.s_run)
-                        with t.cuda.stream(self.s_out):
-                            self.s_out.wait_event(e_run)
-                            meta_host[:2 * n + 1].copy_(meta[:2 * n + 1], non_blocking=True)
-                            e_meta = t.cuda.Event()
-                            e_meta.record(self.s_out)
-                        pending.append((e_meta, meta_host, packed, n, ev))
-                        h2d += n * fs
-                        d2h += (2 * n + 1) * 8
-                        if len(pending) == self.depth:
-                            retire()
-                while pending:
+        with self._draining():
+            for (species, src, stencil), a, b, d_in, (d_split, d_view), ev, k in self._chunks((j, 2) for j in plan):
+                n, h, w = b - a, src.shape[1], src.shape[2]
+                k8 = k8s[(h, w)]
+                ws, jslots, packed, meta, meta_host = self._jpeg_bufs(h, w, k8)[k]
+                with t.cuda.stream(self.s_run):
+                    self._visualize(species, d_in, (d_split, d_view))
+                    eng.split_compose(d_in, d_view, d_split, bool(draw_seam), stencil)
+                    # meta: [0, n] the record offsets (K11), [n + 1, 2n] the JPEG lengths (K8)
+                    st = eng.stream_ptr()
+                    check(k8.launch(d_split.data_ptr(), n, h * w * 3, w * 3, ws.data_ptr(), jslots.data_ptr(), k8.slot,
+                                    meta[n + 1:].data_ptr(), st), k8.name)
+                    check(eng.lib.avb_mjpeg_pack_u8(jslots.data_ptr(), k8.slot, meta[n + 1:].data_ptr(), n,
+                                                    packed.data_ptr(), meta.data_ptr(), st), "avb_mjpeg_pack_u8")
+                    eng.launches += JPEG_LAUNCHES + 1
+                    e_run = self.s_run.record_event()
+                with t.cuda.stream(self.s_out):
+                    self.s_out.wait_event(e_run)
+                    meta_host[:2 * n + 1].copy_(meta[:2 * n + 1], non_blocking=True)
+                    e_meta = self.s_out.record_event()
+                pending.append((e_meta, meta_host, packed, n, ev))
+                h2d += d_in.numel()
+                d2h += (2 * n + 1) * 8
+                if len(pending) == self.depth:
                     retire()
-                if staged:
-                    hand_over()
-            finally:
-                for s in (self.s_rec, self.s_out, self.s_run, self.s_in):
-                    s.synchronize()
+            while pending:
+                retire()
+            if staged:
+                hand_over()
         return h2d, d2h

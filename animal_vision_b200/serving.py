@@ -73,13 +73,19 @@ def _device_runner(device=None) -> _DeviceRunner:
     return _DeviceRunner(device)
 
 
+def _rows(batch, idx: List[int]):
+    """The frames `idx` of a device batch: the batch itself when that is all of them, else one gather."""
+    import torch
+    return batch if len(idx) == batch.shape[0] else batch[torch.tensor(idx, device=batch.device)]
+
+
 def _pixels(view, idx: List[int]) -> List[np.ndarray]:
     """The frames `idx` of a batch result as host arrays (one D2H copy for a device result)."""
     if isinstance(view, np.ndarray):
         return [np.array(view[i], copy=True) for i in idx]
     import torch
     with torch.cuda.device(view.device):
-        sel = view if len(idx) == view.shape[0] else view[torch.tensor(idx, device=view.device)]
+        sel = _rows(view, idx)
         pin = torch.empty(tuple(sel.shape), dtype=torch.uint8).pin_memory()
         pin.copy_(sel, non_blocking=True)
         torch.cuda.current_stream(view.device).synchronize()
@@ -106,7 +112,7 @@ def _encoded(view, idx: List[int], fmt: str) -> List[bytes]:
     from .jpeg import encode_jpeg
     from .png import encode_png
     with torch.cuda.device(view.device):
-        sel = view if len(idx) == view.shape[0] else view[torch.tensor(idx, device=view.device)]
+        sel = _rows(view, idx)
         return encode_jpeg(sel, 95) if fmt == "jpeg" else encode_png(sel)
 
 
@@ -129,11 +135,7 @@ def _split_jpegs(frames: np.ndarray, dev_in, view, idx: List[int], labels: Tuple
     with torch.cuda.device(view.device):
         if dev_in is None:
             dev_in = torch.from_numpy(frames).pin_memory().to(view.device, non_blocking=True)
-        if len(idx) == view.shape[0]:
-            orig, sel = dev_in, view
-        else:
-            ix = torch.tensor(idx, device=view.device)
-            orig, sel = dev_in[ix], view[ix]
+        orig, sel = _rows(dev_in, idx), _rows(view, idx)
         return encode_jpeg(split_compare_batch(orig, sel, draw_seam=seam, labels=labels), 95)
 
 
@@ -288,26 +290,26 @@ def default_batcher() -> FrameBatcher:
         return _default
 
 
-def process_image(imagedata: bytes, animal: str, batcher: Optional[FrameBatcher] = None) -> str:
-    """Drop-in for utils.py:133-199 `processimage`: JPEG bytes in, JPEG data URI out; decoded BGR as cv2.imread gives it
-    (the species index channels 0/1/2, never "R/G/B" -- the reference feeds BGR here too, utils.py:141-142)."""
+def _data_uri(imagedata: bytes, submit: Callable[[np.ndarray], Future], mime: str) -> str:
+    """Decodes `imagedata` BGR as cv2.imread gives it, submits the frame and returns the encoded result as a base64
+    data URI of type `mime`."""
     import cv2
     img = cv2.imdecode(np.frombuffer(imagedata, np.uint8), cv2.IMREAD_COLOR)
     if img is None:
         raise ValueError("could not decode the image")
-    enc = (batcher or default_batcher()).submit_jpeg(img, animal).result()
-    return "data:image/jpeg;base64," + base64.b64encode(enc).decode("utf-8")
+    return f"data:{mime};base64," + base64.b64encode(submit(img).result()).decode("utf-8")
+
+
+def process_image(imagedata: bytes, animal: str, batcher: Optional[FrameBatcher] = None) -> str:
+    """Drop-in for utils.py:133-199 `processimage`: JPEG bytes in, JPEG data URI out; decoded BGR as cv2.imread gives it
+    (the species index channels 0/1/2, never "R/G/B" -- the reference feeds BGR here too, utils.py:141-142)."""
+    return _data_uri(imagedata, lambda img: (batcher or default_batcher()).submit_jpeg(img, animal), "image/jpeg")
 
 
 def process_image_png(imagedata: bytes, animal: str, batcher: Optional[FrameBatcher] = None) -> str:
     """`process_image` with a lossless result: image bytes in, data URI of the PNG of the species view out
     (`FrameBatcher.submit_png`, the bytes of cv2.imencode(".png", view))."""
-    import cv2
-    img = cv2.imdecode(np.frombuffer(imagedata, np.uint8), cv2.IMREAD_COLOR)
-    if img is None:
-        raise ValueError("could not decode the image")
-    enc = (batcher or default_batcher()).submit_png(img, animal).result()
-    return "data:image/png;base64," + base64.b64encode(enc).decode("utf-8")
+    return _data_uri(imagedata, lambda img: (batcher or default_batcher()).submit_png(img, animal), "image/png")
 
 
 def process_split_image(imagedata: bytes, animal: str, labels: Tuple[str, str] = ("Original", "Transformed"),
@@ -315,9 +317,5 @@ def process_split_image(imagedata: bytes, animal: str, labels: Tuple[str, str] =
     """JPEG bytes in, data URI of the JPEG of the labelled split-compare frame out (input on the left, species view on
     the right, seam, corner labels; `FrameBatcher.submit_split_jpeg`).  Decoded BGR as cv2.imread gives it, like
     `process_image`."""
-    import cv2
-    img = cv2.imdecode(np.frombuffer(imagedata, np.uint8), cv2.IMREAD_COLOR)
-    if img is None:
-        raise ValueError("could not decode the image")
-    enc = (batcher or default_batcher()).submit_split_jpeg(img, animal, labels).result()
-    return "data:image/jpeg;base64," + base64.b64encode(enc).decode("utf-8")
+    return _data_uri(imagedata, lambda img: (batcher or default_batcher()).submit_split_jpeg(img, animal, labels),
+                     "image/jpeg")

@@ -236,3 +236,16 @@ def test_a_failing_job_leaves_no_copy_in_flight():
         pipe.run_split([(Invert(), f), (Refuses(), g)])
     assert np.array_equal(f.numpy(), host_route(a, 255 - a, DEFAULT))
     assert np.array_equal(g.numpy(), c)
+
+
+def test_run_leaves_no_copy_in_flight_when_a_job_fails():
+    """run waits for what it enqueued before it raises: the earlier job's views are already in its outputs (1080p
+    frames, so a copy still in flight would be seen), and the pipeline stays usable."""
+    pipe = HostBatchPipeline(chunk_frames=2)
+    a, c = batch(5, 1080, 1920), batch(2, 1080, 1920, seed=30)
+    f, g = pinned(a), pinned(c)
+    outs_f, outs_g = pipe.pinned_like(f, 1), pipe.pinned_like(g, 1)
+    with pytest.raises(RuntimeError, match="refused"):
+        pipe.run([(Invert(), f, outs_f), (Refuses(), g, outs_g)])
+    assert np.array_equal(outs_f[0].numpy(), 255 - a)
+    assert np.array_equal(views_of(pipe, Invert(), c), 255 - c)
