@@ -69,6 +69,9 @@ SIGNATURES = {
     "avb_jpeg_workspace_bytes": (_i64, [_i, _i, _i]),
     "avb_jpeg_encode_u8": (_i, [_p, _i, _i, _i, _i64, _i64, _p, _i, _p, _p, _i64, _p, _p, _p]),
     "avb_jpeg_encode_rgb_u8": (_i, [_p, _i, _i, _i, _i64, _i64, _p, _i, _p, _p, _i64, _p, _p, _p]),
+    "avb_jpeg_opt_workspace_bytes": (_i64, [_i, _i, _i]),
+    "avb_jpeg_opt_encode_u8": (_i, [_p, _i, _i, _i, _i64, _i64, _p, _i, _p, _i, _p, _p, _i64, _p, _p, _p]),
+    "avb_jpeg_opt_encode_rgb_u8": (_i, [_p, _i, _i, _i, _i64, _i64, _p, _i, _p, _i, _p, _p, _i64, _p, _p, _p]),
     "avb_mjpeg_pack_u8": (_i, [_p, _i64, _p, _i, _p, _p, _p]),
     "avb_png_bound_bytes": (_i64, [_i, _i]),
     "avb_png_workspace_bytes": (_i64, [_i, _i, _i]),

@@ -12,6 +12,16 @@
 //   jpeg_ff_count   0xFF bytes per 16-byte chunk
 //   jpeg_ff_scan    one CTA per frame: chunk offsets of the stuffed stream, header + EOI, total length
 //   jpeg_stuff      scatter of the bytes with 0x00 after every 0xFF (jchuff.c emit_byte)
+// The optimized mode (avb_jpeg_opt_encode_u8, cv2.IMWRITE_JPEG_OPTIMIZE) codes each frame with Huffman tables built from
+// its own symbol counts.  The template flag OPT of the shared kernels selects it; the standard instances are unchanged.
+//   jpeg_transform  counts the AC symbols of its blocks in shared memory, adds them to the frame's 64-bit counters;
+//                   writes no code lengths (the tables are not known yet)
+//   jpeg_dc_hist    one thread per MCU: DC symbol counts (they need the previous MCU's DCs)
+//   jpeg_tables     one CTA per frame, one warp per table: jchuff.c jpeg_gen_optimal_table, jpeg_make_c_derived_tbl and
+//                   the DHT segment
+//   jpeg_blen       one thread per block: its code length from the frame's tables
+// then jpeg_mcu_scan and jpeg_emit read the frame's tables from shared memory, jpeg_ff_scan writes the header prefix,
+// the frame's four DHT segments and the SOS segment, and jpeg_stuff starts the data after that frame's header.
 #include <string.h>
 
 #include "avb_common.cuh"
@@ -76,6 +86,21 @@ constexpr HuffTabs make_huff() {
 
 __constant__ HuffTabs c_huff = make_huff();
 
+// The codes a kernel reads: the standard tables in constant memory, or (OPT) the frame's own in shared memory
+template <bool OPT>
+struct Codes {
+    const uint32_t (*dct)[16];
+    const uint32_t (*act)[256];
+    __device__ __forceinline__ uint32_t dc(int tab, int s) const {
+        if constexpr (OPT) return dct[tab][s];
+        else return c_huff.dc[tab][s];
+    }
+    __device__ __forceinline__ uint32_t ac(int tab, int sym) const {
+        if constexpr (OPT) return act[tab][sym];
+        else return c_huff.ac[tab][sym];
+    }
+};
+
 // natural index -> zigzag position
 __constant__ uint8_t c_izz[64] = {0,  1,  5,  6,  14, 15, 27, 28, 2,  4,  7,  13, 16, 26, 29, 42, 3,  8,  12, 17, 25, 30,
                                   41, 43, 9,  11, 18, 24, 31, 40, 44, 53, 10, 19, 23, 32, 39, 45, 52, 54, 20, 22, 33, 38,
@@ -88,6 +113,13 @@ struct QDiv {
 struct Header {
     uint8_t b[AVB_JPEG_HEADER_MAX];
 };
+
+// A DHT segment: marker, length, class / id, bits[1..16], up to 256 values
+constexpr int DHT_SEG_MAX = 4 + 1 + 16 + 256;
+constexpr int DHT_BYTES = (4 * DHT_SEG_MAX + 15) & ~15;     // the four segments of a frame
+// What the four segments take at most: an 8-bit baseline DC table holds the sizes 0..11, an AC table the 160 (run, size)
+// symbols with sizes 1..10, ZRL and EOB -- the symbol sets of the standard tables (jchuff.c MAX_COEF_BITS)
+constexpr int DHT_LEN_MAX = 2 * (4 + 1 + 16 + 12) + 2 * (4 + 1 + 16 + 162);
 
 struct Geo {
     int H, W, mw, mh, bw, bh;
@@ -121,6 +153,16 @@ struct Work {
     uint64_t *bits;             // [n] total entropy bits
 };
 
+// the optimized mode's part of the workspace, after carve's
+struct Opt {
+    uint64_t *freq;             // [n][4][256] symbol counts: DC0, AC0, DC1, AC1
+    HuffTabs *tabs;             // [n] the frame's codes
+    uint8_t *dht;               // [n][DHT_BYTES] the frame's DHT segments, back to back
+    int *dhtlen;                // [n] their bytes
+    int *hlen;                  // [n] header bytes (prefix + DHT segments + SOS)
+    int slen;                   // SOS bytes; the header prefix's are the kernels' hlen argument
+};
+
 int64_t carve(const Geo &g, int n, uint8_t *base, Work *w) {
     int64_t o = 0;
     auto take = [&](int64_t bytes) {
@@ -141,14 +183,32 @@ int64_t carve(const Geo &g, int n, uint8_t *base, Work *w) {
     return o;
 }
 
+int64_t carve_opt(const Geo &g, int n, uint8_t *base, Opt *op) {
+    int64_t o = carve(g, n, nullptr, nullptr);
+    auto take = [&](int64_t bytes) {
+        uint8_t *p = base ? base + o : nullptr;
+        o += (bytes + 15) & ~(int64_t)15;
+        return p;
+    };
+    Opt t{};
+    t.freq = (uint64_t *)take((int64_t)n * 4 * 256 * 8);
+    t.tabs = (HuffTabs *)take((int64_t)n * sizeof(HuffTabs));
+    t.dht = take((int64_t)n * DHT_BYTES);
+    t.dhtlen = (int *)take((int64_t)n * 4);
+    t.hlen = (int *)take((int64_t)n * 4);
+    if (op) *op = t;
+    return o;
+}
+
 __device__ __forceinline__ int nbits_of(int v) {
     v = abs(v);
     return v ? 32 - __clz(v) : 0;
 }
 
-__device__ __forceinline__ int dc_len(int tab, int diff) {
+template <bool OPT>
+__device__ __forceinline__ int dc_len(const Codes<OPT> &c, int tab, int diff) {
     const int s = nbits_of(diff);
-    return (int)(c_huff.dc[tab][s] >> 16) + s;
+    return (int)(c.dc(tab, s) >> 16) + s;
 }
 
 __device__ __forceinline__ int descale(int x, int n) { return (x + (1 << (n - 1))) >> n; }
@@ -180,15 +240,22 @@ __device__ __forceinline__ void fdct8(const int *d, int *o) {
 }
 
 // RGB: the frames hold R, G, B (avb_jpeg_encode_rgb_u8); everything after the gather is shared
-template <bool RGB>
+// OPT: AC symbol counts instead of code lengths
+template <bool RGB, bool OPT>
 __global__ void __launch_bounds__(TF_THREADS) jpeg_transform_kernel(const uint8_t *__restrict__ in, int64_t fs, int64_t rs,
-                                                                     Geo g, QDiv qd, Work w) {
+                                                                     Geo g, QDiv qd, Work w, Opt op) {
     __shared__ uint8_t sY[16][128], sCb[16][128], sCr[16][128], sC[2][8][64];
     __shared__ int work[STRIP * 6][8][9];
     __shared__ __align__(16) int16_t qz[STRIP * 6][64];
     __shared__ uint16_t sdiv[2][64];
     __shared__ uint8_t sizz[64];
     const int tid = threadIdx.x, f = blockIdx.z, my = blockIdx.y, mx0 = blockIdx.x * STRIP;
+    uint32_t *hist = nullptr;                                   // [2][256] AC counts of the CTA: luma, chroma
+    if constexpr (OPT) {
+        __shared__ uint32_t shist[2 * 256];
+        hist = shist;
+        for (int i = tid; i < 2 * 256; i += TF_THREADS) hist[i] = 0;
+    }
     if (tid < 128) sdiv[tid >> 6][tid & 63] = qd.d[tid >> 6][tid & 63];
     if (tid < 64) sizz[tid] = c_izz[tid];
     const uint8_t *fin = in + (int64_t)f * fs;
@@ -267,6 +334,31 @@ __global__ void __launch_bounds__(TF_THREADS) jpeg_transform_kernel(const uint8_
     mask |= __shfl_xor_sync(0xffffffffu, mask, 4);
     mask &= ~1ull;
     const int tab = b >= 4;
+    if constexpr (OPT) {              // jchuff.c htest_one_block; blocks of MCUs past the right edge are not coded
+        if (j < na) {
+#pragma unroll
+            for (int k = 0; k < 8; ++k) {
+                const int zz = lane * 8 + k;
+                if ((mask >> zz) & 1) {
+                    const uint64_t below = mask & ((1ull << zz) - 1);
+                    const int prev = below ? 63 - __clzll((long long)below) : 0;
+                    const int run = zz - prev - 1;
+                    if (run >= 16) atomicAdd(&hist[tab * 256 + 0xF0], (uint32_t)(run >> 4));
+                    atomicAdd(&hist[tab * 256 + (((run & 15) << 4) | nbits_of(qz[bl][zz]))], 1u);
+                }
+            }
+            if (lane == 0) {
+                if (!(mask >> 63)) atomicAdd(&hist[tab * 256], 1u);
+                w.dcs[(mcu0 + j) * 8 + b] = qz[bl][0];
+            }
+        }
+        __syncthreads();
+        for (int i = tid; i < 2 * 256; i += TF_THREADS)
+            if (hist[i])
+                atomicAdd((unsigned long long *)&op.freq[((int64_t)f * 4 + 2 * (i >> 8) + 1) * 256 + (i & 255)],
+                          (unsigned long long)hist[i]);
+        return;
+    }
     const int zrl = (int)(c_huff.ac[tab][0xF0] >> 16);
     int len = 0;
 #pragma unroll
@@ -281,7 +373,7 @@ __global__ void __launch_bounds__(TF_THREADS) jpeg_transform_kernel(const uint8_
     }
     if (lane == 0) {
         if (!(mask >> 63)) len += (int)(c_huff.ac[tab][0] >> 16);
-        if (b >= 1 && b <= 3) len += dc_len(0, qz[bl][0] - qz[bl - 1][0]);
+        if (b >= 1 && b <= 3) len += dc_len(Codes<false>{}, 0, qz[bl][0] - qz[bl - 1][0]);
     }
     len += __shfl_xor_sync(0xffffffffu, len, 1);
     len += __shfl_xor_sync(0xffffffffu, len, 2);
@@ -354,8 +446,9 @@ __device__ __forceinline__ Dc8 load_dc(const int16_t *p) {
 }
 
 // the DC codes that need the previous MCU: block 0 after the previous Y11, Cb and Cr after theirs
-__device__ __forceinline__ int cross_dc_len(const Dc8 &d, const Dc8 &p) {
-    return dc_len(0, d.v[0] - p.v[3]) + dc_len(1, d.v[4] - p.v[4]) + dc_len(1, d.v[5] - p.v[5]);
+template <bool OPT>
+__device__ __forceinline__ int cross_dc_len(const Codes<OPT> &c, const Dc8 &d, const Dc8 &p) {
+    return dc_len(c, 0, d.v[0] - p.v[3]) + dc_len(c, 1, d.v[4] - p.v[4]) + dc_len(c, 1, d.v[5] - p.v[5]);
 }
 
 __device__ __forceinline__ Dc8 prev_dc(const int16_t *dcs, int64_t fm, int64_t m) {
@@ -366,9 +459,227 @@ __device__ __forceinline__ Dc8 prev_dc(const int16_t *dcs, int64_t fm, int64_t m
     return z;
 }
 
-__global__ void __launch_bounds__(SCAN_THREADS) jpeg_mcu_scan_kernel(Geo g, Work w) {
+// The frame's codes into shared memory (OPT); every thread of the CTA takes part
+__device__ __forceinline__ void load_tabs(HuffTabs *s, const HuffTabs *t) {
+    static_assert(sizeof(HuffTabs) % 16 == 0, "HuffTabs is copied in 16-byte pieces");
+    for (int i = threadIdx.x; i < (int)(sizeof(HuffTabs) / 16); i += blockDim.x)
+        reinterpret_cast<uint4 *>(s)[i] = reinterpret_cast<const uint4 *>(t)[i];
+    __syncthreads();
+}
+
+// DC symbol counts of every block (OPT)
+__global__ void __launch_bounds__(256) jpeg_dc_hist_kernel(Geo g, Work w, Opt op) {
+    __shared__ uint32_t hist[2][16];                // luma, chroma; a DC size is at most 12
+    const int f = blockIdx.y;
+    const int64_t m = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (threadIdx.x < 32) hist[threadIdx.x >> 4][threadIdx.x & 15] = 0;
+    __syncthreads();
+    if (m < g.M) {
+        const int64_t fm = (int64_t)f * g.M + m;
+        const Dc8 d = load_dc(w.dcs + fm * 8), p = prev_dc(w.dcs, fm, m);
+#pragma unroll
+        for (int k = 0; k < 6; ++k) {               // predictors as jpeg_emit's
+            const int pk = k == 0 ? p.v[3] : (k < 4 ? d.v[k - 1] : p.v[k]);
+            atomicAdd(&hist[k >= 4][nbits_of(d.v[k] - pk)], 1u);
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x < 32) {
+        const uint32_t v = hist[threadIdx.x >> 4][threadIdx.x & 15];
+        if (v)
+            atomicAdd((unsigned long long *)&op.freq[((int64_t)f * 4 + 2 * (threadIdx.x >> 4)) * 256 + (threadIdx.x & 15)],
+                      (unsigned long long)v);
+    }
+}
+
+// One CTA per frame, one warp per table t (DC0, AC0, DC1, AC1).  jchuff.c jpeg_gen_optimal_table: symbol 256 with count 1
+// reserves the all-ones code; each step merges the two least frequent trees c1, c2 (the smallest count, ties to the
+// largest symbol, counts above libjpeg's initial v = 10^9 never taken) and lengthens the codes of both.  The symbols with
+// a nonzero count are exactly the roots of the trees, so a tree is kept as a label (its root) on each symbol.  Then the
+// lengths above 16 are folded down, the values are ordered by (unlimited) code length, then symbol, and take canonical
+// codes (jpeg_make_c_derived_tbl); the warp writes the frame's codes and its DHT segment.
+__global__ void __launch_bounds__(128) jpeg_tables_kernel(Opt op) {
+    constexpr int K = 9;                            // symbols per lane: lane + 32 k covers 0..256
+    constexpr uint64_t V0 = 1000000000ull, NONE = ~0ull;
+    __shared__ int sbits[4][33], sstart[4][33], sfirst[4][17], scode[4][17], snsym[4];
+    __shared__ uint8_t sval[4][256];
+    const int f = blockIdx.x, t = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint64_t *fr = op.freq + ((int64_t)f * 4 + t) * 256;
+    uint64_t fq[K];
+    int cs[K], lab[K];
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+        const int i = lane + 32 * k;
+        fq[k] = i < 256 ? fr[i] : (uint64_t)(i == 256);
+        cs[k] = 0;
+        lab[k] = i;
+    }
+    for (int i = lane; i < 33; i += 32) sbits[t][i] = sstart[t][i] = 0;
+    // the least key (count << 9) | (256 - symbol) among the candidates: the smallest count, ties to the largest symbol
+    auto least = [&](int skip) {
+        uint64_t m = NONE;
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            const int i = lane + 32 * k;
+            if (fq[k] && fq[k] <= V0 && i != skip) m = min(m, (fq[k] << 9) | (uint64_t)(256 - i));
+        }
+#pragma unroll
+        for (int o = 16; o; o >>= 1) m = min(m, __shfl_xor_sync(0xffffffffu, m, o));
+        return m;
+    };
+    for (;;) {
+        const uint64_t k1 = least(-1);
+        const int c1 = 256 - (int)(k1 & 511);
+        const uint64_t k2 = k1 == NONE ? NONE : least(c1);
+        if (k2 == NONE) break;
+        const int c2 = 256 - (int)(k2 & 511);
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            const int i = lane + 32 * k;
+            if (lab[k] == c1 || lab[k] == c2) {
+                ++cs[k];
+                lab[k] = c1;
+            }
+            if (i == c1) fq[k] += k2 >> 9;
+            if (i == c2) fq[k] = 0;
+        }
+    }
+    __syncwarp();
+#pragma unroll
+    for (int k = 0; k < K; ++k) {                   // jpeg_gen_optimal_table allows code lengths up to 32
+        const int i = lane + 32 * k;
+        if (cs[k] && i <= 256) {
+            atomicAdd(&sbits[t][min(cs[k], 32)], 1);
+            if (i < 256) atomicAdd(&sstart[t][min(cs[k], 32)], 1);
+        }
+    }
+    __syncwarp();
+    if (lane == 0) {
+        int *bits = sbits[t];
+        for (int i = 32; i > 16; --i)
+            while (bits[i] > 0) {
+                int j = i - 2;
+                while (bits[j] == 0) --j;
+                bits[i] -= 2;
+                bits[i - 1] += 1;
+                bits[j + 1] += 2;
+                bits[j] -= 1;
+            }
+        int i = 16;
+        while (bits[i] == 0) --i;
+        bits[i] -= 1;                               // the reserved code
+        int s = 0;
+        for (int L = 1; L <= 32; ++L) {             // first value position of each unlimited length
+            const int c = sstart[t][L];
+            sstart[t][L] = s;
+            s += c;
+        }
+        int code = 0, p = 0;
+        for (int L = 1; L <= 16; ++L) {             // canonical codes: first position and first code of each length
+            sfirst[t][L] = p;
+            scode[t][L] = code;
+            p += bits[L];
+            code = (code + bits[L]) << 1;
+        }
+        snsym[t] = p;
+    }
+    __syncwarp();
+    int pos[K];
+#pragma unroll
+    for (int k = 0; k < K; ++k) {                   // value positions, symbols of one length in increasing order
+        const int i = lane + 32 * k;
+        const int L = i < 256 && cs[k] ? min(cs[k], 32) : 0;
+        const unsigned same = __match_any_sync(0xffffffffu, L);
+        pos[k] = L ? sstart[t][L] + __popc(same & ((1u << lane) - 1u)) : -1;
+        __syncwarp();
+        if (L && lane == __ffs(same) - 1) sstart[t][L] += __popc(same);
+        __syncwarp();
+    }
+    HuffTabs *tabs = op.tabs + f;
+    uint32_t *dst = t & 1 ? tabs->ac[t >> 1] : tabs->dc[t >> 1];
+    const int nent = t & 1 ? 256 : 16;
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+        const int i = lane + 32 * k, p = pos[k];
+        if (p >= 0) sval[t][p] = (uint8_t)i;
+        if (i < nent) {
+            uint32_t e = 0;
+            if (p >= 0)
+                for (int L = 1; L <= 16; ++L)
+                    if (p >= sfirst[t][L] && p < sfirst[t][L] + sbits[t][L])
+                        e = ((uint32_t)L << 16) | (uint32_t)(scode[t][L] + p - sfirst[t][L]);
+            dst[i] = e;
+        }
+    }
+    __syncthreads();
+    int off = 0;
+    for (int u = 0; u < t; ++u) off += 21 + snsym[u];
+    const int nsym = snsym[t];
+    uint8_t *seg = op.dht + (int64_t)f * DHT_BYTES + off;
+    for (int b = lane; b < 21 + nsym; b += 32) {
+        uint8_t v;
+        if (b < 4) v = b == 0 ? 0xFF : b == 1 ? 0xC4 : b == 2 ? (uint8_t)((19 + nsym) >> 8) : (uint8_t)(19 + nsym);
+        else if (b == 4) v = (uint8_t)(((t & 1) << 4) | (t >> 1));
+        else if (b < 21) v = (uint8_t)sbits[t][b - 4];
+        else v = sval[t][b - 21];
+        seg[b] = v;
+    }
+    if (threadIdx.x == 0) op.dhtlen[f] = 4 * 21 + snsym[0] + snsym[1] + snsym[2] + snsym[3];
+}
+
+// the zigzag nonzero mask of a block's AC coefficients
+__device__ __forceinline__ uint64_t ac_mask(const int16_t *cf) {
+    uint64_t mask = 0;
+#pragma unroll
+    for (int q = 0; q < 8; ++q) {
+        const int4 v = __ldg(reinterpret_cast<const int4 *>(cf) + q);
+        const int u[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            mask |= (uint64_t)((u[k] & 0xffff) != 0) << (q * 8 + 2 * k);
+            mask |= (uint64_t)((u[k] >> 16) != 0) << (q * 8 + 2 * k + 1);
+        }
+    }
+    return mask & ~1ull;
+}
+
+// Code length of every block from the frame's codes (OPT): what jpeg_transform writes in the standard mode
+__global__ void __launch_bounds__(256) jpeg_blen_kernel(Geo g, Work w, Opt op) {
+    __shared__ __align__(16) HuffTabs st;
+    const int f = blockIdx.y;
+    load_tabs(&st, op.tabs + f);
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= g.M * 6) return;
+    const int64_t m = t / 6, fm = (int64_t)f * g.M + m;
+    const int b = (int)(t - m * 6), tab = b >= 4;
+    const int16_t *cf = w.coef + fm * 384 + b * 64;
+    const Codes<true> c{st.dc, st.ac};
+    uint64_t mask = ac_mask(cf);
+    const int zrl = (int)(c.ac(tab, 0xF0) >> 16);
+    int len = 0, prev = 0;
+    while (mask) {
+        const int zz = __ffsll((long long)mask) - 1;
+        mask &= mask - 1;
+        const int run = zz - prev - 1, s = nbits_of(__ldg(cf + zz));
+        len += (run >> 4) * zrl + (int)(c.ac(tab, ((run & 15) << 4) | s) >> 16) + s;
+        prev = zz;
+    }
+    if (prev != 63) len += (int)(c.ac(tab, 0) >> 16);
+    if (b >= 1 && b <= 3) len += dc_len(c, 0, __ldg(cf) - __ldg(cf - 64));
+    w.blen[fm * 8 + b] = (uint16_t)len;
+}
+
+template <bool OPT>
+__global__ void __launch_bounds__(SCAN_THREADS) jpeg_mcu_scan_kernel(Geo g, Work w, Opt op) {
     const int f = blockIdx.x;
     const int64_t fm0 = (int64_t)f * g.M;
+    Codes<OPT> c{};
+    if constexpr (OPT) {
+        __shared__ uint32_t sdc[2][16];
+        if (threadIdx.x < 32) sdc[threadIdx.x >> 4][threadIdx.x & 15] = op.tabs[f].dc[threadIdx.x >> 4][threadIdx.x & 15];
+        __syncthreads();
+        c.dct = sdc;
+    }
     const uint64_t total = block_scan(
         g.M,
         [&](int64_t m) -> uint64_t {
@@ -377,7 +688,7 @@ __global__ void __launch_bounds__(SCAN_THREADS) jpeg_mcu_scan_kernel(Geo g, Work
             uint32_t s = 0;
 #pragma unroll
             for (int k = 0; k < 3; ++k) s += (u[k] & 0xffffu) + (u[k] >> 16);
-            return s + cross_dc_len(load_dc(w.dcs + (fm0 + m) * 8), prev_dc(w.dcs, fm0 + m, m));
+            return s + cross_dc_len(c, load_dc(w.dcs + (fm0 + m) * 8), prev_dc(w.dcs, fm0 + m, m));
         },
         [&](int64_t m, uint64_t e) { w.off[fm0 + m] = e; });
     if (threadIdx.x == 0) w.bits[f] = total;
@@ -423,7 +734,14 @@ __device__ __forceinline__ void put_value(BitWriter &bw, uint32_t hc, int v, int
     bw.put(((hc & 0xffffu) << s) | extra, (int)(hc >> 16) + s);
 }
 
-__global__ void __launch_bounds__(256) jpeg_emit_kernel(Geo g, Work w) {
+template <bool OPT>
+__global__ void __launch_bounds__(256) jpeg_emit_kernel(Geo g, Work w, Opt op) {
+    Codes<OPT> c{};
+    if constexpr (OPT) {
+        __shared__ __align__(16) HuffTabs st;
+        load_tabs(&st, op.tabs + blockIdx.y);
+        c = Codes<OPT>{st.dc, st.ac};
+    }
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= g.M * 6) return;
     const int f = blockIdx.y;
@@ -437,7 +755,7 @@ __global__ void __launch_bounds__(256) jpeg_emit_kernel(Geo g, Work w) {
         const int pk = k == 0 ? p.v[3] : (k < 4 ? d.v[k - 1] : p.v[k]);
         if (k < b) {
             pos += w.blen[fm * 8 + k];
-            if (k == 0 || k >= 4) pos += dc_len(k >= 4, d.v[k] - pk);
+            if (k == 0 || k >= 4) pos += dc_len(c, k >= 4, d.v[k] - pk);
         }
         if (k == b) {
             dcv = d.v[k];
@@ -445,33 +763,22 @@ __global__ void __launch_bounds__(256) jpeg_emit_kernel(Geo g, Work w) {
         }
     }
     const int16_t *cf = w.coef + fm * 384 + b * 64;
-    uint64_t mask = 0;
-#pragma unroll
-    for (int q = 0; q < 8; ++q) {
-        const int4 v = __ldg(reinterpret_cast<const int4 *>(cf) + q);
-        const int u[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            mask |= (uint64_t)((u[k] & 0xffff) != 0) << (q * 8 + 2 * k);
-            mask |= (uint64_t)((u[k] >> 16) != 0) << (q * 8 + 2 * k + 1);
-        }
-    }
-    mask &= ~1ull;
+    uint64_t mask = ac_mask(cf);
     const int tab = b >= 4;
     BitWriter bw(w.words + (int64_t)f * (g.wbytes / 4), pos);
     const int diff = dcv - pred;
-    put_value(bw, c_huff.dc[tab][nbits_of(diff)], diff, nbits_of(diff));
+    put_value(bw, c.dc(tab, nbits_of(diff)), diff, nbits_of(diff));
     int prev = 0;
     while (mask) {
         const int zz = __ffsll((long long)mask) - 1;
         mask &= mask - 1;
         int run = zz - prev - 1;
-        for (; run >= 16; run -= 16) bw.put(c_huff.ac[tab][0xF0] & 0xffffu, (int)(c_huff.ac[tab][0xF0] >> 16));
+        for (; run >= 16; run -= 16) bw.put(c.ac(tab, 0xF0) & 0xffffu, (int)(c.ac(tab, 0xF0) >> 16));
         const int v = __ldg(cf + zz), s = nbits_of(v);
-        put_value(bw, c_huff.ac[tab][(run << 4) | s], v, s);
+        put_value(bw, c.ac(tab, (run << 4) | s), v, s);
         prev = zz;
     }
-    if (prev != 63) bw.put(c_huff.ac[tab][0] & 0xffffu, (int)(c_huff.ac[tab][0] >> 16));
+    if (prev != 63) bw.put(c.ac(tab, 0) & 0xffffu, (int)(c.ac(tab, 0) >> 16));
     bw.flush();
 }
 
@@ -497,15 +804,26 @@ __global__ void jpeg_ff_count_kernel(Geo g, Work w, int n) {
     }
 }
 
+// OPT: hdr holds the header prefix (hlen bytes), then the SOS segment (op.slen bytes); the frame's DHT segments go between
+template <bool OPT>
 __global__ void __launch_bounds__(SCAN_THREADS) jpeg_ff_scan_kernel(Geo g, Work w, Header hdr, int hlen, uint8_t *out,
-                                                                   int64_t slot, int64_t *lengths) {
+                                                                   int64_t slot, int64_t *lengths, Opt op) {
     const int f = blockIdx.x;
     const int64_t nbytes = entropy_bytes(w.bits[f]), nch = (nbytes + CHUNK - 1) / CHUNK;
     uint32_t *cnt = w.ffcnt + (int64_t)f * g.chunks;
     const uint64_t ff = block_scan(
         nch, [&](int64_t c) -> uint64_t { return cnt[c]; }, [&](int64_t c, uint64_t e) { cnt[c] = (uint32_t)e; });
     uint8_t *dst = out + (int64_t)f * slot;
-    for (int i = threadIdx.x; i < hlen; i += blockDim.x) dst[i] = hdr.b[i];
+    if constexpr (OPT) {
+        const int dl = op.dhtlen[f], plen = hlen;
+        const uint8_t *dht = op.dht + (int64_t)f * DHT_BYTES;
+        hlen = plen + dl + op.slen;
+        for (int i = threadIdx.x; i < hlen; i += blockDim.x)
+            dst[i] = i < plen ? hdr.b[i] : i < plen + dl ? dht[i - plen] : hdr.b[i - dl];
+        if (threadIdx.x == 0) op.hlen[f] = hlen;
+    } else {
+        for (int i = threadIdx.x; i < hlen; i += blockDim.x) dst[i] = hdr.b[i];
+    }
     if (threadIdx.x == 0) {
         const int64_t end = hlen + nbytes + (int64_t)ff;
         dst[end] = 0xFF;
@@ -514,12 +832,14 @@ __global__ void __launch_bounds__(SCAN_THREADS) jpeg_ff_scan_kernel(Geo g, Work 
     }
 }
 
-__global__ void jpeg_stuff_kernel(Geo g, Work w, int n, int hlen, uint8_t *out, int64_t slot) {
+// OPT: each frame's data starts after its own header (op.hlen, from jpeg_ff_scan)
+template <bool OPT>
+__global__ void jpeg_stuff_kernel(Geo g, Work w, int n, int hlen, uint8_t *out, int64_t slot, Opt op) {
     const int64_t gs = (int64_t)gridDim.x * blockDim.x;
     for (int f = 0; f < n; ++f) {
         const int64_t nbytes = entropy_bytes(w.bits[f]), nch = (nbytes + CHUNK - 1) / CHUNK;
         const uint32_t *wd = w.words + (int64_t)f * (g.wbytes / 4);
-        uint8_t *dst = out + (int64_t)f * slot + hlen;
+        uint8_t *dst = out + (int64_t)f * slot + (OPT ? op.hlen[f] : hlen);
         for (int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; c < nch; c += gs) {
             int64_t o = c * CHUNK + w.ffcnt[(int64_t)f * g.chunks + c];
             const int nb = (int)min((int64_t)CHUNK, nbytes - c * CHUNK);
@@ -534,6 +854,13 @@ __global__ void jpeg_stuff_kernel(Geo g, Work w, int n, int hlen, uint8_t *out, 
 }
 
 bool dims_ok(int H, int W) { return H >= 1 && H <= 65535 && W >= 1 && W <= 65535; }
+
+// the optimized header (prefix, at most DHT_LEN_MAX bytes of DHT segments, SOS) fits AVB_JPEG_HEADER_MAX, which the slot
+// bound counts
+bool prefix_len_ok(int prefix_len, int sos_len) {
+    return prefix_len >= 2 && sos_len >= 2 && prefix_len <= AVB_JPEG_HEADER_MAX &&
+           sos_len <= AVB_JPEG_HEADER_MAX - DHT_LEN_MAX - prefix_len;
+}
 
 }  // namespace
 
@@ -554,6 +881,14 @@ extern "C" int64_t avb_jpeg_workspace_bytes(int n, int H, int W) {
     return carve(geometry(H, W), n, nullptr, nullptr);
 }
 
+extern "C" int64_t avb_jpeg_opt_workspace_bytes(int n, int H, int W) {
+    if (!dims_ok(H, W) || n < 1 || n > 65535) {
+        avb::set_error("avb_jpeg_opt_workspace_bytes: bad geometry");
+        return AVB_E_ARG;
+    }
+    return carve_opt(geometry(H, W), n, nullptr, nullptr);
+}
+
 namespace {
 
 // AVB_REQUIRE with the name of the entry point that was called
@@ -565,15 +900,21 @@ namespace {
         }                                       \
     } while (0)
 
-template <bool RGB>
+// OPT: header_host is the prefix before the DHT segments, sos_host the SOS segment
+template <bool RGB, bool OPT>
 int encode(const char *fn, const uint8_t *in, int n, int H, int W, int64_t in_frame_stride, int64_t in_row_stride,
-           const uint8_t *header_host, int header_len, const uint8_t *qtables_host, uint8_t *out, int64_t out_slot_stride,
-           int64_t *out_lengths_dev, void *workspace_dev, avb_stream_t stream) {
-    K8_REQUIRE(in && header_host && qtables_host && out && out_lengths_dev && workspace_dev, "null pointer");
+           const uint8_t *header_host, int header_len, const uint8_t *sos_host, int sos_len, const uint8_t *qtables_host,
+           uint8_t *out, int64_t out_slot_stride, int64_t *out_lengths_dev, void *workspace_dev, avb_stream_t stream) {
+    K8_REQUIRE(in && header_host && (sos_host || !OPT) && qtables_host && out && out_lengths_dev && workspace_dev,
+               "null pointer");
     K8_REQUIRE(n >= 1 && n <= 65535 && dims_ok(H, W), "n must lie in [1, 65535], H and W in [1, 65535]");
     K8_REQUIRE(in_row_stride >= 3LL * W && (n == 1 || in_frame_stride >= in_row_stride * (H - 1) + 3LL * W),
                 "input strides overlap");
-    K8_REQUIRE(header_len >= 2 && header_len <= AVB_JPEG_HEADER_MAX, "header_len must lie in [2, AVB_JPEG_HEADER_MAX]");
+    if constexpr (OPT)
+        K8_REQUIRE(prefix_len_ok(header_len, sos_len),
+                   "prefix_len and sos_len must be at least 2, prefix_len + sos_len + 432 at most AVB_JPEG_HEADER_MAX");
+    else
+        K8_REQUIRE(header_len >= 2 && header_len <= AVB_JPEG_HEADER_MAX, "header_len must lie in [2, AVB_JPEG_HEADER_MAX]");
     K8_REQUIRE(out_slot_stride >= avb_jpeg_bound_bytes(H, W), "output slot smaller than avb_jpeg_bound_bytes(H, W)");
     K8_REQUIRE(((uintptr_t)workspace_dev & 15) == 0, "workspace must be 16-byte aligned");
     const Geo g = geometry(H, W);
@@ -593,16 +934,38 @@ int encode(const char *fn, const uint8_t *in, int n, int H, int W, int64_t in_fr
     memcpy(hdr.b, header_host, header_len);
     Work w;
     carve(g, n, (uint8_t *)workspace_dev, &w);
+    Opt op{};
+    if constexpr (OPT) {
+        memcpy(hdr.b + header_len, sos_host, sos_len);
+        carve_opt(g, n, (uint8_t *)workspace_dev, &op);
+        op.slen = sos_len;
+    }
     cudaStream_t st = (cudaStream_t)stream;
     const int grid = avb::sm_count() * 4;
+    const unsigned block_ctas = (unsigned)((g.M * 6 + 255) / 256);
+    if constexpr (OPT) AVB_CUDA_OK(cudaMemsetAsync(op.freq, 0, (size_t)n * 4 * 256 * 8, st));
     {
         AVB_TIMED("jpeg_transform", st);
-        jpeg_transform_kernel<RGB><<<dim3((g.mw + STRIP - 1) / STRIP, g.mh, n), TF_THREADS, 0, st>>>(in, in_frame_stride,
-                                                                                                   in_row_stride, g, qd, w);
+        jpeg_transform_kernel<RGB, OPT><<<dim3((g.mw + STRIP - 1) / STRIP, g.mh, n), TF_THREADS, 0, st>>>(
+            in, in_frame_stride, in_row_stride, g, qd, w, op);
+    }
+    if constexpr (OPT) {
+        {
+            AVB_TIMED("jpeg_dc_hist", st);
+            jpeg_dc_hist_kernel<<<dim3((unsigned)((g.M + 255) / 256), n), 256, 0, st>>>(g, w, op);
+        }
+        {
+            AVB_TIMED("jpeg_tables", st);
+            jpeg_tables_kernel<<<n, 128, 0, st>>>(op);
+        }
+        {
+            AVB_TIMED("jpeg_blen", st);
+            jpeg_blen_kernel<<<dim3(block_ctas, n), 256, 0, st>>>(g, w, op);
+        }
     }
     {
         AVB_TIMED("jpeg_mcu_scan", st);
-        jpeg_mcu_scan_kernel<<<n, SCAN_THREADS, 0, st>>>(g, w);
+        jpeg_mcu_scan_kernel<OPT><<<n, SCAN_THREADS, 0, st>>>(g, w, op);
     }
     {
         AVB_TIMED("jpeg_zero", st);
@@ -610,7 +973,7 @@ int encode(const char *fn, const uint8_t *in, int n, int H, int W, int64_t in_fr
     }
     {
         AVB_TIMED("jpeg_emit", st);
-        jpeg_emit_kernel<<<dim3((unsigned)((g.M * 6 + 255) / 256), n), 256, 0, st>>>(g, w);
+        jpeg_emit_kernel<OPT><<<dim3(block_ctas, n), 256, 0, st>>>(g, w, op);
     }
     {
         AVB_TIMED("jpeg_ff_count", st);
@@ -618,11 +981,12 @@ int encode(const char *fn, const uint8_t *in, int n, int H, int W, int64_t in_fr
     }
     {
         AVB_TIMED("jpeg_ff_scan", st);
-        jpeg_ff_scan_kernel<<<n, SCAN_THREADS, 0, st>>>(g, w, hdr, header_len, out, out_slot_stride, out_lengths_dev);
+        jpeg_ff_scan_kernel<OPT><<<n, SCAN_THREADS, 0, st>>>(g, w, hdr, header_len, out, out_slot_stride, out_lengths_dev,
+                                                            op);
     }
     {
         AVB_TIMED("jpeg_stuff", st);
-        jpeg_stuff_kernel<<<grid, 256, 0, st>>>(g, w, n, header_len, out, out_slot_stride);
+        jpeg_stuff_kernel<OPT><<<grid, 256, 0, st>>>(g, w, n, header_len, out, out_slot_stride, op);
     }
     AVB_CUDA_OK(cudaGetLastError());
     return AVB_OK;
@@ -636,14 +1000,32 @@ extern "C" int avb_jpeg_encode_u8(const uint8_t *in, int n, int H, int W, int64_
                                   const uint8_t *header_host, int header_len, const uint8_t *qtables_host, uint8_t *out,
                                   int64_t out_slot_stride, int64_t *out_lengths_dev, void *workspace_dev,
                                   avb_stream_t stream) {
-    return encode<false>(__func__, in, n, H, W, in_frame_stride, in_row_stride, header_host, header_len, qtables_host,
-                         out, out_slot_stride, out_lengths_dev, workspace_dev, stream);
+    return encode<false, false>(__func__, in, n, H, W, in_frame_stride, in_row_stride, header_host, header_len, nullptr, 0,
+                                qtables_host, out, out_slot_stride, out_lengths_dev, workspace_dev, stream);
 }
 
 extern "C" int avb_jpeg_encode_rgb_u8(const uint8_t *in, int n, int H, int W, int64_t in_frame_stride,
                                       int64_t in_row_stride, const uint8_t *header_host, int header_len,
                                       const uint8_t *qtables_host, uint8_t *out, int64_t out_slot_stride,
                                       int64_t *out_lengths_dev, void *workspace_dev, avb_stream_t stream) {
-    return encode<true>(__func__, in, n, H, W, in_frame_stride, in_row_stride, header_host, header_len, qtables_host,
-                        out, out_slot_stride, out_lengths_dev, workspace_dev, stream);
+    return encode<true, false>(__func__, in, n, H, W, in_frame_stride, in_row_stride, header_host, header_len, nullptr, 0,
+                               qtables_host, out, out_slot_stride, out_lengths_dev, workspace_dev, stream);
+}
+
+extern "C" int avb_jpeg_opt_encode_u8(const uint8_t *in, int n, int H, int W, int64_t in_frame_stride,
+                                      int64_t in_row_stride, const uint8_t *prefix_host, int prefix_len,
+                                      const uint8_t *sos_host, int sos_len, const uint8_t *qtables_host, uint8_t *out,
+                                      int64_t out_slot_stride, int64_t *out_lengths_dev, void *workspace_dev,
+                                      avb_stream_t stream) {
+    return encode<false, true>(__func__, in, n, H, W, in_frame_stride, in_row_stride, prefix_host, prefix_len, sos_host,
+                               sos_len, qtables_host, out, out_slot_stride, out_lengths_dev, workspace_dev, stream);
+}
+
+extern "C" int avb_jpeg_opt_encode_rgb_u8(const uint8_t *in, int n, int H, int W, int64_t in_frame_stride,
+                                          int64_t in_row_stride, const uint8_t *prefix_host, int prefix_len,
+                                          const uint8_t *sos_host, int sos_len, const uint8_t *qtables_host, uint8_t *out,
+                                          int64_t out_slot_stride, int64_t *out_lengths_dev, void *workspace_dev,
+                                          avb_stream_t stream) {
+    return encode<true, true>(__func__, in, n, H, W, in_frame_stride, in_row_stride, prefix_host, prefix_len, sos_host,
+                              sos_len, qtables_host, out, out_slot_stride, out_lengths_dev, workspace_dev, stream);
 }

@@ -175,9 +175,10 @@ class HostBatchPipeline:
     def _jpeg_bufs(self, h: int, w: int, k8):
         """`depth` rotating sets of (K8 workspace, K8 slots, packed records, device [offsets | lengths], the same pinned)
         for chunks of h x w frames, used beside _slot_bufs' buffers of the same slot index.  Like _slot_bufs they are
-        kept for the pipeline's lifetime, per (h, w): at 4K in chunks of 2 about 0.5 GB of device memory per slot (K8's
-        worst-case slot bound is 84 MB a frame, for the slots and again for the packed records)."""
-        key = (h, w)
+        kept for the pipeline's lifetime, per (h, w) and K8 mode (the optimized mode's workspace is larger): at 4K in
+        chunks of 2 about 0.5 GB of device memory per slot (K8's worst-case slot bound is 84 MB a frame, for the slots
+        and again for the packed records)."""
+        key = (h, w, k8.optimize)
         if key not in self._jpeg_slots:
             t, dev, c = self.eng.torch, self.eng.device, self.chunk
             rec = 8 + ((k8.slot + 3) & ~3)
@@ -200,9 +201,10 @@ class HostBatchPipeline:
 
     def run_split_jpeg(self, jobs: Sequence[Tuple[object, object]], *,
                        labels: Optional[Tuple[str, str]] = ("Original", "Transformed"), draw_seam: bool = True,
-                       quality: int = 95, out: RecordSink):
+                       quality: int = 95, optimize: bool = False, out: RecordSink):
         """jobs as run_split's; the frames are RGB and are not modified.  Every labelled split frame is encoded on the
-        device as the bytes of `cv2.imencode(".jpg", split[..., ::-1], [IMWRITE_JPEG_QUALITY, quality])` and handed to
+        device as the bytes of `cv2.imencode(".jpg", split[..., ::-1], [IMWRITE_JPEG_QUALITY, quality])` (with
+        IMWRITE_JPEG_OPTIMIZE as well if `optimize`: each frame's own Huffman tables, in its own record) and handed to
         `out.write_records` as an AVI '00dc' record, in frame order: per chunk H2D on s_in; visualize_batch, K9, K8 (RGB)
         and the record pack (K11) on s_run; the record offsets and JPEG lengths to pinned memory on s_out.  Chunk i is
         retired once chunks up to i + depth - 1 are enqueued: the host waits for its offsets, then copies exactly its
@@ -211,7 +213,7 @@ class HostBatchPipeline:
         compressed bytes cross.  Every job, the labels and the quality are checked before anything is enqueued; waits
         once at the end, also when a job fails mid-way (the chunks not yet handed to `out` then are not).  Returns
         (h2d_bytes, d2h_bytes) as copied."""
-        from .jpeg import JPEG_LAUNCHES, JpegLauncher, check_quality
+        from .jpeg import JpegLauncher, check_quality
         t = self.eng.torch
         eng = self.eng
         plan = self._split_plan(jobs, labels, "run_split_jpeg")
@@ -222,7 +224,7 @@ class HostBatchPipeline:
         for _, src, _ in plan:
             hw = (src.shape[1], src.shape[2])
             if hw not in k8s:
-                k8s[hw] = JpegLauncher(eng.lib, *hw, quality, rgb=True)
+                k8s[hw] = JpegLauncher(eng.lib, *hw, quality, rgb=True, optimize=bool(optimize))
         h2d = d2h = 0
         pending = []                      # enqueued chunks whose records are not yet copied, oldest first
         staged = []                       # at most one (copy event, staging, bytes, lengths) not yet handed to `out`
@@ -268,7 +270,7 @@ class HostBatchPipeline:
                                     meta[n + 1:].data_ptr(), st), k8.name)
                     check(eng.lib.avb_mjpeg_pack_u8(jslots.data_ptr(), k8.slot, meta[n + 1:].data_ptr(), n,
                                                     packed.data_ptr(), meta.data_ptr(), st), "avb_mjpeg_pack_u8")
-                    eng.launches += JPEG_LAUNCHES + 1
+                    eng.launches += k8.launches + 1
                     e_run = self.s_run.record_event()
                 with t.cuda.stream(self.s_out):
                     self.s_out.wait_event(e_run)

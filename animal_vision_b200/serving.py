@@ -12,6 +12,8 @@ data-URI result, same string keys: "human", "cat", "cow", ... as utils.py:145-19
 lives decides the encoder: a view left on the device by the default runner is encoded there (K8, `jpeg.encode_jpeg`,
 the bytes of cv2.imencode) and only the compressed bytes come back; a NumPy result is encoded with cv2.imencode.
 `FrameBatcher.submit_png` does the same with PNG (K10, `png.encode_png`), and `process_image_png` wraps it as a data URI.
+`optimize=True` on the JPEG requests asks for the bytes cv2.imencode gives with IMWRITE_JPEG_OPTIMIZE: Huffman tables
+built from each file's own symbol counts, the same pixels in fewer bytes (on the device, K8's optimized mode).
 
 `FrameBatcher.submit_split_jpeg` asks for the JPEG file of the labelled split-compare frame of the request's input and
 its species view -- what the reference's CLI shows (main.py:41-48 `render_split_compare(img, out)`, with the defaults of
@@ -92,12 +94,14 @@ def _pixels(view, idx: List[int]) -> List[np.ndarray]:
         return [pin[k].numpy() for k in range(len(idx))]
 
 
-_HOST_EXT = {"jpeg": ".jpg", "png": ".png"}       # encoded request kinds and cv2's extension for each
+# encoded request kinds: cv2's extension for each, and whether it sets IMWRITE_JPEG_OPTIMIZE
+_HOST_EXT = {"jpeg": (".jpg", False), "jpeg_opt": (".jpg", True), "png": (".png", False)}
 
 
 def _encode_host(frame: np.ndarray, fmt: str = "jpeg") -> bytes:
     import cv2
-    ok, enc = cv2.imencode(_HOST_EXT[fmt], frame)
+    ext, optimize = _HOST_EXT[fmt]
+    ok, enc = cv2.imencode(ext, frame, [cv2.IMWRITE_JPEG_OPTIMIZE, 1]) if optimize else cv2.imencode(ext, frame)
     if not ok:
         raise ValueError("could not encode the result")
     return enc.tobytes()
@@ -105,7 +109,7 @@ def _encode_host(frame: np.ndarray, fmt: str = "jpeg") -> bytes:
 
 def _encoded(view, idx: List[int], fmt: str) -> List[bytes]:
     """Files of the frames `idx` of a batch result, the bytes cv2.imencode gives with its defaults: JPEG at quality 95
-    (fmt "jpeg") or PNG (fmt "png")."""
+    (fmt "jpeg"; "jpeg_opt" with IMWRITE_JPEG_OPTIMIZE) or PNG (fmt "png")."""
     if isinstance(view, np.ndarray):
         return [_encode_host(view[i], fmt) for i in idx]
     import torch
@@ -113,22 +117,23 @@ def _encoded(view, idx: List[int], fmt: str) -> List[bytes]:
     from .png import encode_png
     with torch.cuda.device(view.device):
         sel = _rows(view, idx)
-        return encode_jpeg(sel, 95) if fmt == "jpeg" else encode_png(sel)
+        return encode_png(sel) if fmt == "png" else encode_jpeg(sel, 95, optimize=fmt == "jpeg_opt")
 
 
-def _split_host(frame: np.ndarray, view: np.ndarray, labels: Tuple[str, str], seam: bool) -> bytes:
+def _split_host(frame: np.ndarray, view: np.ndarray, labels: Tuple[str, str], seam: bool, optimize: bool = False) -> bytes:
     """The host route of a split request: slice copies, cv2 labels, cv2.imencode."""
     import torch
     from .renderers.video import draw_split_labels, split_compare_batch
     comp = split_compare_batch(torch.from_numpy(frame[None]), torch.from_numpy(np.ascontiguousarray(view)[None]),
                                draw_seam=seam)[0].numpy()
-    return _encode_host(draw_split_labels(comp, *labels))
+    return _encode_host(draw_split_labels(comp, *labels), "jpeg_opt" if optimize else "jpeg")
 
 
-def _split_jpegs(frames: np.ndarray, dev_in, view, idx: List[int], labels: Tuple[str, str], seam: bool) -> List[bytes]:
+def _split_jpegs(frames: np.ndarray, dev_in, view, idx: List[int], labels: Tuple[str, str], seam: bool,
+                 optimize: bool = False) -> List[bytes]:
     """JPEG files of the labelled split frames (input | species view) of the frames `idx` of a batch."""
     if isinstance(view, np.ndarray):
-        return [_split_host(frames[i], view[i], labels, seam) for i in idx]
+        return [_split_host(frames[i], view[i], labels, seam, optimize) for i in idx]
     import torch
     from .jpeg import encode_jpeg
     from .renderers.video import split_compare_batch
@@ -136,7 +141,7 @@ def _split_jpegs(frames: np.ndarray, dev_in, view, idx: List[int], labels: Tuple
         if dev_in is None:
             dev_in = torch.from_numpy(frames).pin_memory().to(view.device, non_blocking=True)
         orig, sel = _rows(dev_in, idx), _rows(view, idx)
-        return encode_jpeg(split_compare_batch(orig, sel, draw_seam=seam, labels=labels), 95)
+        return encode_jpeg(split_compare_batch(orig, sel, draw_seam=seam, labels=labels), 95, optimize=optimize)
 
 
 def _check_labels(labels) -> Tuple[str, str]:
@@ -167,21 +172,22 @@ class FrameBatcher:
         """Future of the species view of `frame`, an HxWx3 uint8 array."""
         return self._submit(frame, animal, None)
 
-    def submit_jpeg(self, frame: np.ndarray, animal: str) -> Future:
-        """Future of the JPEG file (bytes) of the species view, the bytes cv2.imencode(".jpg", view) gives."""
-        return self._submit(frame, animal, "jpeg")
+    def submit_jpeg(self, frame: np.ndarray, animal: str, optimize: bool = False) -> Future:
+        """Future of the JPEG file (bytes) of the species view, the bytes cv2.imencode(".jpg", view) gives; with
+        `optimize`, the bytes of cv2.imencode(".jpg", view, [cv2.IMWRITE_JPEG_OPTIMIZE, 1])."""
+        return self._submit(frame, animal, "jpeg_opt" if optimize else "jpeg")
 
     def submit_png(self, frame: np.ndarray, animal: str) -> Future:
         """Future of the PNG file (bytes) of the species view, the bytes cv2.imencode(".png", view) gives."""
         return self._submit(frame, animal, "png")
 
     def submit_split_jpeg(self, frame: np.ndarray, animal: str, labels: Tuple[str, str] = ("Original", "Transformed"),
-                          draw_seam: bool = True) -> Future:
+                          draw_seam: bool = True, optimize: bool = False) -> Future:
         """Future of the JPEG file (bytes) of the split-compare frame of `frame` and its species view: left half of
         the input, right half of the view, the seam, and the two corner labels -- the bytes of
-        cv2.imencode(".jpg", draw_split_labels(split frame, *labels))."""
+        cv2.imencode(".jpg", draw_split_labels(split frame, *labels)), with IMWRITE_JPEG_OPTIMIZE if `optimize`."""
         try:
-            kind = ("split", _check_labels(labels), bool(draw_seam))
+            kind = ("split", _check_labels(labels), bool(draw_seam), bool(optimize))
         except TypeError as e:
             fut: Future = Future()
             fut.set_exception(e)
@@ -189,7 +195,7 @@ class FrameBatcher:
         return self._submit(frame, animal, kind)
 
     def _submit(self, frame: np.ndarray, animal: str, kind) -> Future:
-        """kind: None (pixels), "jpeg", "png", or ("split", labels, seam)."""
+        """kind: None (pixels), "jpeg", "jpeg_opt", "png", or ("split", labels, seam, optimize)."""
         fut: Future = Future()
         if animal != "human" and animal not in SERVER_KEYS:
             fut.set_exception(KeyError(f"no case implemented for {animal!r}"))             # utils.py:192-193 prints and fails later
@@ -202,7 +208,7 @@ class FrameBatcher:
                 fut.set_result(frame)
                 return fut
             try:
-                fut.set_result(_encode_host(frame, kind) if kind in _HOST_EXT else _split_host(frame, frame, kind[1], kind[2]))
+                fut.set_result(_encode_host(frame, kind) if kind in _HOST_EXT else _split_host(frame, frame, *kind[1:]))
             except Exception as e:          # noqa: BLE001
                 fut.set_exception(e)
             return fut
@@ -260,8 +266,8 @@ class FrameBatcher:
             idx = [i for i, (_, _, kind) in enumerate(part) if kind == fmt]
             if idx:
                 res.update(zip(idx, _encoded(out, idx, fmt)))
-        for (labels, seam), idx in splits.items():
-            res.update(zip(idx, _split_jpegs(batch, dev_in, out, idx, labels, seam)))
+        for (labels, seam, optimize), idx in splits.items():
+            res.update(zip(idx, _split_jpegs(batch, dev_in, out, idx, labels, seam, optimize)))
         for i, (_, fut, _) in enumerate(part):
             fut.set_result(res[i])
 
@@ -300,10 +306,12 @@ def _data_uri(imagedata: bytes, submit: Callable[[np.ndarray], Future], mime: st
     return f"data:{mime};base64," + base64.b64encode(submit(img).result()).decode("utf-8")
 
 
-def process_image(imagedata: bytes, animal: str, batcher: Optional[FrameBatcher] = None) -> str:
+def process_image(imagedata: bytes, animal: str, batcher: Optional[FrameBatcher] = None, *, optimize: bool = False) -> str:
     """Drop-in for utils.py:133-199 `processimage`: JPEG bytes in, JPEG data URI out; decoded BGR as cv2.imread gives it
-    (the species index channels 0/1/2, never "R/G/B" -- the reference feeds BGR here too, utils.py:141-142)."""
-    return _data_uri(imagedata, lambda img: (batcher or default_batcher()).submit_jpeg(img, animal), "image/jpeg")
+    (the species index channels 0/1/2, never "R/G/B" -- the reference feeds BGR here too, utils.py:141-142).
+    `optimize=True` answers with the smaller file of IMWRITE_JPEG_OPTIMIZE (same pixels)."""
+    return _data_uri(imagedata, lambda img: (batcher or default_batcher()).submit_jpeg(img, animal, optimize),
+                     "image/jpeg")
 
 
 def process_image_png(imagedata: bytes, animal: str, batcher: Optional[FrameBatcher] = None) -> str:
@@ -313,9 +321,9 @@ def process_image_png(imagedata: bytes, animal: str, batcher: Optional[FrameBatc
 
 
 def process_split_image(imagedata: bytes, animal: str, labels: Tuple[str, str] = ("Original", "Transformed"),
-                        batcher: Optional[FrameBatcher] = None) -> str:
+                        batcher: Optional[FrameBatcher] = None, *, optimize: bool = False) -> str:
     """JPEG bytes in, data URI of the JPEG of the labelled split-compare frame out (input on the left, species view on
     the right, seam, corner labels; `FrameBatcher.submit_split_jpeg`).  Decoded BGR as cv2.imread gives it, like
-    `process_image`."""
-    return _data_uri(imagedata, lambda img: (batcher or default_batcher()).submit_split_jpeg(img, animal, labels),
-                     "image/jpeg")
+    `process_image`; `optimize` as there."""
+    return _data_uri(imagedata, lambda img: (batcher or default_batcher()).submit_split_jpeg(
+        img, animal, labels, optimize=optimize), "image/jpeg")

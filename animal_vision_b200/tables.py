@@ -519,20 +519,30 @@ def _jpeg_segment(marker: int, payload: bytes) -> bytes:
     return bytes([0xFF, marker]) + (len(payload) + 2).to_bytes(2, "big") + payload
 
 
-def jpeg_header(H: int, W: int, quality: int) -> bytes:
-    """Every byte cv2.imencode writes before the entropy-coded data: SOI, APP0 JFIF 1.01 (density 1:1, no units),
-    DQT luma / chroma, SOF0 (3 components, 4:2:0), DHT DC0 / AC0 / DC1 / AC1, SOS."""
+def jpeg_header_prefix(H: int, W: int, quality: int) -> bytes:
+    """The bytes cv2.imencode writes before the first DHT segment: SOI, APP0 JFIF 1.01 (density 1:1, no units), DQT
+    luma / chroma, SOF0 (3 components, 4:2:0).  The optimized-table encode writes each frame's DHT segments after it."""
     if not (1 <= int(H) <= 65535 and 1 <= int(W) <= 65535):
         raise ValueError(f"JPEG frame size must lie in [1, 65535]^2, got {H}x{W}")
     qt = jpeg_quant_tables(quality)
     out = b"\xff\xd8" + _jpeg_segment(0xE0, b"JFIF\x00\x01\x01\x00\x00\x01\x00\x01\x00\x00")
     for i in range(2):
         out += _jpeg_segment(0xDB, bytes([i]) + qt[i].tobytes())
-    out += _jpeg_segment(0xC0, bytes([8]) + int(H).to_bytes(2, "big") + int(W).to_bytes(2, "big")
-                         + bytes([3, 1, 0x22, 0, 2, 0x11, 1, 3, 0x11, 1]))
+    return out + _jpeg_segment(0xC0, bytes([8]) + int(H).to_bytes(2, "big") + int(W).to_bytes(2, "big")
+                               + bytes([3, 1, 0x22, 0, 2, 0x11, 1, 3, 0x11, 1]))
+
+
+# The SOS segment that follows the DHT segments: Y with tables 0, Cb and Cr with tables 1, spectral range 0..63
+JPEG_SOS = _jpeg_segment(0xDA, bytes([3, 1, 0x00, 2, 0x11, 3, 0x11, 0, 63, 0]))
+
+
+def jpeg_header(H: int, W: int, quality: int) -> bytes:
+    """Every byte cv2.imencode writes before the entropy-coded data: `jpeg_header_prefix`, DHT DC0 / AC0 / DC1 / AC1
+    (the standard tables), `JPEG_SOS`."""
+    out = jpeg_header_prefix(H, W, quality)
     for tc, bits, vals in _JPEG_STD_HUFF:
         out += _jpeg_segment(0xC4, bytes([tc]) + bytes.fromhex(bits) + bytes.fromhex(vals))
-    return out + _jpeg_segment(0xDA, bytes([3, 1, 0x00, 2, 0x11, 3, 0x11, 0, 63, 0]))
+    return out + JPEG_SOS
 
 
 # ----------------------------------------------------------------------------- PNG (K10)

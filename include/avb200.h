@@ -371,6 +371,26 @@ AVB_API int avb_jpeg_encode_rgb_u8(const uint8_t *in, int n, int H, int W, int64
                                    int64_t in_row_stride, const uint8_t *header_host, int header_len,
                                    const uint8_t *qtables_host, uint8_t *out, int64_t out_slot_stride,
                                    int64_t *out_lengths_dev, void *workspace_dev, avb_stream_t stream);
+/* Optimized Huffman tables: the bytes of cv2.imencode(".jpg", frame, [IMWRITE_JPEG_QUALITY, q, IMWRITE_JPEG_OPTIMIZE, 1])
+ * (libjpeg's jpeg_gen_optimal_table on each frame's own symbol counts; the same pixels, usually a smaller file).  Each
+ * frame's four DHT segments are built and written on the device; no host synchronisation.
+ *   prefix_host     the bytes before the DHT segments (SOI .. SOF0; animal_vision_b200/tables.py jpeg_header_prefix)
+ *   sos_host        the SOS segment (tables.py JPEG_SOS); prefix_len, sos_len >= 2 and
+ *                   prefix_len + sos_len + 432 <= AVB_JPEG_HEADER_MAX (432: the four DHT segments at most)
+ *   workspace_dev   avb_jpeg_opt_workspace_bytes(n, H, W) bytes, 16-byte aligned
+ * Other arguments, the slots and the lengths as avb_jpeg_encode_u8; avb_jpeg_bound_bytes bounds a slot. */
+AVB_API int64_t avb_jpeg_opt_workspace_bytes(int n, int H, int W);
+AVB_API int avb_jpeg_opt_encode_u8(const uint8_t *in, int n, int H, int W, int64_t in_frame_stride,
+                                   int64_t in_row_stride, const uint8_t *prefix_host, int prefix_len,
+                                   const uint8_t *sos_host, int sos_len, const uint8_t *qtables_host, uint8_t *out,
+                                   int64_t out_slot_stride, int64_t *out_lengths_dev, void *workspace_dev,
+                                   avb_stream_t stream);
+/* The same for frames in RGB order (cv2.imencode of frame[..., ::-1] with IMWRITE_JPEG_OPTIMIZE). */
+AVB_API int avb_jpeg_opt_encode_rgb_u8(const uint8_t *in, int n, int H, int W, int64_t in_frame_stride,
+                                       int64_t in_row_stride, const uint8_t *prefix_host, int prefix_len,
+                                       const uint8_t *sos_host, int sos_len, const uint8_t *qtables_host, uint8_t *out,
+                                       int64_t out_slot_stride, int64_t *out_lengths_dev, void *workspace_dev,
+                                       avb_stream_t stream);
 
 /* ---- K11: Motion-JPEG AVI records (csrc/k11_mjpeg.cu) ----------------------------------------------------------
  * Packs n encoded files, file f at slots + f * slot_stride and lengths_dev[f] bytes long (device int64, e.g. the slots
